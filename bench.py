@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- decoded syndromes/s of the fused message-passing decoder (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (GNNI.forward: T message-passing iterations + read-out +
 hard decision) over one batch of synthetic syndromes.  N = 1 workload = BASELINE.json configs[1]:
@@ -21,6 +21,9 @@ data-path collective (SURVEY.md section 8e) -> "scaling": "weak".
            with its peak measured live by gd_microbench.
 `cpu_baseline` / `--impl reference`: the oracle port of the reference's CPU path (same ATen op
            sequence, torch threads = all host cores) on a bounded sample of the same workload.
+`--dump-outputs DIR`: the headline workload's prob and hard decisions from the last timed step, as float32 .npy files.  The
+           inputs are a function of the arguments alone (seeded sampler, shipped weights), so the files of two builds compare
+           output for output.
 """
 import argparse
 import ctypes as C
@@ -209,6 +212,24 @@ def cpu_reference_rate(program, pcm, T, weights, x_sample, chunk, budget_s, thre
     return done / t_used, done, t_used
 
 
+DUMP_BUDGET = 63 * 10 ** 6      # bytes of array data written by --dump-outputs: with the .npy headers, under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each [B, ...] output as path/<name>.npy in float32, so that two builds can be compared output for output.  When they
+    exceed DUMP_BUDGET together, the same fixed, seeded sample of rows is kept from each, and its row indices go to rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes for a in arrays.values()) // max(n, 1)
+    if n * row_bytes > DUMP_BUDGET:
+        rows = np.sort(np.random.RandomState(1234).choice(n, DUMP_BUDGET // (row_bytes + 8), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -219,7 +240,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-autotune", action="store_true", help="keep the planner's model geometry (skip gd_decode_autotune)")
     ap.add_argument("--no-extras", action="store_true", help="headline workload only (skip the short passes over the other BASELINE configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload returned (prob, hard) as DIR/<name>.npy "
+                         "(rank 0's shard under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -408,25 +436,27 @@ def run_workload(name, args, dev, rank, world, clocks, headline):
         step()
         e1.record(stream)
     barrier()
-    clock_probe_s = 0.0
     if clocks is not None and rank == 0:
         clocks.end()
-        # The timed region can be shorter than the clock sampler's period (nvidia-smi reports every 20 ms): keep exactly the same
-        # step running, untimed, for 0.3 s more so the clocks / throttle reasons are sampled under this load.
-        if clocks.windows[-1][1] - clocks.windows[-1][0] < 0.3:
-            clocks.begin()
-            t_probe = time.monotonic()
-            while time.monotonic() - t_probe < 0.3:
-                for _ in range(8):
-                    step()
-                torch.cuda.synchronize(dev)
-            clocks.end()
-            clock_probe_s = round(time.monotonic() - t_probe, 3)
+    prob_ref, hard_ref = prob.cpu(), hard.cpu()             # what the last timed step returned
+    if headline and rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"prob": prob_ref, "hard": hard_ref})
+    clock_probe_s = 0.0
+    # The timed region can be shorter than the clock sampler's period (nvidia-smi reports every 20 ms): keep exactly the same
+    # step running, untimed, for 0.3 s more so the clocks / throttle reasons are sampled under this load.
+    if clocks is not None and rank == 0 and clocks.windows[-1][1] - clocks.windows[-1][0] < 0.3:
+        clocks.begin()
+        t_probe = time.monotonic()
+        while time.monotonic() - t_probe < 0.3:
+            for _ in range(8):
+                step()
+            torch.cuda.synchronize(dev)
+        clocks.end()
+        clock_probe_s = round(time.monotonic() - t_probe, 3)
     kernel_ms = [e0.elapsed_time(e1) for e0, e1 in evs]
     total_ms_max = allmax(sum(kernel_ms))
     ms_per_step = total_ms_max / steps
     value = world * B * steps / (total_ms_max * 1e-3)
-    prob_ref, hard_ref = prob.cpu(), hard.cpu()
 
     # ---- end to end: pinned host buffers -> device -> decode -> host, every step, through the asynchronous pipeline ----
     depth = 3

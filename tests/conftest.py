@@ -55,6 +55,17 @@ def gd_opt():
     o.restore()
 
 
+@pytest.fixture
+def one_cpu_thread():
+    """Run the test's CPU arithmetic on one thread.  How torch's CPU matmuls and reductions split their rows over threads sets
+    the order of floating-point sums, so the bit-exact comparisons with the golden fixtures hold at one thread, on a host with
+    any number of cores, and not at every thread count (at 3, 5 or 7 threads some fixtures differ in the last bit)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    yield
+    torch.set_num_threads(n)
+
+
 def logit_bound(ref, rtol=1e-4):
     """The parity bar on soft logits (BASELINE.json north_star: "within 1e-4 relative in fp32"): |got - ref| <= rtol * max(|ref|, 1),
     i.e. rtol relative for |logit| >= 1 and rtol ABSOLUTE below (a logit is a sum of fp32 terms of magnitude ~10-100, so its

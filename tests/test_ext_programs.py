@@ -11,6 +11,7 @@ from oracle import ref_loader, restate
 
 CASES = {"ext_neural_bp_toricL4": "quantum.neural_BP", "ext_gru_ca_toricL4": "quantum.QGNNNI_ca"}
 RTOL, LOGIT_TIE = 1e-4, 1e-3
+pytestmark = pytest.mark.usefixtures("one_cpu_thread")
 
 
 def _all_prob(name):

@@ -8,6 +8,8 @@ import torch
 from conftest import Golden, golden_cases
 from oracle import ref_loader, restate
 
+pytestmark = pytest.mark.usefixtures("one_cpu_thread")
+
 
 @pytest.mark.parametrize("name", golden_cases())
 def test_restatement_matches_golden_bit_exact(name):
