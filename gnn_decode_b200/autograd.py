@@ -1,6 +1,6 @@
 """Training path: torch.autograd.Function around the hand-written forward-with-stash and backward
-kernels (gd_decode_fwd_train / gd_decode_bwd).  Gradients flow to the decoder's MLP parameters
-(the reference never differentiates w.r.t. its inputs)."""
+kernels (gd_decode_fwd_train / gd_decode_bwd) of decoder_v2_4 and CGNNI.  Gradients flow to the
+decoder's MLP parameters (the reference never differentiates w.r.t. its inputs)."""
 import ctypes as ct
 
 import torch
@@ -32,7 +32,7 @@ class _DecodeFn(torch.autograd.Function):
             _cabi.check(lib.gd_decode_fwd_train(graph.handle, ct.byref(model), _ptr(w), _ptr(x32), _ptr(prob),
                                                 _ptr(logit), _ptr(stash), B, st), "gd_decode_fwd_train")
         ctx.decoder, ctx.graph, ctx.model = decoder, graph, model
-        ctx.save_for_backward(x32, w, stash, prob)
+        ctx.save_for_backward(x32, w, stash, prob, logit)
         ctx.shapes = [(p.shape, p.dtype) for p in params]
         ctx.mark_non_differentiable(logit)
         return prob, logit
@@ -40,12 +40,19 @@ class _DecodeFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_prob, _grad_logit_unused):
         lib = _cabi.lib()
-        x32, w, stash, prob = ctx.saved_tensors
+        x32, w, stash, prob, logit = ctx.saved_tensors
         graph, model = ctx.graph, ctx.model
         dev = x32.device
         B = x32.size(0)
-        # prob = sigmoid(-logit)  ->  dL/dlogit = -dL/dprob * prob * (1 - prob)
-        grad_logit = (-(grad_prob.to(torch.float32)) * prob * (1.0 - prob)).contiguous()
+        g = grad_prob.to(torch.float32)
+        if model.program == _cabi.PROG_CGNNI:
+            # prob = clamp(s, 1e-7, 1 - 1e-7), s = sigmoid(-logit) (CGNNI.py:282): torch.clamp's gradient mask is inclusive,
+            # so clamped outputs pass nothing; dL/dlogit = -dL/dprob * s * (1 - s) on the rest
+            s = torch.sigmoid(-logit)
+            grad_logit = torch.where((s >= 1e-7) & (s <= 1.0 - 1e-7), -g * s * (1.0 - s), torch.zeros_like(s)).contiguous()
+        else:
+            # prob = sigmoid(-logit)  ->  dL/dlogit = -dL/dprob * prob * (1 - prob)
+            grad_logit = (-g * prob * (1.0 - prob)).contiguous()
         n_ws = lib.gd_bwd_workspace_floats(graph.handle, ct.byref(model), B)
         if n_ws < 0:
             _cabi.check(_cabi.GD_ERR_UNSUPPORTED, "gd_bwd_workspace_floats")
@@ -66,8 +73,8 @@ class _DecodeFn(torch.autograd.Function):
 
 
 def decode_with_grad(decoder, graph, x, return_logits=False, return_hard=False):
-    if decoder._gd_program != _cabi.PROG_V2_4:
-        raise _cabi.GdError("training (backward) kernels exist for the decoder_v2_4 program only; "
+    if decoder._gd_program not in (_cabi.PROG_V2_4, _cabi.PROG_CGNNI):
+        raise _cabi.GdError("training (backward) kernels exist for the decoder_v2_4 and CGNNI programs only; "
                             "call .eval() or wrap inference in torch.no_grad()")
     x32 = x.detach().to(torch.float32).contiguous()
     if x32.data_ptr() % 16:

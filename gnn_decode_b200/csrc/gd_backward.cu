@@ -18,6 +18,7 @@
 #include "gd_math.cuh"
 #include "gd_options.cuh"
 #include "gd_lean.cuh"
+#include "gd_light.cuh"
 #include <stdlib.h>
 #include <string.h>
 
@@ -561,8 +562,10 @@ static int plan_bwd(const gd_graph* g, const gd_model* m, int64_t B, BwdPlan* ou
 }  // namespace gd
 
 extern "C" int64_t gd_bwd_workspace_floats(const gd_graph* g, const gd_model* model, int64_t B) {
+    if (g && gd_model_valid(model) && model->program == GD_PROG_CGNNI && B > 0) return gd::light_bwd_workspace_floats(g, model, B);
     if (!g || !gd_model_valid(model) || model->program != GD_PROG_V2_4 || model->hidden > 32 * gd::kUPL || B <= 0) {
-        gd::set_error("gd_bwd_workspace_floats: unsupported model (need GD_PROG_V2_4, hidden <= %d)", 32 * gd::kUPL);
+        gd::set_error("gd_bwd_workspace_floats: unsupported model (need GD_PROG_V2_4 with hidden <= %d, or GD_PROG_CGNNI)",
+                      32 * gd::kUPL);
         return -1;
     }
     gd::BwdPlan pl;
@@ -575,8 +578,8 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
                              const float* stash_dev, const float* grad_logit_dev, float* grad_weights_dev,
                              float* workspace_dev, int32_t accumulate, int64_t B, void* stream) {
     GD_CHECK_ARG(g != nullptr, "gd_decode_bwd: graph is NULL");
-    GD_CHECK_ARG(gd_model_valid(model) && model->program == GD_PROG_V2_4,
-                 "gd_decode_bwd: only GD_PROG_V2_4 has a backward kernel");
+    GD_CHECK_ARG(gd_model_valid(model) && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI),
+                 "gd_decode_bwd: only GD_PROG_V2_4 and GD_PROG_CGNNI have a backward kernel");
     GD_CHECK_ARG(model->hidden <= 32 * gd::kUPL, "gd_decode_bwd: hidden=%d > %d unsupported", model->hidden, 32 * gd::kUPL);
     GD_CHECK_ARG(B >= 0, "gd_decode_bwd: negative B");
     GD_CHECK_ARG(grad_weights_dev != nullptr, "gd_decode_bwd: grad_weights is NULL");
@@ -587,6 +590,15 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
         return GD_OK;
     }
     GD_CHECK_ARG(weights_dev && x_dev && stash_dev && grad_logit_dev && workspace_dev, "gd_decode_bwd: NULL buffer");
+    if (model->program == GD_PROG_CGNNI) {
+        int prev = 0;
+        GD_CUDA(cudaGetDevice(&prev));
+        if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+        const int rc = gd::light_backward(g, model, weights_dev, x_dev, stash_dev, grad_logit_dev, grad_weights_dev, workspace_dev,
+                                          accumulate, B, st);
+        if (prev != g->device) cudaSetDevice(prev);
+        return rc;
+    }
     gd::BwdPlan pl;
     int rc = gd::plan_bwd(g, model, B, &pl);
     if (rc != GD_OK) return rc;

@@ -1264,16 +1264,18 @@ extern "C" int64_t gd_stash_floats(const gd_graph* g, const gd_model* model, int
         gd::set_error("gd_stash_floats: invalid argument");
         return -1;
     }
+    if (model->program == GD_PROG_CGNNI) return (int64_t)model->iters * g->E * B;          // m after every iteration (gd_light.cuh)
     return (int64_t)(model->iters + 1) * 2 * g->E * B + gd::kLeanTrainTailFloats + B;   // + the header and sorted list of gd_lean.cuh
 }
 
 extern "C" int gd_decode_fwd_train(const gd_graph* gc, const gd_model* model, const float* weights_dev,
                                    const float* x_dev, float* prob_dev, float* logit_dev, float* stash_dev, int64_t B,
                                    void* stream) {
-    GD_CHECK_ARG(model && model->program == GD_PROG_V2_4, "gd_decode_fwd_train: only GD_PROG_V2_4 has a backward kernel");
+    GD_CHECK_ARG(model && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI),
+                 "gd_decode_fwd_train: only GD_PROG_V2_4 and GD_PROG_CGNNI have a backward kernel");
     GD_CHECK_ARG(stash_dev != nullptr || B == 0, "gd_decode_fwd_train: stash is NULL");
     gd_launch_info li;
-    if (B > 0) {
+    if (B > 0 && model->program == GD_PROG_V2_4) {      // CGNNI: the node-owner kernel reports what it cannot take
         int rc = gd_decode_launch_info(gc, model, B, &li);
         if (rc != GD_OK) return rc;
         if (!li.resident) {
@@ -1320,6 +1322,12 @@ static int decode_fwd_impl(const gd_graph* gc, const gd_model* model, const floa
             if (prev != g->device) cudaSetDevice(prev);
             return lrc;
         }
+    }
+    if (stash_dev && model->program == GD_PROG_CGNNI) {
+        // CGNNI training: the node-owner kernel with its stash (gd_backward_light.cu mirrors its mapping), or an error
+        const int lrc = gd::light_decode(g, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, B, st, nullptr, stash_dev);
+        if (prev != g->device) cudaSetDevice(prev);
+        return lrc;
     }
     gd::DecodePlan pl;
     int rc = gd::plan_decode(g, model, B, &pl);

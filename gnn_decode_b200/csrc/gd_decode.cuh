@@ -39,7 +39,8 @@ __device__ __forceinline__ void gate_wait(const unsigned int* flag, unsigned int
 
 bool light_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out);
 int light_decode(const gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev,
-                 float* prob_dev, float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st, const Gate* gate = nullptr);
+                 float* prob_dev, float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st, const Gate* gate = nullptr,
+                 float* stash_dev = nullptr);
 
 bool gated_plan(const gd_graph* g, const gd_model* model, int64_t B, int* tile, int* n_tiles);
 int decode_fwd_gated(const gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,

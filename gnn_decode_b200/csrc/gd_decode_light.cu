@@ -19,31 +19,13 @@
 #include "gd_options.cuh"
 #include "gd_decode.cuh"
 #include "gd_nodemath.cuh"
+#include "gd_light.cuh"
 #include <stdlib.h>
 #include <math.h>
 #include <string.h>
 #include <vector>
 
 namespace gd {
-
-struct LightParams {
-    const float* x;
-    float* prob;
-    float* logit;
-    uint8_t* hard;
-    const float* weights;
-    GraphTables tb;
-    long long B;
-    int T, V, C, E, N;
-    int tile, lanes, R, hid, hp, n_tiles, trows;
-    int off_w, off_tab, off_x, off_m, off_t;
-    // gated launch (gd_decode_host, see Gate in gd_decode.cuh); all NULL / 0 otherwise
-    const unsigned int* gate_in;
-    unsigned int* gate_out;
-    int* gate_err;
-    unsigned int gate_epoch;
-    int gate_chunk_tiles;
-};
 
 #define GD_DEGREE_SWITCH4(d, CALL, ...)     \
     switch (d) {                            \
@@ -110,7 +92,8 @@ __device__ __forceinline__ void light_chk_node(const NodeMath<PROG, NPAD>& nm, c
     }
 }
 
-template <int PROG, int NPAD>
+// STASH (CGNNI training): m after every iteration also goes to p.stash[it][E][B] for the backward (gd_backward_light.cu)
+template <int PROG, int NPAD, bool STASH = false>
 __global__ void __launch_bounds__(512, 2) decode_light_kernel(const LightParams p) {
     extern __shared__ __align__(128) unsigned char smem[];
     using NM = NodeMath<PROG, NPAD>;
@@ -276,6 +259,22 @@ __global__ void __launch_bounds__(512, 2) decode_light_kernel(const LightParams 
 #undef GD_LC
                 }
             __syncthreads();
+            if constexpr (STASH) {   // m^{it+1}: [E][tile] rows -> stash[it][E][B]; the next writer of m_st is behind a barrier
+                const int q4 = tile / 4;
+                float* dst = p.stash + (size_t)it * E * (size_t)p.B + s0;
+                for (int i = tid; i < E * q4; i += nthr) {
+                    const int e = i / q4, c = (i - e * q4) * 4;
+                    if (c >= nvalid) continue;
+                    const float4 v = lds4(m_st + e * tile + c);
+                    float* d = dst + (size_t)e * p.B + c;
+                    if ((p.B & 3) == 0) {
+                        __stcg(reinterpret_cast<float4*>(d), v);
+                    } else {
+                        const float vv[4] = {v.x, v.y, v.z, v.w};
+                        for (int j = 0; j < 4 && c + j < nvalid; ++j) __stcg(d + j, vv[j]);
+                    }
+                }
+            }
         }
 
         // ---- read-out (variable owner): logit rows into the t region as lg[V][tile] ----
@@ -546,33 +545,32 @@ __global__ void __launch_bounds__(512, 2) decode_light_ext_kernel(const LightPar
     }
 }
 
-struct LightPlan {
-    LightParams p;
-    int threads, grid, smem, npad, cps;
-    bool ok;
-};
-
 static int align_up_l(int x, int a) { return (x + a - 1) / a * a; }
 
-static void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out) {
+void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out, bool train, int extra_rows, int extra_bytes) {
     LightParams& p = out->p;
     memset(&p, 0, sizeof(p));
     out->ok = false;
+    out->why = "program has no node-owner kernel";
     const int prog = m->program;
     const bool ext = prog == GD_PROG_NEURAL_BP || prog == GD_PROG_GRU_CA;
+    const bool force = train || opt_on(OPT_FORCE_LIGHT);
     if (prog != GD_PROG_CGNNI && prog != GD_PROG_QGNNI && prog != GD_PROG_BP_QUANTUM && prog != GD_PROG_BP_CLASSICAL && !ext) return;
     if (prog == GD_PROG_GRU_CA && (m->hidden >= 32 || (m->flags & GD_FLAG_ALL_ITERS) || opt_on(OPT_NO_PWL))) return;
     if (prog == GD_PROG_NEURAL_BP && m->hidden != g->E) return;      // the caller's argument check reports it
-    if (opt_on(OPT_NO_LIGHT) || opt_on(OPT_FORCE_STREAMED)) return;
-    if ((B + 15) / 16 < g->sm_count && !opt_on(OPT_FORCE_LIGHT)) return;   // cannot fill the GPU at any tile size: skip the search
+    if (train && m->hidden >= 32) { out->why = "hidden >= 32: the MLPs have no piecewise-linear table"; return; }
+    if (!train && (opt_on(OPT_NO_LIGHT) || opt_on(OPT_FORCE_STREAMED))) return;
+    if ((B + 15) / 16 < g->sm_count && !force) return;   // cannot fill the GPU at any tile size: skip the search
+    out->why = "code too large for the node-owner kernel (E >= 65536 or V, C >= 65535)";
     if (g->E >= 65536 || g->V >= 65535 || g->C >= 65535) return;
+    out->why = "edge order is not the canonical variable-sorted order (H.to_sparse())";
     for (size_t i = 0; i < g->h_var_edges.size(); ++i)
         if (g->h_var_edges[i] != (int32_t)i) return;           // needs the canonical variable-sorted edge order
     const bool bp = prog == GD_PROG_BP_QUANTUM || prog == GD_PROG_BP_CLASSICAL || prog == GD_PROG_NEURAL_BP;
     p.B = B; p.T = m->iters; p.V = g->V; p.C = g->C; p.E = (int)g->E; p.N = g->N; p.tb = g->t;
     p.hid = bp ? 0 : m->hidden;
     p.hp = align_up_l(p.hid, 4);
-    out->npad = (!bp && m->hidden < 32 && !opt_on(OPT_NO_PWL)) ? (m->hidden < 16 ? 16 : 32) : 0;
+    out->npad = (!bp && m->hidden < 32 && (train || !opt_on(OPT_NO_PWL))) ? (m->hidden < 16 ? 16 : 32) : 0;
     p.trows = g->E > g->V ? (int)g->E : g->V;                  // the t region doubles as the logit rows lg[V][tile]
     int off = 0;
     p.off_w = off;
@@ -582,7 +580,7 @@ static void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPla
     p.off_tab = off; off += (g->V + 1 + g->C + 1 + (int)g->E) * 2;
     off = align_up_l(off, 128);
     const int fixed = off;
-    const int64_t per_syn = ((int64_t)g->N + g->E + p.trows) * 4;
+    const int64_t per_syn = ((int64_t)g->N + g->E + p.trows + extra_rows) * 4;
     // Geometry: tile in {16, 32, 64, 128} (lanes = tile / 4 divides a warp), R thread groups of `lanes` threads, and as
     // many co-resident CTAs as shared memory and the 64-register build allow (one CTA's barriers overlap another's
     // arithmetic).  Node-owner phases are only as fast as their busiest group, so every candidate is scored by
@@ -595,7 +593,7 @@ static void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPla
     std::vector<int> load;
     for (int t = 16; t <= 128; t *= 2) {
         if (et > 0 && et != t) continue;
-        const int64_t smem = fixed + per_syn * t;
+        const int64_t smem = fixed + per_syn * t + extra_bytes;
         if (smem > g->max_smem_optin) break;
         const int lanes = t / 4;
         int r_max = 512 / lanes;
@@ -631,7 +629,8 @@ static void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPla
             if (cost < best_cost * (1.0 - 1e-12)) { best_cost = cost; best_tile = t; best_cps = cps; best_R = R; best_bal = bal; }
         }
     }
-    if (!best_tile || (best_bal < 0.3 && !opt_on(OPT_FORCE_LIGHT))) return;
+    out->why = "code too large for shared memory (the node-owner kernel keeps a tile's edge state on chip)";
+    if (!best_tile || (best_bal < 0.3 && !force)) return;
     p.tile = best_tile;
     p.lanes = best_tile / 4;
     p.R = best_R;
@@ -640,14 +639,15 @@ static void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPla
     p.off_x = fixed;
     p.off_m = p.off_x + g->N * best_tile * 4;
     p.off_t = p.off_m + (int)g->E * best_tile * 4;
-    out->smem = p.off_t + p.trows * best_tile * 4;
+    out->smem = p.off_t + p.trows * best_tile * 4;      // + extra_rows * tile * 4 + extra_bytes: the caller lays them out
     p.n_tiles = (int)((B + best_tile - 1) / best_tile);
     const int slots = g->sm_count * best_cps;
     // Small batches are latency-bound: four syndromes per lane leave 4x fewer threads than the edge-owner kernel's
     // one-syndrome-per-lane mapping (toy LDPC, B = 1024: 48 vs 35 us).  Take over only when the GPU is filled.
-    if (p.n_tiles < slots && !opt_on(OPT_FORCE_LIGHT)) return;
+    if (p.n_tiles < slots && !force) return;
     out->grid = p.n_tiles < slots ? p.n_tiles : slots;
     out->ok = true;
+    out->why = nullptr;
 }
 
 bool light_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out) {
@@ -661,9 +661,26 @@ bool light_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_l
 
 // rc < 0: not applicable (the caller keeps the edge-owner kernel); otherwise a gd_status.
 int light_decode(const gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                 float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st, const Gate* gate) {
+                 float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st, const Gate* gate, float* stash_dev) {
     LightPlan pl;
-    plan_light(g, model, B, &pl);
+    plan_light(g, model, B, &pl, stash_dev != nullptr);
+    if (stash_dev) {   // CGNNI training: this kernel is the only one the backward mirrors
+        if (model->program != GD_PROG_CGNNI) {
+            set_error("gd_decode_fwd_train: program %d has no node-owner backward", model->program);
+            return GD_ERR_UNSUPPORTED;
+        }
+        if (!pl.ok) {
+            set_error("gd_decode_fwd_train: CGNNI training needs the node-owner kernel: %s", pl.why);
+            return GD_ERR_UNSUPPORTED;
+        }
+        pl.p.x = x_dev; pl.p.prob = prob_dev; pl.p.logit = logit_dev; pl.p.hard = hard_dev; pl.p.weights = weights_dev;
+        pl.p.stash = stash_dev;
+        void (*k)(const LightParams) = pl.npad == 16 ? decode_light_kernel<GD_PROG_CGNNI, 16, true> : decode_light_kernel<GD_PROG_CGNNI, 32, true>;
+        GD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
+        k<<<pl.grid, pl.threads, pl.smem, st>>>(pl.p);
+        GD_CUDA(cudaGetLastError());
+        return GD_OK;
+    }
     if (!pl.ok) return -1;
     if (gate) {
         pl.p.gate_in = gate->in_flags; pl.p.gate_out = gate->out_counts; pl.p.gate_err = gate->err;

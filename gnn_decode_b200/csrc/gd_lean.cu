@@ -898,18 +898,6 @@ struct LeanBwdParams {
     int off_me, off_ms, off_mi, off_var, off_ct, off_rt, off_vt, smem;   // the rest of the layout depends on the pieces in use
 };
 
-// 64-bit add into a shared-memory bin with the hardware's 32-bit atomics (a 64-bit shared atomicAdd compiles to a compare-and-swap
-// spin loop: 32 lanes on one bin -- iteration 0, every message still 0 -- took ~100 us per iteration).  The low word's returned
-// old value tells whether THIS add wrapped it; the high word gets the addend's high word plus that carry, which is 0 for nearly
-// every small addend of either sign, so the second atomic is rare.  Exact and order-independent like the 64-bit add it replaces.
-__device__ __forceinline__ void fx_add(long long* slot, long long x) {
-    if (x == 0) return;
-    unsigned int* w = reinterpret_cast<unsigned int*>(slot);
-    const unsigned int lo = (unsigned int)x, hi = (unsigned int)((unsigned long long)x >> 32);
-    const unsigned int old = atomicAdd(w, lo);
-    const unsigned int h = hi + ((old + lo < old) ? 1u : 0u);
-    if (h) atomicAdd(w + 1, h);
-}
 __device__ __forceinline__ void bin_add(long long* bins, int nb, int piece, float tau, float g) {
     // piece in [-1, n]: nodes piece + 1 and piece + 2 of the (n + 3)-node grid; t in [0, 1] inside the piece
     const float t = tau + 0.5f, t2 = t * t, t3 = t2 * t;

@@ -300,6 +300,15 @@ __device__ __forceinline__ void pwl_build(float* bp, float2* seg, int npad, cons
     if (lane < npad) seg[lane] = make_float2((float)S, (float)I);
 }
 
+// The segment pwl_eval evaluates x on (the backward needs its index and slope).
+template <int NPAD>
+__device__ __forceinline__ int pwl_segment(const PwlSmem& P, float x) {
+    int i = 0;
+#pragma unroll
+    for (int s = NPAD / 2; s >= 1; s >>= 1) i += (P.bp[i + s - 1] < x) ? s : 0;
+    return i;
+}
+
 template <int NPAD>
 __device__ __forceinline__ float pwl_eval(const PwlSmem& P, float x) {
     int i = 0;
@@ -309,6 +318,18 @@ __device__ __forceinline__ float pwl_eval(const PwlSmem& P, float x) {
     return fmaf(sg.x, x, sg.y);
 }
 
+// 64-bit add into a shared-memory bin with the hardware's 32-bit atomics (a 64-bit shared atomicAdd compiles to a compare-and-swap
+// spin loop: 32 lanes on one bin -- iteration 0, every message still 0 -- took ~100 us per iteration).  The low word's returned
+// old value tells whether THIS add wrapped it; the high word gets the addend's high word plus that carry, which is 0 for nearly
+// every small addend of either sign, so the second atomic is rare.  Exact and order-independent like the 64-bit add it replaces.
+__device__ __forceinline__ void fx_add(long long* slot, long long x) {
+    if (x == 0) return;
+    unsigned int* w = reinterpret_cast<unsigned int*>(slot);
+    const unsigned int lo = (unsigned int)x, hi = (unsigned int)((unsigned long long)x >> 32);
+    const unsigned int old = atomicAdd(w, lo);
+    const unsigned int h = hi + ((old + lo < old) ? 1u : 0u);
+    if (h) atomicAdd(w + 1, h);
+}
 // ---- 1 -> h -> 1 Softplus MLP on a COMPACT domain as a cubic table --------------------------------
 // The check-phase MLP of decoder_v2_4 (quantum/decoder_v2_4.py:257, `self.mlp(aggr_out[:, 0])`) is a
 // smooth scalar function f(x) = b2 + sum_k w2_k softplus(w1_k x + b1_k) of ONE variable whose argument

@@ -227,12 +227,20 @@ int gd_pipeline_wait(gd_pipeline* p, int32_t ticket);
 int gd_pipeline_drain(gd_pipeline* p);   /* wait for every batch submitted so far */
 
 /* ---- training (BASELINE config 4): forward that also stashes the per-iteration activations, and
- *      the hand-written backward (replaces autograd through the loop, decoder_v2_4.py:334-340).
- *      GD_PROG_V2_4 only.  stash_dev holds gd_stash_floats() floats: [(iters+1)][2][E][B].
- *      gd_decode_bwd takes dL/dlogit [B,V] (prob = sigmoid(-logit), so dL/dlogit = -dL/dprob *
- *      prob * (1 - prob)) and writes (accumulate == 0) or adds (accumulate != 0) dL/dweights in the
- *      packed order of gd_model.  workspace_dev: gd_bwd_workspace_floats() floats of per-warp
- *      partial sums, reduced in a fixed order -> bit-reproducible gradients. ---- */
+ *      the hand-written backward (replaces autograd through the loop, decoder_v2_4.py:334-340,
+ *      CGNNI.py:314-329).  Programs: GD_PROG_V2_4 and GD_PROG_CGNNI.  stash_dev holds
+ *      gd_stash_floats() floats:
+ *        GD_PROG_V2_4 : [(iters+1)][2][E][B] (+ a header of the table kernel, gd_lean.cuh);
+ *        GD_PROG_CGNNI: [iters][E][B], m after every iteration (the backward recomputes the rest).
+ *      GD_PROG_CGNNI trains on the node-owner kernel only: graphs in another edge order than the canonical
+ *      variable-sorted one, and codes whose edge state does not fit shared memory, return GD_ERR_UNSUPPORTED.
+ *      gd_decode_bwd takes dL/dlogit [B,V], the gradient w.r.t. the logit BEFORE the clamp the classical
+ *      programs apply (prob = sigmoid(-logit), so dL/dlogit = -dL/dprob * prob * (1 - prob); for CGNNI with
+ *      prob = clamp(s, 1e-7, 1-1e-7), s = sigmoid(-logit): -dL/dprob * s * (1 - s) where 1e-7 <= s <= 1-1e-7,
+ *      else 0) and writes (accumulate == 0) or adds (accumulate != 0) dL/dweights in the packed order of
+ *      gd_model.  workspace_dev: gd_bwd_workspace_floats() floats (8-byte aligned) of per-warp partial sums
+ *      (GD_PROG_V2_4) or per-CTA fixed-point bins (GD_PROG_CGNNI), reduced in a fixed order ->
+ *      bit-reproducible gradients; gd_bwd_workspace_floats returns -1 for other programs. ---- */
 int64_t gd_stash_floats(const gd_graph* g, const gd_model* model, int64_t B);
 int gd_decode_fwd_train(const gd_graph* g, const gd_model* model, const float* weights_dev,
                         const float* x_dev, float* prob_dev, float* logit_dev, float* stash_dev,
