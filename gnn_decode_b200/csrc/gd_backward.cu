@@ -17,8 +17,7 @@
 #include "gd_common.cuh"
 #include "gd_math.cuh"
 #include "gd_options.cuh"
-#include "gd_lean.cuh"
-#include "gd_light.cuh"
+#include "gd_decode.cuh"
 #include <stdlib.h>
 #include <string.h>
 
@@ -590,44 +589,33 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
         return GD_OK;
     }
     GD_CHECK_ARG(weights_dev && x_dev && stash_dev && grad_logit_dev && workspace_dev, "gd_decode_bwd: NULL buffer");
-    if (model->program == GD_PROG_CGNNI) {
-        int prev = 0;
-        GD_CUDA(cudaGetDevice(&prev));
-        if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
-        const int rc = gd::light_backward(g, model, weights_dev, x_dev, stash_dev, grad_logit_dev, grad_weights_dev, workspace_dev,
-                                          accumulate, B, st);
-        if (prev != g->device) cudaSetDevice(prev);
-        return rc;
-    }
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    int rc = gd::route_decode(g, model, B, gd::Use::TrainBwd, &r);
+    if (rc != GD_OK) return rc;
+    if (r.family == gd::Family::Light)
+        return gd::light_backward(g, model, weights_dev, x_dev, stash_dev, grad_logit_dev, grad_weights_dev, workspace_dev,
+                                  accumulate, B, st);
     gd::BwdPlan pl;
-    int rc = gd::plan_bwd(g, model, B, &pl);
+    rc = gd::plan_bwd(g, model, B, &pl);
     if (rc != GD_OK) return rc;
     pl.p.x = x_dev; pl.p.stash = stash_dev; pl.p.grad_logit = grad_logit_dev; pl.p.weights = weights_dev;
     pl.p.partials = workspace_dev;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
-    // decoder_v2_4 on surface / toric codes: when the table forward wrote the stash (its header says so, on the device), the
-    // table backward produces the gradient and the two kernels below return at once; otherwise the other way round
-    {
+    if (r.family == gd::Family::Lean) {
+        // decoder_v2_4 on surface / toric codes: when the table forward wrote the stash (its header says so, on the device), the
+        // table backward produces the gradient and the two kernels below return at once; otherwise the other way round
         float* bins = workspace_dev + (((int64_t)pl.n_rows * pl.p.np_pad + 3) & ~(int64_t)3);   // 16-byte aligned (64-bit atomics)
-        const int lrc = gd::lean_backward(const_cast<gd_graph*>(g), model, weights_dev, x_dev, stash_dev, grad_logit_dev,
-                                          grad_weights_dev, bins, accumulate, B, st);
-        if (lrc > 0) {
-            if (prev != g->device) cudaSetDevice(prev);
-            return lrc;
-        }
-        if (lrc == 0) pl.p.run_flag = &gd::lean_train_hdr(const_cast<float*>(stash_dev), g, model, B)->old_count;
+        rc = gd::lean_backward(const_cast<gd_graph*>(g), model, r.lean[0], weights_dev, x_dev, stash_dev, grad_logit_dev,
+                               grad_weights_dev, bins, accumulate, B, st);
+        if (rc != GD_OK) return rc;
+        pl.p.run_flag = &gd::lean_train_hdr(const_cast<float*>(stash_dev), g, model, B)->old_count;
     }
-    cudaError_t e = cudaFuncSetAttribute(gd::decode_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem);
-    if (e == cudaSuccess) {
-        e = gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::decode_bwd_kernel, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, pl.p);
-    }
-    if (e == cudaSuccess) {
-        e = gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::reduce_partials_kernel, dim3((n_params + 127) / 128), dim3(128), 0, st, workspace_dev,
-                              pl.n_rows, pl.p.np_pad, n_params, grad_weights_dev, accumulate ? 1 : 0, pl.p.run_flag);
-    }
-    if (prev != g->device) cudaSetDevice(prev);
-    GD_CUDA(e);
+    GD_CUDA(cudaFuncSetAttribute(gd::decode_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
+    GD_CUDA(gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::decode_bwd_kernel, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem,
+                              st, pl.p));
+    GD_CUDA(gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::reduce_partials_kernel, dim3((n_params + 127) / 128), dim3(128), 0,
+                              st, workspace_dev, pl.n_rows, pl.p.np_pad, n_params, grad_weights_dev, accumulate ? 1 : 0,
+                              pl.p.run_flag));
     return GD_OK;
 }

@@ -73,9 +73,8 @@ __global__ void __launch_bounds__(1024) lds_bench_kernel(float* out, int iters) 
 // result[1] = milliseconds of the timed launch.
 extern "C" int gd_microbench(int32_t kind, int32_t iters, int device, double* result) {
     GD_CHECK_ARG(result && kind >= 0 && kind <= 7 && iters > 0, "gd_microbench: bad argument");
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    GD_CUDA(cudaSetDevice(device));
+    gd::DeviceGuard dg(device);
+    GD_CUDA(dg.status());
     cudaDeviceProp prop;
     GD_CUDA(cudaGetDeviceProperties(&prop, device));
     float* out = nullptr;
@@ -105,7 +104,6 @@ extern "C" int gd_microbench(int32_t kind, int32_t iters, int device, double* re
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     cudaFree(out);
-    cudaSetDevice(prev);
     GD_CUDA(e);
     // kind 7: units = 128-byte shared-memory wavefronts (a warp-wide 128-bit load is 4 of them)
     const double units = (double)grid * threads * (double)iters * 8.0 * (kind == 7 ? 4.0 / 32.0 : 1.0);

@@ -32,6 +32,30 @@ void set_error(const char* fmt, ...);
         }                                                                                    \
     } while (0)
 
+// Makes `device` current for the guard's scope and gives the caller's device back when the scope ends, on every return
+// path.  The library's entry points switch only through this guard.
+class DeviceGuard {
+public:
+    explicit DeviceGuard(int device) {
+        err_ = cudaGetDevice(&prev_);
+        if (err_ == cudaSuccess && prev_ != device) {
+            err_ = cudaSetDevice(device);
+            switched_ = err_ == cudaSuccess;
+        }
+    }
+    ~DeviceGuard() {
+        if (switched_) cudaSetDevice(prev_);
+    }
+    DeviceGuard(const DeviceGuard&) = delete;
+    DeviceGuard& operator=(const DeviceGuard&) = delete;
+    cudaError_t status() const { return err_; }   // of the switch: check it with GD_CUDA before using the device
+
+private:
+    int prev_ = 0;
+    bool switched_ = false;
+    cudaError_t err_ = cudaSuccess;
+};
+
 // Device blob layout (int32 words): all tables of one Tanner graph, uploaded once.
 struct GraphTables {
     const int32_t* edge_var;   // [E]   variable endpoint of edge e

@@ -33,41 +33,6 @@ namespace gd {
 
 constexpr int kMaxThreads = 1024;   // largest CTA; kernels are instantiated for 512 (<=128 regs) and 1024 (<=64 regs)
 
-struct DecodeParams {
-    const float* x;
-    float* prob;
-    float* logit;
-    uint8_t* hard;
-    const float* weights;
-    float* stash;           // training only: [(T+1)][2][E][B] = per-iteration (m_it, a_it), final m in slot T
-    GraphTables tb;
-    long long B;
-    int T, V, C, E, N;
-    int tile, R, hid, hp, n_tiles, maxvc, all_iters, wslot;
-    int n_vact;             // edges on variables of degree >= 2 (GraphTables::vlist)
-    int vdirect, cdirect;   // V2_4: max variable degree <= 2 / max check degree <= 4 -> sibling messages are read directly
-    int scratch_bytes;      // bytes of shared memory from off_x to the end (prologue scratch)
-    int rtab_n, off_rtab;   // V2_4: intervals of the read-out MLP's cubic table (0 = direct) and its smem offset
-    int ctab_n, off_ctab;   // V2_4: intervals of the check-phase cubic table (0 = direct evaluation) and its smem offset
-    float ctab_R;           // half-width of its domain: max check degree - 1
-    // V2_4: cubic tables of the variable-phase MLP's sections f(ext, prior = const), one per distinct prior value a CTA
-    // meets (inputs made like the reference's gen_syn carry one prior per syndrome, drawn from a short list)
-    int vtab_n, vtab_k, off_vtab, off_vmeta;
-    int off_w, off_tab, off_x, off_node, off_m, off_t;
-    // gated launch (gd_decode_host, see Gate in gd_decode.cuh); all NULL / 0 otherwise
-    const unsigned int* gate_in;
-    unsigned int* gate_out;
-    int* gate_err;
-    unsigned int gate_epoch;
-    int gate_chunk_tiles;
-    // deferred pass behind the check-owner table kernel (gd_lean.cu): decode only the listed syndromes (*defer_count > 0),
-    // the whole batch (-1) or nothing (0); all NULL otherwise
-    const int* defer_count;
-    const int* defer_idx;
-    uint32_t* hard_bits;    // optional packed hard decisions [B][ceil(V/32)]
-    float* aux_prob; float* aux_logit;   // GD_PROG_V3_0: the check-node read-out [B][C]
-};
-
 // ---------------- PTX helpers: mbarrier + bulk async copy (TMA 1-D) ----------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return (uint32_t)__cvta_generic_to_shared(p);
@@ -932,11 +897,6 @@ __global__ void __launch_bounds__(MAXT, 1) decode_kernel(const DecodeParams p) {
 }
 
 // ---------------------------------------------------------------------------------------------
-struct DecodePlan {
-    DecodeParams p;
-    int threads, grid, smem, resident, cps, eb, npad;
-};
-
 static int align_up(int x, int a) { return (x + a - 1) / a * a; }
 
 // A (tile, R, EB) candidate of the geometry search with its model score
@@ -974,6 +934,10 @@ static int plan_decode(const gd_graph* g, const gd_model* m, int64_t B, DecodePl
     out->eb = 4;
     p.B = B; p.T = m->iters; p.V = V; p.C = C; p.E = (int)E64; p.N = N; p.hid = hid; p.hp = hp; p.maxvc = maxvc;
     p.tb = g->t;
+    p.all_iters = (m->flags & GD_FLAG_ALL_ITERS) ? 1 : 0;
+    p.n_vact = opt_on(OPT_NO_VSKIP) ? (int)g->E : g->n_vact;
+    p.vdirect = (g->max_var_deg <= 2 && !opt_on(OPT_NO_DIRECT)) ? 1 : 0;
+    p.cdirect = (g->max_chk_deg <= 4 && !opt_on(OPT_NO_DIRECT)) ? 1 : 0;
 
     // CTAs per SM: two half-size CTAs let one CTA's light phases (node sums, table look-ups, barriers) overlap the
     // other's MUFU-bound variable phase
@@ -1140,20 +1104,176 @@ static int launch_decode(const DecodePlan& pl, cudaStream_t st) {
     return GD_OK;
 }
 
+int edge_decode(const gd_graph* g, const gd_model* model, DecodePlan pl, const DecodeIO& io, cudaStream_t st, const Gate* gate,
+                const DeferList* dl) {
+    pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
+    pl.p.stash = io.stash; pl.p.hard_bits = io.hard_bits;
+    pl.p.aux_prob = io.aux_prob; pl.p.aux_logit = io.aux_logit;
+    if (dl) { pl.p.defer_count = dl->count; pl.p.defer_idx = dl->idx; }
+    if (gate) {
+        pl.p.gate_in = gate->in_flags; pl.p.gate_out = gate->out_counts; pl.p.gate_err = gate->err;
+        pl.p.gate_epoch = gate->epoch; pl.p.gate_chunk_tiles = gate->chunk_tiles;
+    }
+    switch (model->program) {
+        case GD_PROG_CGNNI: return launch_decode<GD_PROG_CGNNI>(pl, st);
+        case GD_PROG_QGNNI: return launch_decode<GD_PROG_QGNNI>(pl, st);
+        case GD_PROG_V2_4: return launch_decode<GD_PROG_V2_4>(pl, st);
+        case GD_PROG_BP_QUANTUM: return launch_decode<GD_PROG_BP_QUANTUM>(pl, st);
+        case GD_PROG_NEURAL_BP: return launch_decode<GD_PROG_NEURAL_BP>(pl, st);
+        case GD_PROG_GRU_CA: return launch_decode<GD_PROG_GRU_CA>(pl, st);
+        case GD_PROG_V3_0: return launch_decode<GD_PROG_V3_0>(pl, st);
+        case GD_PROG_V1_2_2: return launch_decode<GD_PROG_V1_2_2>(pl, st);
+        case GD_PROG_V2_4_1: return launch_decode<GD_PROG_V2_4_1>(pl, st);
+        default: return launch_decode<GD_PROG_BP_CLASSICAL>(pl, st);
+    }
+}
+
+int route_decode(const gd_graph* gc, const gd_model* m, int64_t B, Use use, Route* r) {
+    gd_graph* g = const_cast<gd_graph*>(gc);
+    r->lean.clear();
+    if (use == Use::Train || use == Use::TrainBwd) {     // (the callers take GD_PROG_V2_4 and GD_PROG_CGNNI only)
+        if (m->program == GD_PROG_CGNNI) {
+            // the node-owner kernel is the only one with a CGNNI backward; that backward plans its own layout
+            r->family = Family::Light;
+            if (use == Use::TrainBwd) return GD_OK;
+            plan_light(g, m, B, &r->light, true);
+            if (!r->light.ok) {
+                set_error("gd_decode_fwd_train: CGNNI training needs the node-owner kernel: %s", r->light.why);
+                return GD_ERR_UNSUPPORTED;
+            }
+            return GD_OK;
+        }
+        // decoder_v2_4: the table kernel over the whole graph when it plans, and the edge-owner pair in any case -- the header
+        // at the end of the stash tells the device which of them runs (gd_lean.cuh).  The backward plans the table kernel as
+        // the forward did; the edge-owner backward has its own planner (gd_backward.cu).
+        if (use == Use::Train) {
+            const int rc = plan_decode(g, m, B, &r->edge);
+            if (rc != GD_OK) return rc;
+            if (!r->edge.resident) {
+                set_error("gd_decode_fwd_train: code too large for the resident kernel (training needs it)");
+                return GD_ERR_UNSUPPORTED;
+            }
+        }
+        r->family = lean_plan(g, m, B, &r->lean, true) ? Family::Lean : Family::EdgeOwner;
+        return GD_OK;
+    }
+    if (m->program == GD_PROG_V2_4_1) {
+        bool all4 = true;
+        for (int c = 0; c < g->C && all4; ++c) all4 = g->h_chk_ptr[c + 1] - g->h_chk_ptr[c] == 4;
+        GD_CHECK_ARG(all4, "gd_decode_fwd: GD_PROG_V2_4_1 needs every check to have exactly 4 edges (decoder_v2_4_1.py:211-236)");
+    }
+    GD_CHECK_ARG(m->program != GD_PROG_NEURAL_BP || m->hidden == g->E,
+                 "gd_decode_fwd: GD_PROG_NEURAL_BP needs model.hidden == E (%lld per-edge weights), got %d", (long long)g->E,
+                 m->hidden);
+    // Residency first: a code whose edge state does not fit shared memory (or GD_FORCE_STREAMED) takes a streamed kernel
+    // and nothing else.  Every resident route keeps this plan: it is the table kernel's deferred pass.
+    const int rc = plan_decode(g, m, B, &r->edge);
+    if (rc != GD_OK) return rc;
+    if (!r->edge.resident) {
+        if (use == Use::Packed) {
+            set_error("gd_decode_packed_fwd: this code's edge state does not fit shared memory (streamed path has no packed form)");
+            return GD_ERR_UNSUPPORTED;
+        }
+        if (m->program == GD_PROG_NEURAL_BP || m->program == GD_PROG_GRU_CA || m->program == GD_PROG_V3_0 ||
+            m->program == GD_PROG_V1_2_2 || m->program == GD_PROG_V2_4_1) {
+            set_error("gd_decode_fwd: program %d has a resident kernel only and this code's edge state does not fit "
+                      "shared memory", m->program);
+            return GD_ERR_UNSUPPORTED;
+        }
+        plan_streamed_tma(g, m, B, &r->tma);
+        if (r->tma.ok) {
+            r->family = Family::StreamedTma;
+            return GD_OK;
+        }
+        r->family = Family::Streamed;
+        return plan_streamed(g, m, B, &r->streamed);
+    }
+    if (lean_plan(g, m, B, &r->lean)) {
+        r->family = Family::Lean;                        // decoder_v2_4 on surface / toric codes
+        return GD_OK;
+    }
+    plan_light(g, m, B, &r->light);                      // the light programs, when the batch fills the GPU
+    r->family = r->light.ok ? Family::Light : Family::EdgeOwner;
+    return GD_OK;
+}
+
+gd_launch_info route_launch_info(const Route& r) {
+    gd_launch_info li;
+    memset(&li, 0, sizeof(li));
+    li.resident = 1;
+    switch (r.family) {
+        case Family::Lean: {
+            const LeanPlan& pl = r.lean[0];              // (parts: the first launch's geometry; tiles of all launches)
+            li.tile = 32 * pl.p.G; li.threads = pl.threads; li.grid = pl.grid; li.smem_bytes = pl.smem;
+            li.n_tiles = (int)r.lean.size() * ((pl.n_tiles + pl.p.G - 1) / pl.p.G);
+        } break;
+        case Family::Light:
+            li.tile = r.light.p.tile; li.threads = r.light.threads; li.grid = r.light.grid; li.smem_bytes = r.light.smem;
+            li.n_tiles = r.light.p.n_tiles;
+            break;
+        case Family::EdgeOwner:
+            li.tile = r.edge.p.tile; li.threads = r.edge.threads; li.grid = r.edge.grid; li.smem_bytes = r.edge.smem;
+            li.n_tiles = r.edge.p.n_tiles;
+            break;
+        case Family::StreamedTma:
+            li.tile = r.tma.p.tile; li.threads = r.tma.threads; li.grid = r.tma.grid; li.smem_bytes = r.tma.smem;
+            li.resident = 0; li.n_tiles = r.tma.p.n_tiles;
+            break;
+        case Family::Streamed:
+            li.tile = r.streamed.p.tile; li.threads = r.streamed.threads; li.grid = r.streamed.grid;
+            li.smem_bytes = r.streamed.smem; li.resident = 0; li.n_tiles = r.streamed.p.n_tiles;
+            break;
+    }
+    return li;
+}
+
+namespace {
+struct PackedRun {
+    const gd_graph* g; const gd_model* model; const DecodePlan* plan; const DecodeIO* io; cudaStream_t st;
+};
+int packed_run(void* ctx, const float* x_dev) {
+    const PackedRun* r = static_cast<const PackedRun*>(ctx);
+    DecodeIO io = *r->io;
+    io.x = x_dev;
+    return edge_decode(r->g, r->model, *r->plan, io, r->st);
+}
+}  // namespace
+
+int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const DecodeIO& io, int64_t B, cudaStream_t st,
+                  const Gate* gate) {
+    switch (r.family) {
+        case Family::Lean: {
+            bool no_resources = false;
+            const int rc = lean_decode(g, model, r.lean, r.edge, io, B, st, &no_resources);
+            if (!no_resources) return rc;
+            // The one decline only a launch can discover: the table kernel got no memory pool or table set on this device.
+            // The edge-owner kernel decodes the whole batch instead.
+            break;
+        }
+        case Family::Light: return light_decode(r.light, model, io, st, gate);
+        case Family::StreamedTma: return streamed_tma_decode(g, r.tma, model, io, st);
+        case Family::Streamed: return streamed_decode(g, r.streamed, model, io, st);
+        case Family::EdgeOwner: break;
+    }
+    if (!io.x) {             // packed inputs: expand them for the edge-owner kernel
+        PackedRun run{g, model, &r.edge, &io, st};
+        return packed_via_unpack(g, io.prior, io.synd, B, st, packed_run, &run);
+    }
+    return edge_decode(g, model, r.edge, io, st, gate);
+}
+
 }  // namespace gd
 
 extern "C" int gd_decode_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out) {
     GD_CHECK_ARG(g && out, "gd_decode_launch_info: NULL argument");
     GD_CHECK_ARG(gd_model_valid(model), "gd_decode_launch_info: invalid model");
     GD_CHECK_ARG(B > 0, "gd_decode_launch_info: B must be positive");
-    gd::DecodePlan pl;
-    int rc = gd::plan_decode(g, model, B, &pl);
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    const int rc = gd::route_decode(g, model, B, gd::Use::Infer, &r);
     if (rc != GD_OK) return rc;
-    if (!pl.resident) return gd::streamed_launch_info(g, model, B, out);
-    if (gd::lean_launch_info(g, model, B, out)) return GD_OK;       // check-owner table kernel (decoder_v2_4, surface / toric codes)
-    if (gd::light_launch_info(g, model, B, out)) return GD_OK;      // node-owner kernel for the light programs
-    out->tile = pl.p.tile; out->threads = pl.threads; out->grid = pl.grid; out->smem_bytes = pl.smem;
-    out->resident = pl.resident; out->n_tiles = pl.p.n_tiles;
+    *out = gd::route_launch_info(r);
     return GD_OK;
 }
 
@@ -1161,42 +1281,45 @@ extern "C" int gd_decode_tables_info(const gd_graph* g, const gd_model* model, i
     GD_CHECK_ARG(g && out4, "gd_decode_tables_info: NULL argument");
     GD_CHECK_ARG(gd_model_valid(model) && B > 0, "gd_decode_tables_info: invalid model / B");
     out4[0] = out4[1] = out4[2] = out4[3] = 0;
-    gd::DecodePlan pl;
-    gd_launch_info probe;
-    int rc = gd::plan_decode(g, model, B, &pl);
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    const int rc = gd::route_decode(g, model, B, gd::Use::Infer, &r);
     if (rc != GD_OK) return rc;
-    if (!pl.resident || gd::light_launch_info(g, model, B, &probe)) return GD_OK;
-    out4[0] = pl.p.ctab_n; out4[1] = pl.p.rtab_n; out4[2] = pl.p.vtab_n; out4[3] = pl.p.vtab_k;
+    if (r.family != gd::Family::Lean && r.family != gd::Family::EdgeOwner) return GD_OK;
+    const gd::DecodeParams& p = r.edge.p;        // the edge-owner kernel's tables (the table kernel's deferred pass)
+    out4[0] = p.ctab_n; out4[1] = p.rtab_n; out4[2] = p.vtab_n; out4[3] = p.vtab_k;
     return GD_OK;
 }
 
-static int decode_fwd_impl(const gd_graph* gc, const gd_model* model, const float* weights_dev, const float* x_dev,
-                           float* prob_dev, float* logit_dev, uint8_t* hard_dev, float* stash_dev, int64_t B,
-                           void* stream, const gd::Gate* gate = nullptr, const gd::DeferList* dl = nullptr,
-                           uint32_t* hard_bits_dev = nullptr, float* aux_prob_dev = nullptr, float* aux_logit_dev = nullptr);
-
-bool gd::gated_plan(const gd_graph* g, const gd_model* model, int64_t B, int* tile, int* n_tiles) {
-    gd::DecodePlan pl;
-    gd_launch_info probe;
-    if (model->flags != 0 || gd::plan_decode(g, model, B, &pl) != GD_OK || !pl.resident) return false;
-    if (gd::lean_launch_info(g, model, B, &probe)) return false;   // the check-owner table kernel is launched per chunk
-    if (gd::light_launch_info(g, model, B, &probe)) {     // node-owner kernel: gated too
-        *tile = probe.tile; *n_tiles = probe.n_tiles;
-        return true;
-    }
-    *tile = pl.p.tile; *n_tiles = pl.p.n_tiles;
-    return true;
-}
-
-int gd::decode_fwd_gated(const gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                         uint8_t* hard_dev, int64_t B, cudaStream_t st, const gd::Gate& gate) {
-    return decode_fwd_impl(g, model, weights_dev, x_dev, prob_dev, nullptr, hard_dev, nullptr, B, (void*)st, &gate);
+// Argument checks, then the route and its launch on the graph's device.
+static int decode_fwd_impl(const gd_graph* gc, const gd_model* model, const gd::DecodeIO& io, int64_t B, void* stream,
+                           gd::Use use = gd::Use::Infer) {
+    gd_graph* g = const_cast<gd_graph*>(gc);
+    GD_CHECK_ARG(g != nullptr, "gd_decode_fwd: graph is NULL");
+    GD_CHECK_ARG(gd_model_valid(model), "gd_decode_fwd: invalid model (program=%d hidden=%d iters=%d)",
+                 model ? model->program : -1, model ? model->hidden : -1, model ? model->iters : -1);
+    GD_CHECK_ARG(B >= 0 && B < ((int64_t)1 << 31), "gd_decode_fwd: B=%lld out of range", (long long)B);
+    if (B == 0) return GD_OK;  // empty batch: nothing to do (the reference would crash; we return cleanly)
+    GD_CHECK_ARG(io.x != nullptr, "gd_decode_fwd: x is NULL");
+    GD_CHECK_ARG(gd_weights_size(model) == 0 || io.weights != nullptr, "gd_decode_fwd: weights is NULL");
+    GD_CHECK_ARG(((uintptr_t)io.x & 15) == 0, "gd_decode_fwd: x must be 16-byte aligned");
+    GD_CHECK_ARG(((uintptr_t)io.prob & 15) == 0 && ((uintptr_t)io.logit & 15) == 0 && ((uintptr_t)io.hard & 3) == 0,
+                 "gd_decode_fwd: outputs must be 16-byte (prob, logit) / 4-byte (hard) aligned");
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    const int rc = gd::route_decode(g, model, B, use, &r);
+    if (rc != GD_OK) return rc;
+    return gd::decode_routed(g, model, r, io, B, (cudaStream_t)stream);
 }
 
 extern "C" int gd_decode_fwd(const gd_graph* gc, const gd_model* model, const float* weights_dev,
                              const float* x_dev, float* prob_dev, float* logit_dev, uint8_t* hard_dev, int64_t B,
                              void* stream) {
-    return decode_fwd_impl(gc, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, nullptr, B, stream);
+    gd::DecodeIO io{};
+    io.weights = weights_dev; io.x = x_dev; io.prob = prob_dev; io.logit = logit_dev; io.hard = hard_dev;
+    return decode_fwd_impl(gc, model, io, B, stream);
 }
 
 extern "C" int gd_decode_fwd_aux(const gd_graph* gc, const gd_model* model, const float* weights_dev, const float* x_dev,
@@ -1206,22 +1329,14 @@ extern "C" int gd_decode_fwd_aux(const gd_graph* gc, const gd_model* model, cons
         gd::set_error("gd_decode_fwd_aux: program %d has no second read-out (GD_PROG_V3_0 only)", model ? model->program : -1);
         return GD_ERR_UNSUPPORTED;
     }
-    return decode_fwd_impl(gc, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, nullptr, B, stream, nullptr, nullptr, nullptr,
-                           aux_prob_dev, aux_logit_dev);
+    gd::DecodeIO io{};
+    io.weights = weights_dev; io.x = x_dev; io.prob = prob_dev; io.logit = logit_dev; io.hard = hard_dev;
+    io.aux_prob = aux_prob_dev; io.aux_logit = aux_logit_dev;
+    return decode_fwd_impl(gc, model, io, B, stream);
 }
 
 // ---- packed form of the same decode (include/gnn_decode.h): what the reference's x actually carries per syndrome is ONE
 // prior value and C check signs (gen_syn, quantum/error_generate.py:258, 270-276) ----
-namespace {
-struct PackedRun {
-    const gd_graph* g; const gd_model* model; const float* w; float* prob; uint32_t* bits; int64_t B; void* stream;
-};
-int packed_run(void* ctx, const float* x_dev) {
-    const PackedRun* r = static_cast<const PackedRun*>(ctx);
-    return decode_fwd_impl(r->g, r->model, r->w, x_dev, r->prob, nullptr, nullptr, nullptr, r->B, r->stream, nullptr, nullptr, r->bits);
-}
-}  // namespace
-
 extern "C" int gd_decode_packed_fwd(const gd_graph* gc, const gd_model* model, const float* weights_dev, const float* prior_dev,
                                     const uint32_t* synd_dev, float* prob_dev, uint32_t* hard_bits_dev, int64_t B, void* stream) {
     gd_graph* g = const_cast<gd_graph*>(gc);
@@ -1238,25 +1353,14 @@ extern "C" int gd_decode_packed_fwd(const gd_graph* gc, const gd_model* model, c
         gd::set_error("gd_decode_packed_fwd: packed inputs are implemented for GD_PROG_V2_4 only");
         return GD_ERR_UNSUPPORTED;
     }
-    cudaStream_t st = (cudaStream_t)stream;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
-    int rc = gd::lean_decode(g, model, weights_dev, nullptr, prior_dev, synd_dev, prob_dev, nullptr, nullptr, hard_bits_dev, B, st);
-    if (rc < 0) {                // not a surface / toric code: expand and take the edge-owner kernel
-        gd_launch_info li;
-        rc = gd_decode_launch_info(g, model, B, &li);
-        if (rc == GD_OK && !li.resident) {
-            gd::set_error("gd_decode_packed_fwd: this code's edge state does not fit shared memory (streamed path has no packed form)");
-            rc = GD_ERR_UNSUPPORTED;
-        }
-        if (rc == GD_OK) {
-            PackedRun r{g, model, weights_dev, prob_dev, hard_bits_dev, B, stream};
-            rc = gd::packed_via_unpack(g, prior_dev, synd_dev, B, st, packed_run, &r);
-        }
-    }
-    if (prev != g->device) cudaSetDevice(prev);
-    return rc;
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    const int rc = gd::route_decode(g, model, B, gd::Use::Packed, &r);
+    if (rc != GD_OK) return rc;
+    gd::DecodeIO io{};
+    io.weights = weights_dev; io.prior = prior_dev; io.synd = synd_dev; io.prob = prob_dev; io.hard_bits = hard_bits_dev;
+    return gd::decode_routed(g, model, r, io, B, (cudaStream_t)stream);
 }
 
 extern "C" int64_t gd_stash_floats(const gd_graph* g, const gd_model* model, int64_t B) {
@@ -1274,123 +1378,10 @@ extern "C" int gd_decode_fwd_train(const gd_graph* gc, const gd_model* model, co
     GD_CHECK_ARG(model && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI),
                  "gd_decode_fwd_train: only GD_PROG_V2_4 and GD_PROG_CGNNI have a backward kernel");
     GD_CHECK_ARG(stash_dev != nullptr || B == 0, "gd_decode_fwd_train: stash is NULL");
-    gd_launch_info li;
-    if (B > 0 && model->program == GD_PROG_V2_4) {      // CGNNI: the node-owner kernel reports what it cannot take
-        int rc = gd_decode_launch_info(gc, model, B, &li);
-        if (rc != GD_OK) return rc;
-        if (!li.resident) {
-            gd::set_error("gd_decode_fwd_train: code too large for the resident kernel (training needs it)");
-            return GD_ERR_UNSUPPORTED;
-        }
-    }
-    return decode_fwd_impl(gc, model, weights_dev, x_dev, prob_dev, logit_dev, nullptr, stash_dev, B, stream);
+    gd::DecodeIO io{};
+    io.weights = weights_dev; io.x = x_dev; io.prob = prob_dev; io.logit = logit_dev; io.stash = stash_dev;
+    return decode_fwd_impl(gc, model, io, B, stream, gd::Use::Train);
 }
-
-int gd::decode_fwd_deferred(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                            float* logit_dev, uint8_t* hard_dev, uint32_t* hard_bits_dev, int64_t B, cudaStream_t st,
-                            const gd::DeferList& dl, float* stash_dev) {
-    return decode_fwd_impl(g, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, stash_dev, B, (void*)st, nullptr, &dl,
-                           hard_bits_dev);
-}
-
-static int decode_fwd_impl(const gd_graph* gc, const gd_model* model, const float* weights_dev, const float* x_dev,
-                           float* prob_dev, float* logit_dev, uint8_t* hard_dev, float* stash_dev, int64_t B,
-                           void* stream, const gd::Gate* gate, const gd::DeferList* dl, uint32_t* hard_bits_dev, float* aux_prob_dev,
-                           float* aux_logit_dev) {
-    gd_graph* g = const_cast<gd_graph*>(gc);
-    GD_CHECK_ARG(g != nullptr, "gd_decode_fwd: graph is NULL");
-    GD_CHECK_ARG(gd_model_valid(model), "gd_decode_fwd: invalid model (program=%d hidden=%d iters=%d)",
-                 model ? model->program : -1, model ? model->hidden : -1, model ? model->iters : -1);
-    GD_CHECK_ARG(B >= 0 && B < ((int64_t)1 << 31), "gd_decode_fwd: B=%lld out of range", (long long)B);
-    if (B == 0) return GD_OK;  // empty batch: nothing to do (the reference would crash; we return cleanly)
-    GD_CHECK_ARG(x_dev != nullptr, "gd_decode_fwd: x is NULL");
-    GD_CHECK_ARG(gd_weights_size(model) == 0 || weights_dev != nullptr, "gd_decode_fwd: weights is NULL");
-    GD_CHECK_ARG(((uintptr_t)x_dev & 15) == 0, "gd_decode_fwd: x must be 16-byte aligned");
-    GD_CHECK_ARG(((uintptr_t)prob_dev & 15) == 0 && ((uintptr_t)logit_dev & 15) == 0 && ((uintptr_t)hard_dev & 3) == 0,
-                 "gd_decode_fwd: outputs must be 16-byte (prob, logit) / 4-byte (hard) aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
-    if (!gate && !dl) {
-        // decoder_v2_4 on surface / toric codes: the check-owner table kernel (gd_lean.cu); what it cannot serve comes back
-        // here through decode_fwd_deferred.  Training (stash_dev): the table kernel writes an m-only stash when it can serve
-        // EVERY row, else this kernel writes the full one; the header at the end of the stash says which (gd_lean.cuh).
-        const int lrc = gd::lean_decode(g, model, weights_dev, x_dev, nullptr, nullptr, prob_dev, logit_dev, hard_dev, hard_bits_dev,
-                                        B, st, stash_dev);
-        if (lrc >= 0) {
-            if (prev != g->device) cudaSetDevice(prev);
-            return lrc;
-        }
-    }
-    if (stash_dev && model->program == GD_PROG_CGNNI) {
-        // CGNNI training: the node-owner kernel with its stash (gd_backward_light.cu mirrors its mapping), or an error
-        const int lrc = gd::light_decode(g, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, B, st, nullptr, stash_dev);
-        if (prev != g->device) cudaSetDevice(prev);
-        return lrc;
-    }
-    gd::DecodePlan pl;
-    int rc = gd::plan_decode(g, model, B, &pl);
-    if (rc != GD_OK) {
-        if (prev != g->device) cudaSetDevice(prev);
-        return rc;
-    }
-    pl.p.x = x_dev; pl.p.prob = prob_dev; pl.p.logit = logit_dev; pl.p.hard = hard_dev; pl.p.weights = weights_dev;
-    pl.p.stash = stash_dev; pl.p.hard_bits = hard_bits_dev;
-    pl.p.aux_prob = aux_prob_dev; pl.p.aux_logit = aux_logit_dev;
-    if (dl) { pl.p.defer_count = dl->count; pl.p.defer_idx = dl->idx; }
-    if (gate) {
-        GD_CHECK_ARG(pl.resident && gate->chunk_tiles > 0, "gd_decode_host: gated launch needs the resident kernel");
-        pl.p.gate_in = gate->in_flags; pl.p.gate_out = gate->out_counts; pl.p.gate_err = gate->err;
-        pl.p.gate_epoch = gate->epoch; pl.p.gate_chunk_tiles = gate->chunk_tiles;
-    }
-    pl.p.all_iters = (model->flags & GD_FLAG_ALL_ITERS) ? 1 : 0;
-    pl.p.n_vact = gd::opt_on(gd::OPT_NO_VSKIP) ? (int)g->E : g->n_vact;
-    pl.p.vdirect = (g->max_var_deg <= 2 && !gd::opt_on(gd::OPT_NO_DIRECT)) ? 1 : 0;
-    pl.p.cdirect = (g->max_chk_deg <= 4 && !gd::opt_on(gd::OPT_NO_DIRECT)) ? 1 : 0;
-    if (model->program == GD_PROG_V2_4_1) {
-        bool all4 = true;
-        for (int c = 0; c < g->C && all4; ++c) all4 = g->h_chk_ptr[c + 1] - g->h_chk_ptr[c] == 4;
-        GD_CHECK_ARG(all4, "gd_decode_fwd: GD_PROG_V2_4_1 needs every check to have exactly 4 edges (decoder_v2_4_1.py:211-236)");
-    }
-    GD_CHECK_ARG(model->program != GD_PROG_NEURAL_BP || model->hidden == g->E,
-                 "gd_decode_fwd: GD_PROG_NEURAL_BP needs model.hidden == E (%lld per-edge weights), got %d",
-                 (long long)g->E, model->hidden);
-    if (!pl.resident && (model->program == GD_PROG_NEURAL_BP || model->program == GD_PROG_GRU_CA || model->program == GD_PROG_V3_0 ||
-                         model->program == GD_PROG_V1_2_2 || model->program == GD_PROG_V2_4_1)) {
-        gd::set_error("gd_decode_fwd: program %d has a resident kernel only and this code's edge state does not fit "
-                      "shared memory", model->program);
-        return GD_ERR_UNSUPPORTED;
-    }
-    if (!pl.resident) {
-        rc = gd::streamed_decode(g, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, B, st);
-        if (prev != g->device) cudaSetDevice(prev);
-        return rc;
-    }
-    if (!stash_dev && !dl) {
-        // light programs (CGNNI, QGNNI, sum-product): the node-owner kernel of gd_decode_light.cu
-        const int lrc = gd::light_decode(g, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, B, st, gate);
-        if (lrc >= 0) {
-            if (prev != g->device) cudaSetDevice(prev);
-            return lrc;
-        }
-    }
-    switch (model->program) {
-        case GD_PROG_CGNNI: rc = gd::launch_decode<GD_PROG_CGNNI>(pl, st); break;
-        case GD_PROG_QGNNI: rc = gd::launch_decode<GD_PROG_QGNNI>(pl, st); break;
-        case GD_PROG_V2_4: rc = gd::launch_decode<GD_PROG_V2_4>(pl, st); break;
-        case GD_PROG_BP_QUANTUM: rc = gd::launch_decode<GD_PROG_BP_QUANTUM>(pl, st); break;
-        case GD_PROG_NEURAL_BP: rc = gd::launch_decode<GD_PROG_NEURAL_BP>(pl, st); break;
-        case GD_PROG_GRU_CA: rc = gd::launch_decode<GD_PROG_GRU_CA>(pl, st); break;
-        case GD_PROG_V3_0: rc = gd::launch_decode<GD_PROG_V3_0>(pl, st); break;
-        case GD_PROG_V1_2_2: rc = gd::launch_decode<GD_PROG_V1_2_2>(pl, st); break;
-        case GD_PROG_V2_4_1: rc = gd::launch_decode<GD_PROG_V2_4_1>(pl, st); break;
-        default: rc = gd::launch_decode<GD_PROG_BP_CLASSICAL>(pl, st); break;
-    }
-    if (prev != g->device) cudaSetDevice(prev);
-    return rc;
-}
-
 
 // ---- geometry autotuner: measure, don't guess ------------------------------------------------------------------------
 // The (tile, R, EB) model above ranks hundreds of geometries; its top picks are usually within a few percent of each
@@ -1402,15 +1393,15 @@ extern "C" int gd_decode_autotune(const gd_graph* gc, const gd_model* model, con
     gd_graph* g = const_cast<gd_graph*>(gc);
     GD_CHECK_ARG(g != nullptr && gd_model_valid(model) && x_dev != nullptr && B > 0, "gd_decode_autotune: bad argument");
     GD_CHECK_ARG(gd_weights_size(model) == 0 || weights_dev != nullptr, "gd_decode_autotune: weights is NULL");
-    GD_CHECK_ARG(model->program != GD_PROG_NEURAL_BP || model->hidden == g->E, "gd_decode_autotune: NEURAL_BP needs hidden == E");
     cudaStream_t st = (cudaStream_t)stream;
-    gd_launch_info li;
-    int rc = gd_decode_launch_info(g, model, B, &li);
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    int rc = gd::route_decode(g, model, B, gd::Use::Infer, &r);
     if (rc != GD_OK) return rc;
-    if (chosen) *chosen = li;
-    // only the edge-owner resident kernel has a geometry to tune; the light / streamed kernels plan themselves
-    gd_launch_info probe;
-    if (!li.resident || gd::lean_launch_info(g, model, B, &probe) || gd::light_launch_info(g, model, B, &probe)) return GD_OK;
+    if (chosen) *chosen = gd::route_launch_info(r);
+    // only the edge-owner resident kernel has a geometry to tune; the other families plan themselves
+    if (r.family != gd::Family::EdgeOwner) return GD_OK;
     std::vector<gd::GeomCand> cands;
     gd::DecodePlan pl;
     rc = gd::plan_decode(g, model, B, &pl, nullptr, &cands);
@@ -1425,9 +1416,6 @@ extern "C" int gd_decode_autotune(const gd_graph* gc, const gd_model* model, con
         if (!dup) pick.push_back(c);
         if ((int)pick.size() >= K) break;
     }
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
     float* prob = nullptr;
     cudaError_t e = cudaMalloc((void**)&prob, (size_t)B * g->V * sizeof(float));
     cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -1470,7 +1458,6 @@ extern "C" int gd_decode_autotune(const gd_graph* gc, const gd_model* model, con
                 g->tuned[q].tile = best.tile; g->tuned[q].R = best.R; g->tuned[q].eb = best.eb;
             }
     }
-    if (prev != g->device) cudaSetDevice(prev);
     if (rc != GD_OK) return rc;
     GD_CUDA(e);
     if (chosen) gd_decode_launch_info(g, model, B, chosen);

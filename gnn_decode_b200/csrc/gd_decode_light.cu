@@ -650,47 +650,21 @@ void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out,
     out->why = nullptr;
 }
 
-bool light_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out) {
-    LightPlan pl;
-    plan_light(g, model, B, &pl);
-    if (!pl.ok) return false;
-    out->tile = pl.p.tile; out->threads = pl.threads; out->grid = pl.grid; out->smem_bytes = pl.smem;
-    out->resident = 1; out->n_tiles = pl.p.n_tiles;
-    return true;
-}
-
-// rc < 0: not applicable (the caller keeps the edge-owner kernel); otherwise a gd_status.
-int light_decode(const gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                 float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st, const Gate* gate, float* stash_dev) {
-    LightPlan pl;
-    plan_light(g, model, B, &pl, stash_dev != nullptr);
-    if (stash_dev) {   // CGNNI training: this kernel is the only one the backward mirrors
-        if (model->program != GD_PROG_CGNNI) {
-            set_error("gd_decode_fwd_train: program %d has no node-owner backward", model->program);
-            return GD_ERR_UNSUPPORTED;
-        }
-        if (!pl.ok) {
-            set_error("gd_decode_fwd_train: CGNNI training needs the node-owner kernel: %s", pl.why);
-            return GD_ERR_UNSUPPORTED;
-        }
-        pl.p.x = x_dev; pl.p.prob = prob_dev; pl.p.logit = logit_dev; pl.p.hard = hard_dev; pl.p.weights = weights_dev;
-        pl.p.stash = stash_dev;
-        void (*k)(const LightParams) = pl.npad == 16 ? decode_light_kernel<GD_PROG_CGNNI, 16, true> : decode_light_kernel<GD_PROG_CGNNI, 32, true>;
-        GD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
-        k<<<pl.grid, pl.threads, pl.smem, st>>>(pl.p);
-        GD_CUDA(cudaGetLastError());
-        return GD_OK;
-    }
-    if (!pl.ok) return -1;
+int light_decode(const LightPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st, const Gate* gate) {
+    LightPlan pl = plan;
+    pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
+    pl.p.stash = io.stash;
     if (gate) {
         pl.p.gate_in = gate->in_flags; pl.p.gate_out = gate->out_counts; pl.p.gate_err = gate->err;
         pl.p.gate_epoch = gate->epoch; pl.p.gate_chunk_tiles = gate->chunk_tiles;
     }
-    pl.p.x = x_dev; pl.p.prob = prob_dev; pl.p.logit = logit_dev; pl.p.hard = hard_dev; pl.p.weights = weights_dev;
     void (*k)(const LightParams);
     switch (model->program) {
         case GD_PROG_CGNNI:
-            k = pl.npad == 16 ? decode_light_kernel<GD_PROG_CGNNI, 16>
+            if (io.stash)   // training: the forward with stash that gd_backward_light.cu mirrors (always the piecewise-linear tables)
+                k = pl.npad == 16 ? decode_light_kernel<GD_PROG_CGNNI, 16, true> : decode_light_kernel<GD_PROG_CGNNI, 32, true>;
+            else
+                k = pl.npad == 16 ? decode_light_kernel<GD_PROG_CGNNI, 16>
                 : pl.npad == 32 ? decode_light_kernel<GD_PROG_CGNNI, 32> : decode_light_kernel<GD_PROG_CGNNI, 0>;
             break;
         case GD_PROG_QGNNI:

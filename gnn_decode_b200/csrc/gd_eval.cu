@@ -56,13 +56,11 @@ extern "C" int gd_eval_failures(const gd_graph* g, const uint8_t* logical_dev, i
     GD_CHECK_ARG(err_dev && hard_dev && counts_dev, "gd_eval_failures: NULL buffer");
     int64_t blocks = (B + 3) / 4;
     if (blocks > (int64_t)g->sm_count * 16) blocks = (int64_t)g->sm_count * 16;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     gd::eval_kernel<<<(int)blocks, 128, 0, (cudaStream_t)stream>>>(err_dev, hard_dev, logical_dev, K, g->t, B, g->V,
                                                                   g->C, counts_dev);
     cudaError_t e = cudaGetLastError();
-    if (prev != g->device) cudaSetDevice(prev);
     GD_CUDA(e);
     return GD_OK;
 }

@@ -113,19 +113,17 @@ extern "C" int gd_graph_create(const int64_t* ei, int64_t E, int32_t V, int32_t 
     put(g->h_edge_var, o_ev); put(g->h_edge_chk, o_ec); put(g->h_var_ptr, o_vp);
     put(g->h_var_edges, o_ve); put(g->h_chk_ptr, o_cp); put(g->h_chk_edges, o_ce); put(g->h_vlist, o_vl);
 
-    int prev = 0;
-    cudaError_t e1 = cudaGetDevice(&prev);
-    cudaError_t e2 = cudaSetDevice(device);
-    cudaError_t e3 = cudaMalloc((void**)&g->blob_dev, words * sizeof(int32_t));
-    cudaError_t e4 = e3 == cudaSuccess
-                         ? cudaMemcpy(g->blob_dev, blob.data(), words * sizeof(int32_t), cudaMemcpyHostToDevice)
-                         : e3;
+    cudaError_t e;
     cudaDeviceProp prop;
-    cudaError_t e5 = cudaGetDeviceProperties(&prop, device);
-    if (e1 == cudaSuccess) cudaSetDevice(prev);
-    if (e1 != cudaSuccess || e2 != cudaSuccess || e4 != cudaSuccess || e5 != cudaSuccess) {
-        cudaError_t bad = e1 != cudaSuccess ? e1 : e2 != cudaSuccess ? e2 : e4 != cudaSuccess ? e4 : e5;
-        gd::set_error("gd_graph_create: CUDA failure: %s", cudaGetErrorString(bad));
+    {
+        gd::DeviceGuard dg(device);
+        e = dg.status();
+        if (e == cudaSuccess) e = cudaMalloc((void**)&g->blob_dev, words * sizeof(int32_t));
+        if (e == cudaSuccess) e = cudaMemcpy(g->blob_dev, blob.data(), words * sizeof(int32_t), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, device);
+    }
+    if (e != cudaSuccess) {
+        gd::set_error("gd_graph_create: CUDA failure: %s", cudaGetErrorString(e));
         if (g->blob_dev) cudaFree(g->blob_dev);
         delete g;
         return GD_ERR_CUDA;
@@ -149,14 +147,13 @@ void gd_lean_ctx_destroy(gd_graph* g);  // gd_lean.cu
 
 extern "C" void gd_graph_destroy(gd_graph* g) {
     if (!g) return;
-    int prev = 0;
-    bool have_prev = cudaGetDevice(&prev) == cudaSuccess;
-    cudaSetDevice(g->device);
-    gd_host_ctx_destroy(g);
-    gd_lean_ctx_destroy(g);
-    if (g->gstate) cudaFree(g->gstate);
-    if (g->blob_dev) cudaFree(g->blob_dev);
-    if (have_prev) cudaSetDevice(prev);
+    {
+        gd::DeviceGuard dg(g->device);
+        gd_host_ctx_destroy(g);
+        gd_lean_ctx_destroy(g);
+        if (g->gstate) cudaFree(g->gstate);
+        if (g->blob_dev) cudaFree(g->blob_dev);
+    }
     delete g;
 }
 
@@ -176,9 +173,8 @@ extern "C" int gd_graph_tables(const gd_graph* g, int32_t* var_ptr, int32_t* var
     GD_CHECK_ARG(g != nullptr, "gd_graph_tables: graph is NULL");
     // read back from the DEVICE copy so tests pin what the kernels actually index with
     const size_t E = (size_t)g->E;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     auto get = [&](int32_t* dst, const int32_t* src, size_t n) -> cudaError_t {
         return dst ? cudaMemcpy(dst, src, n * sizeof(int32_t), cudaMemcpyDeviceToHost) : cudaSuccess;
     };
@@ -188,7 +184,6 @@ extern "C" int gd_graph_tables(const gd_graph* g, int32_t* var_ptr, int32_t* var
     if (e == cudaSuccess) e = get(chk_edges, g->t.chk_edges, E);
     if (e == cudaSuccess) e = get(edge_var, g->t.edge_var, E);
     if (e == cudaSuccess) e = get(edge_chk, g->t.edge_chk, E);
-    cudaSetDevice(prev);
     GD_CUDA(e);
     return GD_OK;
 }
@@ -217,9 +212,8 @@ extern "C" int gd_graph_check_batched(const gd_graph* g, const int64_t* ei_dev, 
     GD_CHECK_ARG(g && ei_dev && mismatches_host, "gd_graph_check_batched: NULL argument");
     GD_CHECK_ARG(B > 0, "gd_graph_check_batched: B must be positive");
     cudaStream_t st = (cudaStream_t)stream;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     unsigned long long* bad = nullptr;
     cudaError_t e = cudaMalloc((void**)&bad, sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0, sizeof(unsigned long long), st);
@@ -235,7 +229,6 @@ extern "C" int gd_graph_check_batched(const gd_graph* g, const int64_t* ei_dev, 
     if (e == cudaSuccess) e = cudaMemcpyAsync(&h, bad, sizeof(h), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (bad) cudaFree(bad);
-    cudaSetDevice(prev);
     GD_CUDA(e);
     *mismatches_host = (int64_t)h;
     return GD_OK;

@@ -116,9 +116,11 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
     const int64_t n_w = gd_weights_size(model);
     GD_CHECK_ARG(n_w == 0 || weights_host, "gd_decode_host: weights is NULL");
 
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
+    gd::Route r;
+    int rc = gd::route_decode(g, model, B, gd::Use::Infer, &r);
+    if (rc != GD_OK) return rc;
     std::unique_lock<std::mutex> lk(g->mu);
     if (!g->host_ctx) g->host_ctx = new gd::HostCtx();
     gd::HostCtx* c = static_cast<gd::HostCtx*>(g->host_ctx);
@@ -126,11 +128,11 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
     // one call at a time per graph from here on: the staging buffers, streams, gate flags and epochs are shared state
     std::lock_guard<std::mutex> call_lk(c->call_mu);
     cudaError_t e = gd::ensure(c, g, B, n_w);
-    int rc = GD_OK;
     if (e == cudaSuccess && c->memops < 0) gd::probe_memops(c, g->device);
-    int tile = 0, n_tiles = 0;
-    if (e == cudaSuccess && c->memops == 1 && B >= 16384 && gd::gated_plan(g, model, B, &tile, &n_tiles)) {
+    if (e == cudaSuccess && c->memops == 1 && B >= 16384 && gd::route_gated(r, model)) {
         // ---- gated pipeline: st[0] = kernel, st[1] = copies in, st[2] = copies out ----
+        const gd_launch_info li = gd::route_launch_info(r);
+        const int tile = li.tile, n_tiles = li.n_tiles;
         int n_chunks = (int)std::max<long long>(1, gd::opt_int(gd::OPT_GATE_CHUNKS, 16));   // measured on B200, rotated d=5 B=65536: 4 -> 19.20, 8 -> 19.41, 16 -> 19.55 M syn/s
         n_chunks = std::min(std::min(n_chunks, gd::kMaxGateChunks), std::max(1, (int)(B / 4096)));
         const int chunk_tiles = (n_tiles + n_chunks - 1) / n_chunks;
@@ -155,8 +157,10 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
         bool memop_failed = false, launched = false;
         auto launch = [&]() {
             gd::Gate gate{in_flags, out_counts, c->gate_err_dev, epoch, chunk_tiles};
-            rc = gd::decode_fwd_gated(g, model, c->w_dev, c->x_dev, prob_host ? c->prob_dev : nullptr,
-                                      hard_host ? c->hard_dev : nullptr, B, c->st[0], gate);
+            gd::DecodeIO io{};
+            io.weights = c->w_dev; io.x = c->x_dev; io.prob = prob_host ? c->prob_dev : nullptr;
+            io.hard = hard_host ? c->hard_dev : nullptr;
+            rc = gd::decode_routed(g, model, r, io, B, c->st[0], &gate);
             launched = rc == GD_OK;
         };
         if (e == cudaSuccess && kernel_first) launch();
@@ -198,7 +202,6 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
         cudaError_t s1 = cudaStreamSynchronize(c->st[1]);
         cudaError_t s2 = cudaStreamSynchronize(c->st[2]);   // the kernel always drains, so every queued wait is satisfied
         if (e == cudaSuccess) e = s0 != cudaSuccess ? s0 : (s1 != cudaSuccess ? s1 : s2);
-        if (prev != g->device) cudaSetDevice(prev);
         if (rc != GD_OK) return rc;
         GD_CUDA(e);
         c->last_launches = 1;
@@ -206,7 +209,6 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
         // a gate timed out (the copy-in stream was held up behind the kernel) or a memory operation was refused: results
         // are not trustworthy -> never gate again on this graph and redo the batch with one launch per chunk
         c->memops = 0;
-        if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
     }
     if (e == cudaSuccess && n_w) {
         e = cudaMemcpyAsync(c->w_dev, weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice, c->st[0]);
@@ -215,8 +217,7 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
     if (e == cudaSuccess) {
         // chunks: multiples of 8 syndromes (output alignment); >= 4096 syndromes each, at most 4
         int n_chunks = (int)std::min<int64_t>(4, std::max<int64_t>(1, B / 8192));
-        gd_launch_info li;
-        if (gd_decode_launch_info(g, model, B, &li) == GD_OK && !li.resident) n_chunks = 1;  // one shared slab
+        if (r.family == gd::Family::StreamedTma || r.family == gd::Family::Streamed) n_chunks = 1;  // one shared slab
         int64_t per = ((B + n_chunks - 1) / n_chunks + 7) / 8 * 8;
         c->last_launches = 0;
         for (int k = 0; k < n_chunks && e == cudaSuccess && rc == GD_OK; ++k) {
@@ -242,7 +243,6 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
         cudaError_t s1 = cudaStreamSynchronize(c->st[1]);
         if (e == cudaSuccess) e = s0 != cudaSuccess ? s0 : s1;
     }
-    if (prev != g->device) cudaSetDevice(prev);
     if (rc != GD_OK) return rc;
     GD_CUDA(e);
     return GD_OK;

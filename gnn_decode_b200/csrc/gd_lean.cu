@@ -45,28 +45,6 @@ constexpr float kBudgetR = 4e-6f;     // read-out table: adds <= 2 terms to the 
 
 static_assert(sizeof(LeanHeader) <= kHdrBytes, "header");
 
-struct LeanParams {
-    // packed inputs, sorted by prior
-    const int* idx;              // [B] syndrome ids: first the call->count[0] ones that carry the prior of slot 0, then slot 1's, ...
-    const uint32_t* sgn;         // [B][nw] bit c = check c's input is -1
-    float* prob; float* logit; uint8_t* hard; uint32_t* hard_bits;
-    LeanHeader* hdr;
-    LeanCall* call;              // this call's state
-    LeanCall* next_call;         // the next call's: cleared here
-    float* stash;                // training: m after every iteration, [T][E][B] by sorted position (NULL otherwise)
-    LeanTrainHdr* train;         // training: the header at the end of the stash buffer
-    const int* idx_src;          // training: the prior-sorted list, copied behind the header
-    const float4* ctab; const float4* rtab; const float4* vtab;   // global tables: (n + 2) pieces each, piece 0 = interval -1
-    const uint32_t* meta;        // device metadata blob of this (graph, R)
-    long long B;
-    int T, V, C, E, nw, vw, P;   // P = odd pitch of the staged logits; E = edges of THIS launch's part of the graph
-    int v_lo, nv, part;          // the part's variables [v_lo, v_lo + nv); part = 1: one of several launches (connected components)
-    int R, G, NCH;               // owners per group, groups per CTA, checks per owner (padded)
-    int ct_n, rt_n, vt_n;        // vt_n: BASE piece count of the variable-phase tables (the header holds the one in use)
-    int train_vt_max;            // training: most pieces the backward kernel can seat
-    int off_me, off_ms, off_mi, off_var, off_ct, off_rt, off_vt, off_state;   // shared-memory byte offsets
-};
-
 // ------------------------------------------------------------------------------------------------------------------
 // shared-memory access by 32-bit address
 __device__ __forceinline__ uint32_t lds_u32(uint32_t a) {
@@ -1235,13 +1213,6 @@ struct LeanCtx {
     unsigned long long tick = 0;
 };
 
-struct LeanPlan {
-    LeanParams p;
-    int threads, grid, smem, n_tiles;
-    const LeanMeta* meta;
-    int n_parts = 1;                       // launches this plan is one of
-};
-
 static int align_up_i(int x, int a) { return (x + a - 1) / a * a; }
 
 // owners' check lists: longest-processing-time assignment by degree (ties: ascending check id) -> balanced edge counts
@@ -1521,7 +1492,7 @@ static bool lean_fill(gd_graph* g, const LeanSub* sub, const gd_model* m, int64_
 // so the same results) -- when the whole graph's edge state does not fit shared memory (toric L = 11: 960 edges x 256 B per group),
 // or when halving the state seats more groups (GD_LEAN_PARTS).  Training always takes the whole graph (its stash is laid out by
 // global edge id).
-static bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>* out, bool whole_only = false) {
+bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>* out, bool whole_only) {
     out->clear();
     if (!lean_applicable(g, m)) return false;
     const std::vector<LeanSub*>& subs = lean_subs(g);
@@ -1582,15 +1553,6 @@ static bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<Lea
         out->push_back(pl);
     }
     return !out->empty();
-}
-
-bool lean_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out) {
-    std::vector<LeanPlan> pls;
-    if (!lean_plan(const_cast<gd_graph*>(g), model, B, &pls)) return false;
-    const LeanPlan& pl = pls[0];                               // (parts: the first launch's geometry; tiles of all launches)
-    out->tile = 32 * pl.p.G; out->threads = pl.threads; out->grid = pl.grid; out->smem_bytes = pl.smem;
-    out->resident = 1; out->n_tiles = (int)pls.size() * ((pl.n_tiles + pl.p.G - 1) / pl.p.G);
-    return true;
 }
 
 // the passes of a decode call follow one another by programmatic dependent launch (gd_common.cuh: pdl_enter / pdl_launch_on)
@@ -1736,18 +1698,28 @@ static LeanEntry* lean_entry(gd_graph* g, LeanCtx* ctx, const LeanParams& p, con
     return hit;
 }
 
-int lean_decode(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, const float* prior_dev,
-                const uint32_t* synd_dev, float* prob_dev, float* logit_dev, uint8_t* hard_dev, uint32_t* hard_bits_dev,
-                int64_t B, cudaStream_t st, float* stash_dev) {
-    std::vector<LeanPlan> pls;
-    if (!lean_plan(g, model, B, &pls, stash_dev != nullptr)) return -1;
+int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>& plans, const DecodePlan& deferred,
+                const DecodeIO& io, int64_t B, cudaStream_t st, bool* no_resources) {
+    *no_resources = false;
+    const float* x_dev = io.x;
+    const float* weights_dev = io.weights;
+    float* stash_dev = io.stash;
+    std::vector<LeanPlan> pls = plans;
+    LeanParams& p = pls[0].p;                                   // table sizes and batch layout are the same for every part
+    // rows per CTA of the prep pass: 64 (x given: 8 warps x 4 rows, twice) or 256 (packed: a thread per row), more only for
+    // batches beyond 2^24
+    int prep_rows = x_dev ? 64 : kPrepRows;
+    while ((B + prep_rows - 1) / prep_rows > (1 << 18) && prep_rows < kPrepRows) prep_rows *= 2;
+    const long long prep_blocks = (B + prep_rows - 1) / prep_rows;
+    GD_CHECK_ARG(prep_blocks < (1ll << 30), "gd_decode_fwd: batch too large for the table kernel's prep pass");
     cudaMemPool_t pool = lean_pool(g);
-    if (!pool) return -1;
     LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
     std::lock_guard<std::mutex> enq(ctx->enq);
-    LeanParams& p = pls[0].p;                                   // table sizes and batch layout are the same for every part
-    LeanEntry* ent = lean_entry(g, ctx, p, model, weights_dev, st);
-    if (!ent) return -1;
+    LeanEntry* ent = pool ? lean_entry(g, ctx, p, model, weights_dev, st) : nullptr;
+    if (!ent) {
+        *no_resources = true;
+        return GD_OK;
+    }
     const int N = g->N;
     // per-call workspace: slot | pos | idx | sgn | defer_idx | (x for the deferred pass of packed calls)
     size_t off = 0;
@@ -1771,19 +1743,15 @@ int lean_decode(gd_graph* g, const gd_model* model, const float* weights_dev, co
         memset(&pp, 0, sizeof(pp));
         pp.x = x_dev; pp.weights = weights_dev; pp.hdr = hdr; pp.call = call;
         pp.sgn_out = reinterpret_cast<uint32_t*>(ws + o_sgn);
-        pp.prior_in = prior_dev; pp.slot = reinterpret_cast<short*>(ws + o_slot); pp.pos = reinterpret_cast<int*>(ws + o_pos);
+        pp.prior_in = io.prior; pp.slot = reinterpret_cast<short*>(ws + o_slot); pp.pos = reinterpret_cast<int*>(ws + o_pos);
         pp.defer_idx = reinterpret_cast<int*>(ws + o_defer);
         pp.B = B; pp.V = g->V; pp.C = g->C; pp.N = N; pp.nw = p.nw;
         pp.n_w = (int)gd_weights_size(model); pp.T = model->iters; pp.ct_n = p.ct_n; pp.rt_n = p.rt_n; pp.vt_n = p.vt_n;
-        // rows per CTA: 64 (x given: 8 warps x 4 rows, twice) or 256 (packed: a thread per row), more only for batches beyond 2^24
-        pp.rows_per_block = x_dev ? 64 : kPrepRows;
-        while ((B + pp.rows_per_block - 1) / pp.rows_per_block > (1 << 18) && pp.rows_per_block < kPrepRows) pp.rows_per_block *= 2;
-        const long long blocks = (B + pp.rows_per_block - 1) / pp.rows_per_block;
-        GD_CHECK_ARG(blocks < (1ll << 30), "gd_decode_fwd: batch too large for the table kernel's prep pass");
+        pp.rows_per_block = prep_rows;
         pp.hid = model->hidden;
         pp.keep_mult = stash_dev ? 1 : 0;
         pp.fm_blocks = (p.ct_n + 3 + kD3Points + 7) / 8;          // 8 warps = 8 points per CTA (check-table nodes, then the mlp3' grid)
-        e = pdl_launch(lean_prep_kernel, dim3((unsigned int)(1 + pp.fm_blocks + blocks)), dim3(256), 0, st, pp);
+        e = pdl_launch(lean_prep_kernel, dim3((unsigned int)(1 + pp.fm_blocks + prep_blocks)), dim3(256), 0, st, pp);
     }
     if (e == cudaSuccess) {
         TabParams tp;
@@ -1798,14 +1766,14 @@ int lean_decode(gd_graph* g, const gd_model* model, const float* weights_dev, co
         tp.scatter_blocks = (int)std::max<long long>(1, std::min<long long>((B + 1023) / 1024, (long long)g->sm_count * 4));
         e = pdl_launch(lean_tables_kernel, dim3(tp.scatter_blocks + tp.ct_blocks + tp.rt_blocks + tp.vt_chunks), dim3(256), 0, st, tp);
     }
-    if (e == cudaSuccess && pls.size() > 1 && hard_bits_dev)    // parts share the words at their borders and OR their bits in
-        e = cudaMemsetAsync(hard_bits_dev, 0, (size_t)B * p.vw * sizeof(uint32_t), st);
+    if (e == cudaSuccess && pls.size() > 1 && io.hard_bits)     // parts share the words at their borders and OR their bits in
+        e = cudaMemsetAsync(io.hard_bits, 0, (size_t)B * p.vw * sizeof(uint32_t), st);
     for (size_t pi = 0; pi < pls.size() && e == cudaSuccess; ++pi) {
         LeanPlan& pl = pls[pi];
         LeanParams& q = pl.p;
         q.idx = reinterpret_cast<const int*>(ws + o_idx);
-        q.sgn = x_dev ? reinterpret_cast<const uint32_t*>(ws + o_sgn) : synd_dev;
-        q.prob = prob_dev; q.logit = logit_dev; q.hard = hard_dev; q.hard_bits = hard_bits_dev;
+        q.sgn = x_dev ? reinterpret_cast<const uint32_t*>(ws + o_sgn) : io.synd;
+        q.prob = io.prob; q.logit = io.logit; q.hard = io.hard; q.hard_bits = io.hard_bits;
         q.hdr = hdr; q.call = call; q.next_call = next_call;
         q.ctab = ctab; q.rtab = rtab; q.vtab = vtab;
         q.stash = stash_dev;
@@ -1821,19 +1789,19 @@ int lean_decode(gd_graph* g, const gd_model* model, const float* weights_dev, co
     }
     cudaEventRecord(ent->ev, st);                                // the entry's tables are free again after this point of the stream
     // the syndromes the tables could not serve: edge-owner kernel, direct evaluation, per item
-    const float* x_for_deferred = x_dev;
+    DecodeIO dio = io;
     if (e == cudaSuccess && !x_dev) {
         float* xw = reinterpret_cast<float*>(ws + o_x);
-        lean_unpack_kernel<<<g->sm_count * 4, 256, 0, st>>>(prior_dev, synd_dev, call, reinterpret_cast<const int*>(ws + o_defer), xw,
+        lean_unpack_kernel<<<g->sm_count * 4, 256, 0, st>>>(io.prior, io.synd, call, reinterpret_cast<const int*>(ws + o_defer), xw,
                                                             B, g->V, g->C, p.nw);
         e = cudaGetLastError();
-        x_for_deferred = xw;
+        dio.x = xw;
     }
     if (e == cudaSuccess) {
         // training: all rows or none (the header's old_count is 0 or -1), and the edge-owner kernel writes its own stash layout
         const DeferList dl{stash_dev ? &lean_train_hdr(stash_dev, g, model, B)->old_count : &call->defer_count,
                            reinterpret_cast<const int*>(ws + o_defer)};
-        rc = decode_fwd_deferred(g, model, weights_dev, x_for_deferred, prob_dev, logit_dev, hard_dev, hard_bits_dev, B, st, dl, stash_dev);
+        rc = edge_decode(g, model, deferred, dio, st, nullptr, &dl);
     }
     cudaError_t ef = cudaFreeAsync(ws, st);
     if (rc != GD_OK) return rc;
@@ -1870,11 +1838,9 @@ int64_t lean_bwd_bins_floats(const gd_graph* g, const gd_model* model) {
     return 2 * 2 * ((int64_t)(ct_n + 3) + (2048 + 3) + (int64_t)kMaxSlots * (4 * vt_n + 3));   // [2][nodes] 64-bit bins
 }
 
-int lean_backward(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, const float* stash_dev,
-                  const float* grad_logit_dev, float* grad_weights_dev, float* bins_dev, int accumulate, int64_t B, cudaStream_t st) {
-    std::vector<LeanPlan> fwds;
-    if (!lean_plan(g, model, B, &fwds, true)) return -1;       // the forward took the edge-owner kernel as well
-    const LeanPlan& fwd = fwds[0];
+int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const float* weights_dev, const float* x_dev,
+                  const float* stash_dev, const float* grad_logit_dev, float* grad_weights_dev, float* bins_dev, int accumulate,
+                  int64_t B, cudaStream_t st) {
     LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
     std::lock_guard<std::mutex> enq(ctx->enq);
     // the table set the forward of this step used (same stream, same weights): it is not touched in between
@@ -1891,10 +1857,13 @@ int lean_backward(gd_graph* g, const gd_model* model, const float* weights_dev, 
     memset(&p, 0, sizeof(p));
     const int E = (int)g->E, ct_n = fwd.p.ct_n, rt_n = fwd.p.rt_n, vt_n = fwd.p.vt_n;
     LeanBwdGeom bg;
-    if (!lean_bwd_geom(g, fwd.p, &bg)) return -1;              // (the forward saw the same answer and left the stash to the edge-owner kernel)
+    if (!lean_bwd_geom(g, fwd.p, &bg)) return GD_OK;           // the forward saw the same answer and left the stash to the edge-owner kernel
     const int bestR = bg.R, bestG = bg.G;
     const LeanMeta* meta = get_meta(g, lean_subs(g)[0], bestR);
-    if (!meta) return -1;
+    if (!meta) {
+        set_error("gd_decode_bwd: could not upload the table backward's metadata on device %d", g->device);
+        return GD_ERR_CUDA;
+    }
     const LeanTrainHdr* hdr = lean_train_hdr(const_cast<float*>(stash_dev), g, model, B);
     p.x = x_dev; p.stash = stash_dev; p.train = hdr; p.grad_logit = grad_logit_dev;
     p.ctab = reinterpret_cast<const float4*>(ent->dev + ent->o_ct);

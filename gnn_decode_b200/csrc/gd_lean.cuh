@@ -66,27 +66,51 @@ struct DeferList {
     const int* idx;              // [B] syndrome indices (valid when *count > 0)
 };
 
-// returns -1 when the lean path does not apply to (graph, model) -- the caller then takes the edge-owner kernel --
-// otherwise a gd_status.  Exactly one of x_dev / (prior_dev, synd_dev) is given.
-int lean_decode(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, const float* prior_dev,
-                const uint32_t* synd_dev, float* prob_dev, float* logit_dev, uint8_t* hard_dev, uint32_t* hard_bits_dev,
-                int64_t B, cudaStream_t st, float* stash_dev = nullptr);
-// training: the table backward (returns -1 when the lean path does not apply to (graph, model)); it runs only if the stash header
-// says the table forward wrote it.  grad_weights_dev receives (or accumulates) the 10h+3 gradients; bins_dev: lean_bwd_bins_floats() floats.
-int lean_backward(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, const float* stash_dev,
-                  const float* grad_logit_dev, float* grad_weights_dev, float* bins_dev, int accumulate, int64_t B, cudaStream_t st);
+struct LeanParams {
+    // packed inputs, sorted by prior
+    const int* idx;              // [B] syndrome ids: first the call->count[0] ones that carry the prior of slot 0, then slot 1's, ...
+    const uint32_t* sgn;         // [B][nw] bit c = check c's input is -1
+    float* prob; float* logit; uint8_t* hard; uint32_t* hard_bits;
+    LeanHeader* hdr;
+    LeanCall* call;              // this call's state
+    LeanCall* next_call;         // the next call's: cleared here
+    float* stash;                // training: m after every iteration, [T][E][B] by sorted position (NULL otherwise)
+    LeanTrainHdr* train;         // training: the header at the end of the stash buffer
+    const int* idx_src;          // training: the prior-sorted list, copied behind the header
+    const float4* ctab; const float4* rtab; const float4* vtab;   // global tables: (n + 2) pieces each, piece 0 = interval -1
+    const uint32_t* meta;        // device metadata blob of this (graph, R)
+    long long B;
+    int T, V, C, E, nw, vw, P;   // P = odd pitch of the staged logits; E = edges of THIS launch's part of the graph
+    int v_lo, nv, part;          // the part's variables [v_lo, v_lo + nv); part = 1: one of several launches (connected components)
+    int R, G, NCH;               // owners per group, groups per CTA, checks per owner (padded)
+    int ct_n, rt_n, vt_n;        // vt_n: BASE piece count of the variable-phase tables (the header holds the one in use)
+    int train_vt_max;            // training: most pieces the backward kernel can seat
+    int off_me, off_ms, off_mi, off_var, off_ct, off_rt, off_vt, off_state;   // shared-memory byte offsets
+};
+
+struct LeanMeta;
+// One launch of the table kernel: the whole graph, or one of its connected components.
+struct LeanPlan {
+    LeanParams p;
+    int threads, grid, smem, n_tiles;
+    const LeanMeta* meta;
+    int n_parts = 1;                       // launches this plan is one of
+};
+
+// Plans the table kernel for (graph, model, B); false when it does not serve them.  whole_only: training (the stash is laid
+// out by global edge id), and the forward and the backward of a step plan alike.
+bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>* out, bool whole_only = false);
+// training: the table backward of the forward `fwd` planned.  It runs only if the stash header says the table forward wrote
+// the stash; when it has no room at all it launches nothing (the forward saw the same and left the stash to the edge-owner
+// kernel).  grad_weights_dev receives (or accumulates) the 10h+3 gradients; bins_dev: lean_bwd_bins_floats() floats.
+int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const float* weights_dev, const float* x_dev,
+                  const float* stash_dev, const float* grad_logit_dev, float* grad_weights_dev, float* bins_dev, int accumulate,
+                  int64_t B, cudaStream_t st);
 int64_t lean_bwd_bins_floats(const gd_graph* g, const gd_model* model);
 inline LeanTrainHdr* lean_train_hdr(float* stash, const gd_graph* g, const gd_model* m, int64_t B) {
     return reinterpret_cast<LeanTrainHdr*>(stash + (int64_t)(m->iters + 1) * 2 * g->E * B);
 }
 int packed_via_unpack(gd_graph* g, const float* prior_dev, const uint32_t* synd_dev, int64_t B, cudaStream_t st,
                       int (*run)(void* ctx, const float* x_dev), void* ctx);
-bool lean_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out);
-
-// gd_decode.cu: run the edge-owner resident kernel over a deferred list (no variable-phase tables: per-item direct
-// evaluation, so a deferred syndrome's result never depends on what else was deferred)
-int decode_fwd_deferred(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                        float* logit_dev, uint8_t* hard_dev, uint32_t* hard_bits_dev, int64_t B, cudaStream_t st,
-                        const DeferList& dl, float* stash_dev = nullptr);
 
 }  // namespace gd

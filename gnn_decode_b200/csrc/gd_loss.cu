@@ -74,16 +74,14 @@ extern "C" int gd_loss_v2_4(const gd_graph* g, const uint8_t* logical_dev, int32
     int64_t blocks = (B + 3) / 4;
     if (blocks > (int64_t)g->sm_count * 16) blocks = (int64_t)g->sm_count * 16;
     const int smem = 4 * (g->V + g->C + K) * (int)sizeof(float);
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     cudaError_t e = cudaSuccess;
     if (smem > 48 * 1024) e = cudaFuncSetAttribute(gd::loss_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e == cudaSuccess) {
         e = gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::loss_kernel, dim3((unsigned)blocks), dim3(128), (size_t)smem, (cudaStream_t)stream,
                               prob_dev, y_dev, logical_dev, K, g->t, B, g->V, g->C, loss_per_syndrome_dev, grad_prob_dev, grad_logit_dev);
     }
-    if (prev != g->device) cudaSetDevice(prev);
     GD_CUDA(e);
     return GD_OK;
 }

@@ -39,9 +39,7 @@ namespace {
 
 void pipeline_free(gd_pipeline* p) {
     if (!p) return;
-    int prev = 0;
-    const bool have_prev = cudaGetDevice(&prev) == cudaSuccess;
-    cudaSetDevice(p->g->device);
+    gd::DeviceGuard dg(p->g->device);
     for (auto& s : p->slots) {
         if (s.ev_out && s.in_flight) cudaEventSynchronize(s.ev_out);
         cudaFree(s.x); cudaFree(s.prior); cudaFree(s.synd); cudaFree(s.prob); cudaFree(s.hard); cudaFree(s.bits);
@@ -53,7 +51,6 @@ void pipeline_free(gd_pipeline* p) {
     if (p->s_comp) cudaStreamDestroy(p->s_comp);
     if (p->s_out) cudaStreamDestroy(p->s_out);
     cudaFree(p->w_dev);
-    if (have_prev) cudaSetDevice(prev);
     delete p;
 }
 
@@ -79,9 +76,8 @@ extern "C" int gd_pipeline_create(const gd_graph* g, const gd_model* model, cons
     GD_CHECK_ARG(depth >= 1 && depth <= 8, "gd_pipeline_create: depth must be 1..8");
     const int64_t n_w = gd_weights_size(model);
     GD_CHECK_ARG(n_w == 0 || weights_host, "gd_pipeline_create: weights is NULL");
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     gd_pipeline* p = new gd_pipeline();
     p->g = g; p->model = *model; p->max_B = max_B; p->depth = depth;
     p->nw = (g->C + 31) / 32; p->vw = (g->V + 31) / 32;
@@ -99,7 +95,6 @@ extern "C" int gd_pipeline_create(const gd_graph* g, const gd_model* model, cons
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_comp, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_out, cudaEventDisableTiming);
     }
-    cudaSetDevice(prev);
     if (e != cudaSuccess) {
         gd::set_error("gd_pipeline_create: %s", cudaGetErrorString(e));
         pipeline_free(p);
@@ -117,12 +112,10 @@ extern "C" int gd_pipeline_set_weights(gd_pipeline* p, const float* weights_host
     if (n_w == 0) return GD_OK;
     GD_CHECK_ARG(weights_host != nullptr, "gd_pipeline_set_weights: weights is NULL");
     std::lock_guard<std::mutex> lk(p->mu);
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    GD_CUDA(cudaSetDevice(p->g->device));
+    gd::DeviceGuard dg(p->g->device);
+    GD_CUDA(dg.status());
     // in compute-stream order: batches already submitted keep the old weights (pageable source: staged before the call returns)
     cudaError_t e = cudaMemcpyAsync(p->w_dev, weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice, p->s_comp);
-    cudaSetDevice(prev);
     GD_CUDA(e);
     return GD_OK;
 }
@@ -146,9 +139,8 @@ extern "C" int gd_pipeline_submit_packed(gd_pipeline* p, const float* prior_host
     GD_CHECK_ARG(prob_host || hard_bits_host, "gd_pipeline_submit_packed: no output requested");
     std::lock_guard<std::mutex> lk(p->mu);
     const gd_graph* g = p->g;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     const int i = (int)(p->submitted % p->depth);
     gd_pipeline::Slot& s = p->slots[i];
     int rc = slot_acquire(p, i);
@@ -170,7 +162,6 @@ extern "C" int gd_pipeline_submit_packed(gd_pipeline* p, const float* prior_host
             e = cudaMemcpyAsync(prob_host, s.prob, (size_t)B * g->V * sizeof(float), cudaMemcpyDeviceToHost, p->s_out);
         if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_out, p->s_out);
     }
-    if (prev != g->device) cudaSetDevice(prev);
     return pipeline_finish(p, s, rc, e, ticket);
 }
 
@@ -182,9 +173,8 @@ extern "C" int gd_pipeline_submit(gd_pipeline* p, const float* x_host, float* pr
     GD_CHECK_ARG(prob_host || hard_host, "gd_pipeline_submit: no output requested");
     std::lock_guard<std::mutex> lk(p->mu);
     const gd_graph* g = p->g;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     const int i = (int)(p->submitted % p->depth);
     gd_pipeline::Slot& s = p->slots[i];
     int rc = slot_acquire(p, i);
@@ -207,7 +197,6 @@ extern "C" int gd_pipeline_submit(gd_pipeline* p, const float* x_host, float* pr
             e = cudaMemcpyAsync(hard_host, s.hard, (size_t)B * g->V, cudaMemcpyDeviceToHost, p->s_out);
         if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_out, p->s_out);
     }
-    if (prev != g->device) cudaSetDevice(prev);
     return pipeline_finish(p, s, rc, e, ticket);
 }
 

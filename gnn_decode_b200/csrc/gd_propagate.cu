@@ -198,9 +198,8 @@ extern "C" int gd_propagate_fwd(const gd_graph* g, const gd_model* model, int32_
     if (blocks > (int64_t)g->sm_count * 16) blocks = (int64_t)g->sm_count * 16;
     const int smem = 4 * p.hp * (int)sizeof(float) + 16;
     cudaStream_t st = (cudaStream_t)stream;
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     int rc;
     switch (prog) {
         case GD_PROG_CGNNI: rc = gd::launch_prop<GD_PROG_CGNNI>(p, phase, (int)blocks, smem, st); break;
@@ -213,6 +212,5 @@ extern "C" int gd_propagate_fwd(const gd_graph* g, const gd_model* model, int32_
         case GD_PROG_V1_2_2: rc = gd::launch_prop<GD_PROG_V1_2_2>(p, phase, (int)blocks, smem, st); break;
         default: rc = gd::launch_prop<GD_PROG_BP_CLASSICAL>(p, phase, (int)blocks, smem, st); break;
     }
-    if (prev != g->device) cudaSetDevice(prev);
     return rc;
 }

@@ -143,9 +143,8 @@ extern "C" int gd_sample(const gd_graph* g, int32_t noise, const float* p_list, 
     int64_t blocks = (B + 3) / 4;
     if (blocks > (int64_t)g->sm_count * 16) blocks = (int64_t)g->sm_count * 16;
     const int smem = 4 * ((g->V + 15) / 16 * 16);
-    int prev = 0;
-    GD_CUDA(cudaGetDevice(&prev));
-    if (prev != g->device) GD_CUDA(cudaSetDevice(g->device));
+    gd::DeviceGuard dg(g->device);
+    GD_CUDA(dg.status());
     cudaError_t e = cudaSuccess;
     if (smem > 48 * 1024)
         e = cudaFuncSetAttribute(gd::sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
@@ -153,7 +152,6 @@ extern "C" int gd_sample(const gd_graph* g, int32_t noise, const float* p_list, 
         gd::sample_kernel<<<(int)blocks, 128, smem, (cudaStream_t)stream>>>(p);
         e = cudaGetLastError();
     }
-    if (prev != g->device) cudaSetDevice(prev);
     GD_CUDA(e);
     return GD_OK;
 }

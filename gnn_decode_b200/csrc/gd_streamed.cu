@@ -20,22 +20,6 @@
 
 namespace gd {
 
-struct StreamParams {
-    const float* x;
-    float* prob;
-    float* logit;
-    uint8_t* hard;
-    const float* weights;
-    GraphTables tb;
-    float* slab;
-    long long B;
-    long long slab_floats;   // per CTA
-    int T, V, C, E, N;
-    int tile, R, hid, hp, n_tiles;
-    int ctab_n, rtab_n;      // V2_4: intervals of the check-phase / read-out cubic tables (0 = direct evaluation)
-    float ctab_R;
-};
-
 __device__ __forceinline__ void stage_mlp_s(float* dst, int hp, int hid, const float* w1, int w1_stride, bool two_in,
                                             const float* b1, const float* w2, float s1, float s2, int tid, int nthr) {
     for (int k = tid; k < hp; k += nthr) {
@@ -299,12 +283,7 @@ __global__ void __launch_bounds__(1024, 1) decode_streamed_kernel(const StreamPa
     }
 }
 
-struct StreamPlan {
-    StreamParams p;
-    int threads, grid, smem;
-};
-
-static int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* out) {
+int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* out) {
     const bool bp = m->program == GD_PROG_BP_QUANTUM || m->program == GD_PROG_BP_CLASSICAL;
     StreamParams& p = out->p;
     memset(&p, 0, sizeof(p));
@@ -349,46 +328,28 @@ static int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, Stream
     return GD_OK;
 }
 
-int streamed_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out) {
-    if (streamed_tma_launch_info(g, model, B, out)) return GD_OK;   // the TMA-staged kernel (gd_streamed_tma.cu)
-    StreamPlan pl;
-    int rc = plan_streamed(g, model, B, &pl);
-    if (rc != GD_OK) return rc;
-    out->tile = pl.p.tile; out->threads = pl.threads; out->grid = pl.grid; out->smem_bytes = pl.smem;
-    out->resident = 0; out->n_tiles = pl.p.n_tiles;
-    return GD_OK;
+float* streamed_slab(gd_graph* g, size_t bytes) {
+    // The slab is per graph: concurrent streamed decodes of one graph on different streams
+    // must be serialised by the caller (documented in include/gnn_decode.h).
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (bytes > g->gstate_bytes) {
+        if (g->gstate) cudaFree(g->gstate);
+        g->gstate = nullptr; g->gstate_bytes = 0;
+        cudaError_t e = cudaMalloc((void**)&g->gstate, bytes);
+        if (e != cudaSuccess) {
+            set_error("gd_decode_fwd: cudaMalloc of the %zu-byte streamed edge-state slab failed: %s", bytes, cudaGetErrorString(e));
+            return nullptr;
+        }
+        g->gstate_bytes = bytes;
+    }
+    return g->gstate;
 }
 
-int streamed_decode(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                    float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st) {
-    {
-        // default: the TMA-staged kernel; it declines (rc < 0) graphs whose edges are not in the
-        // canonical variable-sorted order or whose largest node does not fit a pipeline stage
-        const int rc = streamed_tma_decode(g, model, weights_dev, x_dev, prob_dev, logit_dev, hard_dev, B, st);
-        if (rc >= 0) return rc;
-    }
-    StreamPlan pl;
-    int rc = plan_streamed(g, model, B, &pl);
-    if (rc != GD_OK) return rc;
-    pl.p.x = x_dev; pl.p.prob = prob_dev; pl.p.logit = logit_dev; pl.p.hard = hard_dev; pl.p.weights = weights_dev;
-    const size_t need = (size_t)pl.grid * (size_t)pl.p.slab_floats * sizeof(float);
-    {
-        // The slab is per graph: concurrent streamed decodes of one graph on different streams
-        // must be serialised by the caller (documented in include/gnn_decode.h).
-        std::lock_guard<std::mutex> lk(g->mu);
-        if (need > g->gstate_bytes) {
-            if (g->gstate) cudaFree(g->gstate);
-            g->gstate = nullptr; g->gstate_bytes = 0;
-            cudaError_t e = cudaMalloc((void**)&g->gstate, need);
-            if (e != cudaSuccess) {
-                set_error("gd_decode_fwd: cudaMalloc of the %zu-byte streamed edge-state slab failed: %s", need,
-                          cudaGetErrorString(e));
-                return GD_ERR_CUDA;
-            }
-            g->gstate_bytes = need;
-        }
-        pl.p.slab = g->gstate;
-    }
+int streamed_decode(gd_graph* g, const StreamPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st) {
+    StreamPlan pl = plan;
+    pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
+    pl.p.slab = streamed_slab(g, (size_t)pl.grid * (size_t)pl.p.slab_floats * sizeof(float));
+    if (!pl.p.slab) return GD_ERR_CUDA;
     void (*k)(const StreamParams);
     const bool v8 = g->max_var_deg > 4, c8 = g->max_chk_deg > 4;
     bool vsort = true;

@@ -31,27 +31,6 @@
 
 namespace gd {
 
-struct StreamTmaParams {
-    const float* x;
-    float* prob;
-    float* logit;
-    uint8_t* hard;
-    const float* weights;
-    GraphTables tb;
-    float* slab;
-    long long B;
-    long long slab_floats;   // per CTA
-    int T, V, C, E, N;
-    int tile, lanes, W, hid, hp, n_tiles;
-    int stage_rows;          // rows of tile floats per pipeline stage
-    int S;                   // pipeline stages per warp (2..4): S - 1 nodes are in flight while one is evaluated
-    int vchunk;              // variables per variable-phase item
-    int vrows;               // row index of the first prior row inside a variable-phase stage
-    int off_w, off_stage;    // shared-memory byte offsets (mbarriers sit at 0)
-    int off_ctab, off_rtab, ctab_n, rtab_n;   // decoder_v2_4: cubic tables of the check-phase and read-out MLPs (0: none)
-    float ctab_R;
-};
-
 namespace tma {
 __device__ __forceinline__ uint32_t s32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void bar_init(uint64_t* bar, uint32_t count) {
@@ -450,17 +429,11 @@ _Pragma("unroll")
     }
 }
 
-struct StreamTmaPlan {
-    StreamTmaParams p;
-    int threads, grid, smem, npad;
-    bool ok;
-};
-
 static int align_up_i(int x, int a) { return (x + a - 1) / a * a; }
 
 // Returns ok == false when the graph does not qualify (edges not in variable-sorted order, or a
 // node's rows do not fit a pipeline stage): the caller then takes the register-batched kernel.
-static void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out) {
+void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out) {
     StreamTmaParams& p = out->p;
     memset(&p, 0, sizeof(p));
     out->ok = false;
@@ -546,38 +519,11 @@ static void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, S
     out->ok = true;
 }
 
-bool streamed_tma_launch_info(const gd_graph* g, const gd_model* model, int64_t B, gd_launch_info* out) {
-    StreamTmaPlan pl;
-    plan_streamed_tma(g, model, B, &pl);
-    if (!pl.ok) return false;
-    out->tile = pl.p.tile; out->threads = pl.threads; out->grid = pl.grid; out->smem_bytes = pl.smem;
-    out->resident = 0; out->n_tiles = pl.p.n_tiles;
-    return true;
-}
-
-// rc < 0: not applicable (caller falls back); otherwise a gd_status.
-int streamed_tma_decode(gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, float* prob_dev,
-                        float* logit_dev, uint8_t* hard_dev, int64_t B, cudaStream_t st) {
-    StreamTmaPlan pl;
-    plan_streamed_tma(g, model, B, &pl);
-    if (!pl.ok) return -1;
-    pl.p.x = x_dev; pl.p.prob = prob_dev; pl.p.logit = logit_dev; pl.p.hard = hard_dev; pl.p.weights = weights_dev;
-    const size_t need = (size_t)pl.grid * (size_t)pl.p.slab_floats * sizeof(float);
-    {
-        std::lock_guard<std::mutex> lk(g->mu);
-        if (need > g->gstate_bytes) {
-            if (g->gstate) cudaFree(g->gstate);
-            g->gstate = nullptr; g->gstate_bytes = 0;
-            cudaError_t e = cudaMalloc((void**)&g->gstate, need);
-            if (e != cudaSuccess) {
-                set_error("gd_decode_fwd: cudaMalloc of the %zu-byte streamed edge-state slab failed: %s", need,
-                          cudaGetErrorString(e));
-                return GD_ERR_CUDA;
-            }
-            g->gstate_bytes = need;
-        }
-        pl.p.slab = g->gstate;
-    }
+int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st) {
+    StreamTmaPlan pl = plan;
+    pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
+    pl.p.slab = streamed_slab(g, (size_t)pl.grid * (size_t)pl.p.slab_floats * sizeof(float));
+    if (!pl.p.slab) return GD_ERR_CUDA;
     void (*k)(const StreamTmaParams);
     switch (model->program) {
         case GD_PROG_CGNNI:
