@@ -507,8 +507,8 @@ static int plan_bwd(const gd_graph* g, const gd_model* m, int64_t B, BwdPlan* ou
     const int tab_bytes = (5 * E + V + C + 2) * 2;
     int fixed = align_up_b(tab_bytes, 128);
     p.n_vact = opt_on(OPT_NO_VSKIP) ? E : g->n_vact;
-    if (!opt_on(OPT_NO_CTAB) && !opt_on(OPT_NO_BWD_CTAB)) {
-        p.ctab_n = 512;
+    if (!opt_on(OPT_NO_CTAB)) {
+        p.ctab_n = kCtabN;
         p.ctab_R = (float)(g->max_chk_deg > 1 ? g->max_chk_deg - 1 : 1);
         const int hp = (m->hidden + 7) / 8 * 8;
         p.off_ctab = fixed; fixed += p.ctab_n * 16;
@@ -612,10 +612,8 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
         pl.p.run_flag = &gd::lean_train_hdr(const_cast<float*>(stash_dev), g, model, B)->old_count;
     }
     GD_CUDA(cudaFuncSetAttribute(gd::decode_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
-    GD_CUDA(gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::decode_bwd_kernel, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem,
-                              st, pl.p));
-    GD_CUDA(gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::reduce_partials_kernel, dim3((n_params + 127) / 128), dim3(128), 0,
-                              st, workspace_dev, pl.n_rows, pl.p.np_pad, n_params, grad_weights_dev, accumulate ? 1 : 0,
-                              pl.p.run_flag));
+    GD_CUDA(gd::pdl_launch(gd::decode_bwd_kernel, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, pl.p));
+    GD_CUDA(gd::pdl_launch(gd::reduce_partials_kernel, dim3((n_params + 127) / 128), dim3(128), 0, st, workspace_dev, pl.n_rows,
+                           pl.p.np_pad, n_params, grad_weights_dev, accumulate ? 1 : 0, pl.p.run_flag));
     return GD_OK;
 }

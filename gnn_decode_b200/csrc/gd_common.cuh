@@ -77,13 +77,13 @@ __device__ __forceinline__ void pdl_enter() {
     asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 template <typename... KArgs, typename... Args>
-static inline cudaError_t pdl_launch_on(bool enable, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+static inline cudaError_t pdl_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = enable ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }

@@ -930,38 +930,24 @@ static int plan_decode(const gd_graph* g, const gd_model* m, int64_t B, DecodePl
     const int maxvc = V > C ? V : C;
     DecodeParams& p = out->p;
     memset(&p, 0, sizeof(p));
-    out->cps = 1;
     out->eb = 4;
     p.B = B; p.T = m->iters; p.V = V; p.C = C; p.E = (int)E64; p.N = N; p.hid = hid; p.hp = hp; p.maxvc = maxvc;
     p.tb = g->t;
     p.all_iters = (m->flags & GD_FLAG_ALL_ITERS) ? 1 : 0;
     p.n_vact = opt_on(OPT_NO_VSKIP) ? (int)g->E : g->n_vact;
-    p.vdirect = (g->max_var_deg <= 2 && !opt_on(OPT_NO_DIRECT)) ? 1 : 0;
-    p.cdirect = (g->max_chk_deg <= 4 && !opt_on(OPT_NO_DIRECT)) ? 1 : 0;
-
-    // CTAs per SM: two half-size CTAs let one CTA's light phases (node sums, table look-ups, barriers) overlap the
-    // other's MUFU-bound variable phase
-    {
-        out->cps = (int)opt_int(OPT_CPS, 1);
-        if (out->cps < 1 || out->cps > 4) out->cps = 1;
-    }
-    const int smem_max = out->cps == 1 ? g->max_smem_optin : (g->max_smem_sm - 1024 * out->cps) / out->cps;
-    const int thr_max = out->cps == 1 ? kMaxThreads : (kMaxThreads / out->cps) / 32 * 32;
+    p.vdirect = g->max_var_deg <= 2 ? 1 : 0;
+    p.cdirect = g->max_chk_deg <= 4 ? 1 : 0;
     int off = 16;                                  // mbarrier
     // ReLU programs with h < 32: piecewise-linear tables (3 * NPAD floats per MLP) instead of the SoA weight rows
     const bool relu_prog = m->program == GD_PROG_CGNNI || m->program == GD_PROG_QGNNI || m->program == GD_PROG_GRU_CA;   // 1-input ReLU MLPs
-    out->npad = (relu_prog && hid < 32 && !opt_on(OPT_NO_PWL)) ? (hid < 16 ? 16 : 32) : 0;
+    out->npad = (relu_prog && hid < 32) ? (hid < 16 ? 16 : 32) : 0;
     p.wslot = 4 * hp > 3 * out->npad ? 4 * hp : 3 * out->npad;
     p.off_w = off; off += n_slots * p.wslot * 4 + (gru ? 40 * 4 : 0); off = align_up(off, 16);
-    if (m->program == GD_PROG_V2_4 && !opt_on(OPT_NO_CTAB) && !opt_on(OPT_NO_RTAB)) {
-        p.rtab_n = (int)opt_int(OPT_RTAB_N, 2048);
-        if (p.rtab_n < 16 || p.rtab_n > 8192) p.rtab_n = 2048;
+    if (m->program == GD_PROG_V2_4 && !opt_on(OPT_NO_CTAB)) {
+        p.rtab_n = kRtabN;
         p.off_rtab = off;
         off += p.rtab_n * 16;
-    }
-    if (m->program == GD_PROG_V2_4 && !opt_on(OPT_NO_CTAB)) {
-        p.ctab_n = (int)opt_int(OPT_CTAB_N, 512);
-        if (p.ctab_n < 16 || p.ctab_n > 4096) p.ctab_n = 512;
+        p.ctab_n = kCtabN;
         p.ctab_R = (float)(g->max_chk_deg > 1 ? g->max_chk_deg - 1 : 1);
         p.off_ctab = off;
         off += p.ctab_n * 16;
@@ -969,38 +955,33 @@ static int plan_decode(const gd_graph* g, const gd_model* m, int64_t B, DecodePl
     const bool fits16 = E64 < 65536 && V < 65535 && C < 65535;
     const int tab_bytes = (int)(9 * E64 + V + C + 2) * 2;
     if (p.ctab_n > 0 && !opt_on(OPT_NO_VTAB)) {
-        const long long ek = opt_int(OPT_VTAB_K, 0);
         // 12 tables x 512 intervals (96 KB): the reference draws p from a list of 10 (decoder_v2_4.py:187).  Measured on B200,
         // rotated d=5, B=65536, 10 distinct priors: direct 3.43 ms; 4 x 1024 3.68 (6 of 10 priors overflow the slots);
         // 12 x 384 1.21; 10..12 x 512..640 0.81 ms.  With 4 distinct priors 4 x 1024 takes 0.69 ms.
-        int vn = (int)opt_int(OPT_VTAB_N, 512);
-        if (vn < 64 || vn > 4096) vn = 512;
         const int64_t per_syn_est = ((int64_t)N + maxvc + 2 * E64) * 4;
-        const int64_t t_without = fits16 ? (smem_max - align_up(off + tab_bytes, 128)) / per_syn_est / 8 * 8 : 0;
+        const int64_t t_without = fits16 ? (g->max_smem_optin - align_up(off + tab_bytes, 128)) / per_syn_est / 8 * 8 : 0;
         // slots: as many (12, 8, 6) as still leave tiles as large as the code gets anyway, up to 16 syndromes (rotated d = 5 / 7
         // and toric L = 5 take 12; rotated d = 11 takes 8, toric L = 11 takes 6).  A tile whose syndromes carry more distinct
         // priors than there are slots takes the direct evaluation as a whole (no mixed warps).
         static const int ks[] = {12, 8, 6};
         for (int ki = 0; ki < 3 && t_without >= 8; ++ki) {
-            int vk = ek > 0 ? (int)ek : ks[ki];
-            if (vk < 1 || vk > 16) vk = ks[ki];
-            const int vbytes = vk * vn * 16 + 16 + 16 * 4 + 128 * 4;
-            const int64_t t_with = (smem_max - align_up(off + vbytes + tab_bytes, 128)) / per_syn_est / 8 * 8;
+            const int vk = ks[ki];
+            const int vbytes = vk * kVtabN * 16 + 16 + 16 * 4 + 128 * 4;
+            const int64_t t_with = (g->max_smem_optin - align_up(off + vbytes + tab_bytes, 128)) / per_syn_est / 8 * 8;
             if (t_with >= 8 && t_with >= (t_without < 16 ? t_without : 16)) {
-                p.vtab_n = vn; p.vtab_k = vk;
-                p.off_vtab = off; off += vk * vn * 16;
+                p.vtab_n = kVtabN; p.vtab_k = vk;
+                p.off_vtab = off; off += vk * kVtabN * 16;
                 p.off_vmeta = off; off += 16 + 16 * 4 + 128 * 4;
                 break;
             }
-            if (ek > 0) break;
         }
     }
     // resident layout first
     int tile = 0, resident = 0, R = 0;
-    if (fits16 && off + tab_bytes < smem_max) {
+    if (fits16 && off + tab_bytes < g->max_smem_optin) {
         const int fixed = align_up(off + tab_bytes, 128);
         const int64_t per_syn = ((int64_t)N + (int64_t)maxvc * (sp2 ? 2 : 1) + 2 * E64) * 4;
-        const int64_t tmax = (smem_max - fixed) / per_syn;
+        const int64_t tmax = (g->max_smem_optin - fixed) / per_syn;
         if (tmax >= 8) {
             // Pick (tile, R, EB): tile = syndromes per CTA, R = threads per syndrome.  Score =
             //   (fraction of the SMs' tile slots doing useful work over all rounds)
@@ -1008,20 +989,16 @@ static int plan_decode(const gd_graph* g, const gd_model* m, int64_t B, DecodePl
             // x w(threads): measured sensitivity of the MUFU-bound inner loop to resident warps
             //   and to the register blocking (profiles/r01_geometry_sweep.txt).
             const int E = (int)E64;
-            const int64_t slots = (int64_t)g->sm_count * out->cps;
             static const int wx[] = {32, 128, 256, 384, 512, 640, 896, 1024};
             static const double wy[] = {0.20, 0.62, 0.80, 0.90, 0.96, 0.985, 1.0, 1.0};
             double best = -1.0;
-            const long long et = opt_int(OPT_TILE, 0), er = opt_int(OPT_R, 0), eb = opt_int(OPT_EB, 0);
-            for (int t = 8; t <= tmax && t <= thr_max; t += 8) {
-                if (et > 0 && et != t) continue;
+            for (int t = 8; t <= tmax && t <= kMaxThreads; t += 8) {
                 if (force && force->tile != t) continue;
                 if (t < 32 && (32 % t)) continue;
                 const int64_t n_t = (B + t - 1) / t;
-                const int64_t rounds = (n_t + slots - 1) / slots;
-                const double eff_round = (double)B / ((double)rounds * (double)slots * t);
-                for (int r = 1; r * t <= thr_max && r <= E; ++r) {
-                    if (er > 0 && er != r) continue;
+                const int64_t rounds = (n_t + g->sm_count - 1) / g->sm_count;
+                const double eff_round = (double)B / ((double)rounds * (double)g->sm_count * t);
+                for (int r = 1; r * t <= kMaxThreads && r <= E; ++r) {
                     if (force && force->R != r) continue;
                     const int thr = r * t;
                     if (thr % 32) continue;
@@ -1036,7 +1013,6 @@ static int plan_decode(const gd_graph* g, const gd_model* m, int64_t B, DecodePl
                     const double node_cost = (double)((V + r - 1) / r) * g->max_var_deg + (double)((Cn + r - 1) / r) * g->max_chk_deg;
                     const double ideal = E * c_edge + 2.0 * E * c_ld;
                     for (int ebk = 4; ebk >= 2; ebk -= 2) {
-                        if (eb > 0 && eb != ebk) continue;
                         if (force && force->eb != ebk) continue;
                         const int blocks = (n_iter + ebk - 1) / ebk;
                         const double per_thread = (bp ? n_iter : blocks * ebk) * c_edge + node_cost * c_ld;
@@ -1068,7 +1044,7 @@ static int plan_decode(const gd_graph* g, const gd_model* m, int64_t B, DecodePl
     p.R = R;
     out->threads = R * tile;
     p.n_tiles = (int)((B + tile - 1) / tile);
-    out->grid = p.n_tiles < g->sm_count * out->cps ? p.n_tiles : g->sm_count * out->cps;
+    out->grid = p.n_tiles < g->sm_count ? p.n_tiles : g->sm_count;
     out->resident = resident;
     return GD_OK;
 }
@@ -1077,14 +1053,10 @@ template <int PROG>
 static int launch_decode(const DecodePlan& pl, cudaStream_t st) {
     void (*k)(const DecodeParams);
     if constexpr (PROG == GD_PROG_V2_4) {
-        // NPOLY: how many of every 4 hidden-unit pairs take the FMA-pipe polynomial lg2 (-1 = scalar MUFU loop).
-        // Measured on B200 (profiles/r01_npoly_sweep.txt): 2 is best (8.70 vs 6.84 M syndromes/s for -1).
-        const int np = (int)opt_int(OPT_NPOLY, 2);
-#define GD_PICK(MT, EBV)                                                                               \
-        (np < 0 ? decode_kernel<PROG, MT, EBV, -1> : np == 3 ? decode_kernel<PROG, MT, EBV, 3> : decode_kernel<PROG, MT, EBV, 2>)
-        if (pl.threads > 512 || pl.cps > 1) k = pl.eb == 2 ? GD_PICK(1024, 2) : GD_PICK(1024, 4);   // the <= 64-register build
-        else k = pl.eb == 2 ? GD_PICK(512, 2) : GD_PICK(512, 4);
-#undef GD_PICK
+        // NPOLY = 2 of every 4 hidden-unit pairs take the FMA-pipe polynomial lg2.  Measured on B200
+        // (profiles/r01_npoly_sweep.txt): 8.70 M syndromes/s against 6.84 M for the scalar MUFU loop.
+        if (pl.threads > 512) k = pl.eb == 2 ? decode_kernel<PROG, 1024, 2, 2> : decode_kernel<PROG, 1024, 4, 2>;   // the <= 64-register build
+        else k = pl.eb == 2 ? decode_kernel<PROG, 512, 2, 2> : decode_kernel<PROG, 512, 4, 2>;
     } else if constexpr (PROG == GD_PROG_CGNNI || PROG == GD_PROG_QGNNI || PROG == GD_PROG_GRU_CA) {
         if (pl.npad == 16) k = pl.threads > 512 ? decode_kernel<PROG, 1024, 2, 16> : decode_kernel<PROG, 512, 2, 16>;
         else if (pl.npad == 32) k = pl.threads > 512 ? decode_kernel<PROG, 1024, 2, 32> : decode_kernel<PROG, 512, 2, 32>;
@@ -1095,8 +1067,8 @@ static int launch_decode(const DecodePlan& pl, cudaStream_t st) {
         else k = pl.eb == 2 ? decode_kernel<PROG, 512, 2, -1> : decode_kernel<PROG, 512, 4, -1>;
     }
     GD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
-    if (pl.p.defer_count && !gd::opt_on(gd::OPT_NO_PDL)) {          // deferred pass of the table kernel: overlap its launch with that kernel's tail
-        GD_CUDA(gd::pdl_launch_on(true, k, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, pl.p));
+    if (pl.p.defer_count) {          // deferred pass of the table kernel: overlap its launch with that kernel's tail
+        GD_CUDA(gd::pdl_launch(k, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, pl.p));
     } else {
         k<<<pl.grid, pl.threads, pl.smem, st>>>(pl.p);
         GD_CUDA(cudaGetLastError());

@@ -46,8 +46,12 @@ struct DecodeParams {
 
 struct DecodePlan {
     DecodeParams p;
-    int threads, grid, smem, resident, cps, eb, npad;
+    int threads, grid, smem, resident, eb, npad;
 };
+
+// Intervals of decoder_v2_4's cubic tables in the edge-owner kernel: check phase, read-out, variable phase.  The edge-owner
+// backward builds its adjoint check table with kCtabN too: it differentiates the function the forward evaluated.
+constexpr int kCtabN = 512, kRtabN = 2048, kVtabN = 512;
 
 // ---- streamed kernels: the edge state lives in a per-CTA slab in global memory ----
 struct StreamParams {

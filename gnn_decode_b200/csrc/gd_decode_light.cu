@@ -556,10 +556,10 @@ void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out,
     const bool ext = prog == GD_PROG_NEURAL_BP || prog == GD_PROG_GRU_CA;
     const bool force = train || opt_on(OPT_FORCE_LIGHT);
     if (prog != GD_PROG_CGNNI && prog != GD_PROG_QGNNI && prog != GD_PROG_BP_QUANTUM && prog != GD_PROG_BP_CLASSICAL && !ext) return;
-    if (prog == GD_PROG_GRU_CA && (m->hidden >= 32 || (m->flags & GD_FLAG_ALL_ITERS) || opt_on(OPT_NO_PWL))) return;
+    if (prog == GD_PROG_GRU_CA && (m->hidden >= 32 || (m->flags & GD_FLAG_ALL_ITERS))) return;
     if (prog == GD_PROG_NEURAL_BP && m->hidden != g->E) return;      // the caller's argument check reports it
     if (train && m->hidden >= 32) { out->why = "hidden >= 32: the MLPs have no piecewise-linear table"; return; }
-    if (!train && (opt_on(OPT_NO_LIGHT) || opt_on(OPT_FORCE_STREAMED))) return;
+    if (!train && opt_on(OPT_FORCE_STREAMED)) return;
     if ((B + 15) / 16 < g->sm_count && !force) return;   // cannot fill the GPU at any tile size: skip the search
     out->why = "code too large for the node-owner kernel (E >= 65536 or V, C >= 65535)";
     if (g->E >= 65536 || g->V >= 65535 || g->C >= 65535) return;
@@ -570,7 +570,7 @@ void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out,
     p.B = B; p.T = m->iters; p.V = g->V; p.C = g->C; p.E = (int)g->E; p.N = g->N; p.tb = g->t;
     p.hid = bp ? 0 : m->hidden;
     p.hp = align_up_l(p.hid, 4);
-    out->npad = (!bp && m->hidden < 32 && (train || !opt_on(OPT_NO_PWL))) ? (m->hidden < 16 ? 16 : 32) : 0;
+    out->npad = (!bp && m->hidden < 32) ? (m->hidden < 16 ? 16 : 32) : 0;
     p.trows = g->E > g->V ? (int)g->E : g->V;                  // the t region doubles as the logit rows lg[V][tile]
     int off = 0;
     p.off_w = off;
@@ -588,11 +588,9 @@ void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out,
     // graphs whose balance falls below 0.3 keep the edge-owner kernel.
     int best_tile = 0, best_cps = 1, best_R = 1;
     double best_cost = 1e300, best_bal = 0.0;
-    const long long et = opt_int(OPT_LTILE, 0), er = opt_int(OPT_LR, 0);
     const int maxn = g->V > g->C ? g->V : g->C;
     std::vector<int> load;
     for (int t = 16; t <= 128; t *= 2) {
-        if (et > 0 && et != t) continue;
         const int64_t smem = fixed + per_syn * t + extra_bytes;
         if (smem > g->max_smem_optin) break;
         const int lanes = t / 4;
@@ -602,7 +600,6 @@ void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out,
         for (int ci = 0; ci < 8; ++ci) {
             const int R = cand[ci];
             if (R < 1 || R > r_max) continue;
-            if (er > 0 && er != R) continue;
             bool dup = false;
             for (int cj = 0; cj < ci; ++cj) dup = dup || cand[cj] == R;
             if (dup) continue;

@@ -133,8 +133,8 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
         // ---- gated pipeline: st[0] = kernel, st[1] = copies in, st[2] = copies out ----
         const gd_launch_info li = gd::route_launch_info(r);
         const int tile = li.tile, n_tiles = li.n_tiles;
-        int n_chunks = (int)std::max<long long>(1, gd::opt_int(gd::OPT_GATE_CHUNKS, 16));   // measured on B200, rotated d=5 B=65536: 4 -> 19.20, 8 -> 19.41, 16 -> 19.55 M syn/s
-        n_chunks = std::min(std::min(n_chunks, gd::kMaxGateChunks), std::max(1, (int)(B / 4096)));
+        // 16 chunks: measured on B200, rotated d=5 B=65536: 4 -> 19.20, 8 -> 19.41, 16 -> 19.55 M syn/s
+        int n_chunks = std::min(16, std::max(1, (int)(B / 4096)));
         const int chunk_tiles = (n_tiles + n_chunks - 1) / n_chunks;
         n_chunks = (n_tiles + chunk_tiles - 1) / chunk_tiles;
         const int64_t per = (int64_t)chunk_tiles * tile;
@@ -153,7 +153,7 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
         // goes undetected the gates time out (seconds), the batch is redone by the chunked pipeline and gating is turned off.
         // (Nsight Compute marks its target with NV_NSIGHT_INJECTION_PORT_BASE / NV_COMPUTE_PROFILER_PERFWORKS_DIR; other
         // injectors use CUDA_INJECTION64_PATH)
-        const bool kernel_first = !gd::opt_on(gd::OPT_LAUNCH_BLOCKING) && !gd::opt_on(gd::OPT_GATE_COPIES_FIRST);
+        const bool kernel_first = !gd::opt_on(gd::OPT_LAUNCH_BLOCKING);
         bool memop_failed = false, launched = false;
         auto launch = [&]() {
             gd::Gate gate{in_flags, out_counts, c->gate_err_dev, epoch, chunk_tiles};

@@ -38,6 +38,8 @@ namespace gd {
 
 constexpr uint32_t kNone = 0xFFFFFFFFu;
 constexpr int kMaxSlots = kLeanMaxSlots;
+constexpr int kLeanCtN = 128;         // check-phase table pieces (replicated per bank group in shared memory)
+constexpr int kLeanVtN = 512;         // base pieces of each variable-phase table (the kernel refines them by powers of 2)
 constexpr int kHdrBytes = 2048;
 constexpr float kBudgetC = 1e-7f;     // check table: feeds the iteration (+ half an fp32 ulp of its values: 6e-8 max|f2|)
 constexpr float kBudgetV = 1e-6f;     // variable table, in units of tanh output (the MUFU tanh it replaces: ~2e-7)
@@ -1182,7 +1184,7 @@ struct LeanMeta {
     int off_ms = 0, off_mi = 0, off_var = 0;   // byte offsets inside the blob (me at 0)
     double balance = 0.0;
 };
-struct LeanGeom { int R = 0, G = 0, NCH = 0, rt_n = 0, ct_n = 0, vt_n = 0; long long opt_epoch = -1; int tpc = -1, sub = -1; bool valid = false; };
+struct LeanGeom { int R = 0, G = 0, NCH = 0, rt_n = 0; long long opt_epoch = -1; int tpc = -1, sub = -1; bool valid = false; };
 // geometry of the training backward: (R, G) for the base table size, and the finest variable-phase table that still seats one group
 struct LeanBwdGeom { int R = 0, G = 0, vt_max = 0, ct_n = 0, rt_n = 0, vt_n = 0, tpc = 0; long long opt_epoch = -1; bool valid = false; };
 // One table set on the device, keyed on the host by (stream, weights pointer, T, table sizes) and VALIDATED on the device
@@ -1374,7 +1376,7 @@ static bool lean_applicable(const gd_graph* g, const gd_model* m) {
 // chosen per graph (and set of parts) from what shared memory can seat at all -- 2048 pieces unless that costs more than one of
 // the (up to 4) groups 1024 pieces would allow -- and never traded against the geometry.  Returns 0 (2048), 1 (1024) or -1.
 static const int kLeanRts[] = {2048, 1024};
-static int lean_rt_choice(gd_graph* g, const std::vector<const LeanSub*>& parts, int ct_n, int vt_n) {
+static int lean_rt_choice(gd_graph* g, const std::vector<const LeanSub*>& parts) {
     const int smem_max = g->max_smem_optin - 1024;
     int ri_all = 0;
     for (const LeanSub* sub : parts) {
@@ -1387,7 +1389,7 @@ static int lean_rt_choice(gd_graph* g, const std::vector<const LeanSub*>& parts,
             if (nch > 32 || nch == 0) continue;
             const int meta = align_up_i(align_up_i(2 * R * nch * 16 + R * nch * 4, 16) + sub->nv * 8, 16);
             for (int ri = 0; ri < 2; ++ri) {
-                const int fixed = align_up_i(meta + (ct_n + 2) * 128 + (kLeanRts[ri] + 2) * 16 + (vt_n + 2) * 128, 128);
+                const int fixed = align_up_i(meta + (kLeanCtN + 2) * 128 + (kLeanRts[ri] + 2) * 16 + (kLeanVtN + 2) * 128, 128);
                 g_cap[ri] = std::max(g_cap[ri], std::min((smem_max - fixed) / (sub->E * 256), std::min(32 / R, 15)));
             }
         }
@@ -1400,15 +1402,11 @@ static int lean_rt_choice(gd_graph* g, const std::vector<const LeanSub*>& parts,
 // the search itself (host work proportional to C * 32^2: done once per graph part and option set, not per call)
 static bool lean_search(gd_graph* g, const LeanSub* sub, int tpc, int ri_fixed, LeanGeom* out) {
     const int E = sub->E, V = sub->nv;
-    const int ct_n = (int)std::min<long long>(1024, std::max<long long>(32, opt_int(OPT_LEAN_CTAB_N, 128)));
-    const int vt_n = (int)std::min<long long>(4096, std::max<long long>(64, opt_int(OPT_LEAN_VTAB_N, 512)));
     const int state = E * 256;
     const int smem_max = g->max_smem_optin - 1024;              // the kernel's static shared memory (tile / row prefixes)
     struct Cand { int R, G, NCH, rt_n; double score; };
     Cand best{0, 0, 0, 0, -1.0};
-    const int* rts = kLeanRts;
     const long long force_R = opt_int(OPT_LEAN_R, 0), force_G = opt_int(OPT_LEAN_G, 0);
-    const long long force_rt = opt_int(OPT_LEAN_RTAB_N, 0);
     std::vector<int> nchs(33, 0);
     std::vector<double> bals(33, 0.0);
     for (int R = 1; R <= 32; ++R) {
@@ -1423,8 +1421,8 @@ static bool lean_search(gd_graph* g, const LeanSub* sub, int tpc, int ri_fixed, 
         const int meta = align_up_i(align_up_i(2 * R * nch * 16 + R * nch * 4, 16) + V * 8, 16);
         for (int ri = ri_fixed; ri <= ri_fixed; ++ri) {
             // shared memory: metadata, check table and ONE variable-phase table replicated per bank group, read-out table
-            const int rt_n = force_rt > 0 ? (int)force_rt : rts[ri];
-            const int fixed = align_up_i(meta + (ct_n + 2) * 128 + (rt_n + 2) * 16 + (vt_n + 2) * 128, 128);
+            const int rt_n = kLeanRts[ri];
+            const int fixed = align_up_i(meta + (kLeanCtN + 2) * 128 + (rt_n + 2) * 16 + (kLeanVtN + 2) * 128, 128);
             int G = (smem_max - fixed) / state;
             G = std::min(G, std::min(32 / R, 15));
             if (force_G > 0) G = G >= force_G ? (int)force_G : 0;
@@ -1449,19 +1447,18 @@ static bool lean_search(gd_graph* g, const LeanSub* sub, int tpc, int ri_fixed, 
         for (int R = best.R + 1; R <= 32 && R * best.G <= 32; ++R) {
             if (nchs[R] == 0 || nchs[R] > best.NCH || max_load(R) > mx0) continue;
             const int meta = align_up_i(align_up_i(2 * R * nchs[R] * 16 + R * nchs[R] * 4, 16) + V * 8, 16);
-            const int fixed = align_up_i(meta + (ct_n + 2) * 128 + (best.rt_n + 2) * 16 + (vt_n + 2) * 128, 128);
+            const int fixed = align_up_i(meta + (kLeanCtN + 2) * 128 + (best.rt_n + 2) * 16 + (kLeanVtN + 2) * 128, 128);
             if ((smem_max - fixed) / state < best.G) continue;
             best.R = R; best.NCH = nchs[R];
         }
     }
     out->valid = true;                                          // "does not fit" is a cached answer too (R == 0)
     out->R = best.R; out->G = best.G; out->NCH = best.NCH; out->rt_n = best.rt_n;
-    out->ct_n = ct_n; out->vt_n = vt_n;
     return true;
 }
 
 static bool lean_fill(gd_graph* g, const LeanSub* sub, const gd_model* m, int64_t B, const LeanGeom& best, const LeanMeta* meta, LeanPlan* out) {
-    const int E = sub->E, V = g->V, ct_n = best.ct_n, vt_n = best.vt_n, state = E * 256;
+    const int E = sub->E, V = g->V, state = E * 256;
     const int smem_max = g->max_smem_optin;
     LeanParams& p = out->p;
     memset(&p, 0, sizeof(p));
@@ -1469,13 +1466,13 @@ static bool lean_fill(gd_graph* g, const LeanSub* sub, const gd_model* m, int64_
     p.nw = (g->C + 31) / 32; p.vw = (V + 31) / 32; p.P = sub->nv | 1;
     p.v_lo = sub->v_lo; p.nv = sub->nv; p.part = sub->id >= 0 ? 1 : 0;
     p.R = best.R; p.G = best.G; p.NCH = meta->NCH;
-    p.ct_n = ct_n; p.rt_n = best.rt_n; p.vt_n = vt_n;
+    p.ct_n = kLeanCtN; p.rt_n = best.rt_n; p.vt_n = kLeanVtN;
     p.meta = meta->dev;
     p.off_me = 0; p.off_ms = meta->off_ms; p.off_mi = meta->off_mi; p.off_var = meta->off_var;
     p.off_ct = (int)meta->bytes;
-    p.off_rt = p.off_ct + (ct_n + 2) * 128;
+    p.off_rt = p.off_ct + (kLeanCtN + 2) * 128;
     p.off_vt = p.off_rt + (best.rt_n + 2) * 16;
-    p.off_state = align_up_i(p.off_vt + (vt_n + 2) * 128, 128);
+    p.off_state = align_up_i(p.off_vt + (kLeanVtN + 2) * 128, 128);
     out->smem = p.off_state + best.G * state;
     out->threads = 32 * best.G * best.R;
     out->n_tiles = (int)((B + 31) / 32);                       // (+ at most one partial tile per distinct prior)
@@ -1496,8 +1493,6 @@ bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>*
     out->clear();
     if (!lean_applicable(g, m)) return false;
     const std::vector<LeanSub*>& subs = lean_subs(g);
-    const int ct_n = (int)std::min<long long>(1024, std::max<long long>(32, opt_int(OPT_LEAN_CTAB_N, 128)));
-    const int vt_n = (int)std::min<long long>(4096, std::max<long long>(64, opt_int(OPT_LEAN_VTAB_N, 512)));
     // tiles of 32 syndromes a CTA will see (one CTA per SM; large batches: the quantisation no longer matters)
     const int tpc = (int)std::min<long long>(64, std::max<long long>(1, ((B + 31) / 32 + g->sm_count - 1) / g->sm_count));
     LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
@@ -1510,11 +1505,11 @@ bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>*
     if (mode == -2) {
         int modes[2], ris[2];
         // (nv | 1) <= E: the staged logits reuse the free message buffer
-        const int ri_whole = (subs[0]->nv | 1) <= subs[0]->E ? lean_rt_choice(g, {subs[0]}, ct_n, vt_n) : -1;
+        const int ri_whole = (subs[0]->nv | 1) <= subs[0]->E ? lean_rt_choice(g, {subs[0]}) : -1;
         std::vector<const LeanSub*> comps(subs.begin() + 1, subs.end());
         bool comps_ok = !comps.empty();
         for (const LeanSub* c : comps) comps_ok = comps_ok && (c->nv | 1) <= c->E;
-        const int ri_comps = comps_ok ? lean_rt_choice(g, comps, ct_n, vt_n) : -1;
+        const int ri_comps = comps_ok ? lean_rt_choice(g, comps) : -1;
         const long long want = opt_int(OPT_LEAN_PARTS, -1);
         modes[1] = ri_whole >= 0 ? 0 : -1; ris[1] = ri_whole;                       // training: whole graph or nothing
         if (ri_comps >= 0 && (ri_whole < 0 || want == 1) && want != 0) { modes[0] = 1; ris[0] = ri_comps; }
@@ -1553,12 +1548,6 @@ bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>*
         out->push_back(pl);
     }
     return !out->empty();
-}
-
-// the passes of a decode call follow one another by programmatic dependent launch (gd_common.cuh: pdl_enter / pdl_launch_on)
-template <typename P>
-static cudaError_t pdl_launch(void (*kern)(const P), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const P& params) {
-    return pdl_launch_on(!opt_on(OPT_NO_PDL), kern, grid, block, smem, st, params);
 }
 
 static cudaMemPool_t lean_pool(gd_graph* g) {
@@ -1831,11 +1820,13 @@ int packed_via_unpack(gd_graph* g, const float* prior_dev, const uint32_t* synd_
     return GD_OK;
 }
 
+// adjoint bins of the table backward with an rt_n-piece read-out table: [2][nodes] 64-bit bins of the three tables
+static int64_t lean_bins_floats(int rt_n) {
+    return 2 * 2 * ((int64_t)(kLeanCtN + 3) + (rt_n + 3) + (int64_t)kMaxSlots * (4 * kLeanVtN + 3));
+}
+
 int64_t lean_bwd_bins_floats(const gd_graph* g, const gd_model* model) {
-    if (!lean_applicable(g, model)) return 0;
-    const int ct_n = (int)std::min<long long>(1024, std::max<long long>(32, opt_int(OPT_LEAN_CTAB_N, 128)));
-    const int vt_n = (int)std::min<long long>(4096, std::max<long long>(64, opt_int(OPT_LEAN_VTAB_N, 512)));
-    return 2 * 2 * ((int64_t)(ct_n + 3) + (2048 + 3) + (int64_t)kMaxSlots * (4 * vt_n + 3));   // [2][nodes] 64-bit bins
+    return lean_applicable(g, model) ? lean_bins_floats(kLeanRts[0]) : 0;   // the larger read-out table
 }
 
 int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const float* weights_dev, const float* x_dev,
@@ -1878,13 +1869,12 @@ int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const
     p.off_vt = p.off_rt + (rt_n + 2) * 16;
     const int smem = g->max_smem_optin - 1024;                  // all of it: the kernel lays the rest out for the table size in use
     p.smem = smem;
-    const size_t bins_bytes = (size_t)2 * 8 * ((ct_n + 3) + (rt_n + 3) + (size_t)kMaxSlots * (4 * vt_n + 3));
-    GD_CUDA(cudaMemsetAsync(bins_dev, 0, bins_bytes, st));
+    GD_CUDA(cudaMemsetAsync(bins_dev, 0, (size_t)lean_bins_floats(rt_n) * sizeof(float), st));
     GD_CUDA(cudaFuncSetAttribute(lean_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    GD_CUDA(pdl_launch_on(!opt_on(OPT_NO_PDL), lean_bwd_kernel, dim3(g->sm_count), dim3(32 * bestG * bestR), (size_t)smem, st, p));
+    GD_CUDA(pdl_launch(lean_bwd_kernel, dim3(g->sm_count), dim3(32 * bestG * bestR), (size_t)smem, st, p));
     ContractParams cp{weights_dev, hdr, reinterpret_cast<const long long*>(bins_dev), grad_weights_dev, model->hidden, model->iters,
                       ct_n, rt_n, vt_n, accumulate};
-    GD_CUDA(pdl_launch_on(!opt_on(OPT_NO_PDL), lean_contract_kernel, dim3(3 * (model->hidden + 1)), dim3(256), 0, st, cp));
+    GD_CUDA(pdl_launch(lean_contract_kernel, dim3(3 * (model->hidden + 1)), dim3(256), 0, st, cp));
     return GD_OK;
 }
 

@@ -7,7 +7,6 @@
 // directly in the layout the backward kernel reads.  Per-syndrome losses are written out and summed
 // by the caller in a fixed order (deterministic).
 #include "gd_common.cuh"
-#include "gd_options.cuh"
 
 namespace gd {
 
@@ -79,8 +78,8 @@ extern "C" int gd_loss_v2_4(const gd_graph* g, const uint8_t* logical_dev, int32
     cudaError_t e = cudaSuccess;
     if (smem > 48 * 1024) e = cudaFuncSetAttribute(gd::loss_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e == cudaSuccess) {
-        e = gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::loss_kernel, dim3((unsigned)blocks), dim3(128), (size_t)smem, (cudaStream_t)stream,
-                              prob_dev, y_dev, logical_dev, K, g->t, B, g->V, g->C, loss_per_syndrome_dev, grad_prob_dev, grad_logit_dev);
+        e = gd::pdl_launch(gd::loss_kernel, dim3((unsigned)blocks), dim3(128), (size_t)smem, (cudaStream_t)stream,
+                           prob_dev, y_dev, logical_dev, K, g->t, B, g->V, g->C, loss_per_syndrome_dev, grad_prob_dev, grad_logit_dev);
     }
     GD_CUDA(e);
     return GD_OK;

@@ -3,7 +3,6 @@
 // 12 parameter tensors.  The data-parallel variant fuses the same update into the peer-memory all-reduce (gd_p2p.cu).
 #include "gd_adam.cuh"
 #include "gd_common.cuh"
-#include "gd_options.cuh"
 #include <algorithm>
 
 namespace gd {
@@ -28,8 +27,8 @@ extern "C" int gd_adam_step(const gd_adam* opt, float* weights_dev, const float*
                  && opt->weight_decay >= 0., "gd_adam_step: invalid hyper-parameters");
     const gd::AdamCoef c = gd::adam_coef(opt->lr, opt->beta1, opt->beta2, opt->eps, opt->weight_decay, opt->step);
     const int grid = (int)std::min<int64_t>((n + 255) / 256, 1184);
-    GD_CUDA(gd::pdl_launch_on(!gd::opt_on(gd::OPT_NO_PDL), gd::adam_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, c, weights_dev, grad_dev, exp_avg_dev,
-                              exp_avg_sq_dev, grad_scale, (long long)n));
+    GD_CUDA(gd::pdl_launch(gd::adam_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, c, weights_dev, grad_dev, exp_avg_dev,
+                           exp_avg_sq_dev, grad_scale, (long long)n));
     GD_CUDA(cudaGetLastError());
     return GD_OK;
 }

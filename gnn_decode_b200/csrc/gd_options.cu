@@ -9,11 +9,8 @@
 namespace gd {
 
 static const char* const kOptNames[OPT_COUNT] = {
-    "GD_CPS", "GD_NO_PWL", "GD_NO_CTAB", "GD_NO_RTAB", "GD_NO_VTAB", "GD_RTAB_N", "GD_CTAB_N", "GD_VTAB_N", "GD_VTAB_K",
-    "GD_TILE", "GD_R", "GD_EB", "GD_FORCE_STREAMED", "GD_NPOLY", "GD_NO_VSKIP", "GD_NO_DIRECT", "GD_NO_LIGHT",
-    "GD_FORCE_LIGHT", "GD_LTILE", "GD_LR", "GD_NO_GATED_HOST", "GD_GATE_CHUNKS", "GD_GATE_COPIES_FIRST", "GD_STILE",
-    "GD_STHREADS", "GD_STREAM_LEGACY", "GD_SROWS", "GD_SSTAGES", "GD_SWARPS", "GD_NO_BWD_CTAB", "GD_NO_LEAN", "GD_LEAN_R",
-    "GD_LEAN_G", "GD_LEAN_VTAB_N", "GD_LEAN_CTAB_N", "GD_LEAN_RTAB_N", "GD_LEAN_PARTS", "GD_NO_PDL", "GD_LAUNCH_BLOCKING"};
+    "GD_NO_CTAB", "GD_NO_VTAB", "GD_FORCE_STREAMED", "GD_NO_VSKIP", "GD_FORCE_LIGHT", "GD_NO_GATED_HOST", "GD_NO_LEAN",
+    "GD_LEAN_R", "GD_LEAN_G", "GD_LEAN_PARTS", "GD_LAUNCH_BLOCKING"};
 
 static std::atomic<long long> g_opt[OPT_COUNT];
 static std::once_flag g_opt_once;

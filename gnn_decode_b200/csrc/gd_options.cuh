@@ -6,44 +6,16 @@
 namespace gd {
 
 enum Opt {
-    OPT_CPS = 0,          // GD_CPS            CTAs per SM of the edge-owner resident kernel (1)
-    OPT_NO_PWL,           // GD_NO_PWL         ReLU MLPs as FMA sums instead of piecewise-linear tables
     OPT_NO_CTAB,          // GD_NO_CTAB        decoder_v2_4 check-phase MLP evaluated directly
-    OPT_NO_RTAB,          // GD_NO_RTAB        decoder_v2_4 read-out MLP evaluated directly
     OPT_NO_VTAB,          // GD_NO_VTAB        decoder_v2_4 variable-phase MLP evaluated directly
-    OPT_RTAB_N,           // GD_RTAB_N         read-out table intervals (2048)
-    OPT_CTAB_N,           // GD_CTAB_N         check-phase table intervals (512)
-    OPT_VTAB_N,           // GD_VTAB_N         variable-phase table intervals (512)
-    OPT_VTAB_K,           // GD_VTAB_K         variable-phase table slots (12 / 8 / 6 by code size)
-    OPT_TILE,             // GD_TILE           force the edge-owner kernel's tile
-    OPT_R,                // GD_R              force its threads per syndrome
-    OPT_EB,               // GD_EB             force its register blocking
     OPT_FORCE_STREAMED,   // GD_FORCE_STREAMED take the streamed global-memory kernel even when the state fits on chip
-    OPT_NPOLY,            // GD_NPOLY          hidden-unit pairs of 4 whose lg2 runs on the FMA pipe (2)
     OPT_NO_VSKIP,         // GD_NO_VSKIP       re-evaluate degree-1 variables every iteration
-    OPT_NO_DIRECT,        // GD_NO_DIRECT      node-sum passes instead of direct sibling reads
-    OPT_NO_LIGHT,         // GD_NO_LIGHT       light programs on the edge-owner kernel
     OPT_FORCE_LIGHT,      // GD_FORCE_LIGHT    node-owner kernel even where the planner declines
-    OPT_LTILE,            // GD_LTILE          node-owner kernel tile
-    OPT_LR,               // GD_LR             node-owner kernel thread groups
     OPT_NO_GATED_HOST,    // GD_NO_GATED_HOST  chunked host pipeline instead of the gated single launch
-    OPT_GATE_CHUNKS,      // GD_GATE_CHUNKS    chunks of the gated host pipeline (16)
-    OPT_GATE_COPIES_FIRST,// GD_GATE_COPIES_FIRST enqueue copies before the gated kernel
-    OPT_STILE,            // GD_STILE          streamed kernels: tile
-    OPT_STHREADS,         // GD_STHREADS       register-batched streamed kernel: threads
-    OPT_STREAM_LEGACY,    // GD_STREAM_LEGACY  register-batched streamed kernel instead of the TMA pipeline
-    OPT_SROWS,            // GD_SROWS          TMA streamed kernel: rows per stage
-    OPT_SSTAGES,          // GD_SSTAGES        TMA streamed kernel: stages
-    OPT_SWARPS,           // GD_SWARPS         TMA streamed kernel: warps
-    OPT_NO_BWD_CTAB,      // GD_NO_BWD_CTAB    backward: per-unit check-phase MLP instead of the adjoint table
     OPT_NO_LEAN,          // GD_NO_LEAN        decoder_v2_4 on surface/toric codes: skip the table-only check-owner kernel
     OPT_LEAN_R,           // GD_LEAN_R         its owners (warps) per group of 32 syndromes
     OPT_LEAN_G,           // GD_LEAN_G         its groups per CTA
-    OPT_LEAN_VTAB_N,      // GD_LEAN_VTAB_N    its variable-phase table intervals (512)
-    OPT_LEAN_CTAB_N,      // GD_LEAN_CTAB_N    its check-phase table intervals (128, replicated per bank group)
-    OPT_LEAN_RTAB_N,      // GD_LEAN_RTAB_N    its read-out table intervals (2048)
     OPT_LEAN_PARTS,       // GD_LEAN_PARTS     1: decode the graph's connected components in separate launches, 0: never (unset: when that seats more groups)
-    OPT_NO_PDL,           // GD_NO_PDL         launch the table kernel's passes without programmatic dependent launch
     OPT_LAUNCH_BLOCKING,  // (derived) a tool that makes launches block the host is attached (ncu / sanitizer / CUDA_LAUNCH_BLOCKING)
     OPT_COUNT
 };

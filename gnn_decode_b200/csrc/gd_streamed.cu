@@ -293,7 +293,7 @@ int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* o
     out->smem = n_slots * 4 * p.hp * 4 + 16;
     if (m->program == GD_PROG_V2_4 && !opt_on(OPT_NO_CTAB)) {
         p.ctab_n = 512;
-        p.rtab_n = opt_on(OPT_NO_RTAB) ? 0 : 2048;
+        p.rtab_n = 2048;
         p.ctab_R = (float)(g->max_chk_deg > 1 ? g->max_chk_deg - 1 : 1);
         const int big = p.ctab_n > p.rtab_n ? p.ctab_n : p.rtab_n;
         out->smem += (p.ctab_n + p.rtab_n) * 16 + (big + 8) * 4 + 16;
@@ -309,11 +309,8 @@ int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* o
             if (eff > best + 1e-9) { best = eff; tile = t; }
         }
     }
-    if (opt_on(OPT_STILE)) tile = (int)opt_int(OPT_STILE, tile);
-    if (tile < 8 || tile > 512 || (tile % 8)) tile = 32;
     p.tile = tile;
-    int maxthr = 1024;
-    maxthr = (int)opt_int(OPT_STHREADS, maxthr);
+    const int maxthr = 1024;
     int R = maxthr / tile;
     const int maxn = g->V > g->C ? g->V : g->C;
     if (R > maxn) R = maxn;

@@ -437,7 +437,6 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
     StreamTmaParams& p = out->p;
     memset(&p, 0, sizeof(p));
     out->ok = false;
-    if (opt_on(OPT_STREAM_LEGACY)) return;
     for (size_t i = 0; i < g->h_var_edges.size(); ++i)
         if (g->h_var_edges[i] != (int32_t)i) return;
     const bool bp = m->program == GD_PROG_BP_QUANTUM || m->program == GD_PROG_BP_CLASSICAL;
@@ -450,7 +449,7 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
     // batch fills all 32 lanes of every SM; smaller batches take the register-batched kernel.
     if (m->program == GD_PROG_V2_4 && B < (int64_t)128 * g->sm_count) return;
     out->npad = 0;
-    if ((m->program == GD_PROG_CGNNI || m->program == GD_PROG_QGNNI) && m->hidden < 32 && !opt_on(OPT_NO_PWL))
+    if ((m->program == GD_PROG_CGNNI || m->program == GD_PROG_QGNNI) && m->hidden < 32)
         out->npad = m->hidden < 16 ? 16 : 32;
     // tile: multiple of 4 (a lane owns one float4 of a row), <= 128.  Cost model: the kernel is
     // HBM-bound, a tile's time ~ its bytes ~ tile (with a floor: a warp instruction costs the
@@ -465,18 +464,13 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
             if (cost <= best * (1.0 + 1e-12)) { best = cost; tile = t; }
         }
     }
-    const long long et = opt_int(OPT_STILE, 0);
-    if (et >= 4 && et <= 128 && et % 4 == 0) tile = (int)et;
     p.tile = tile;
     p.lanes = tile / 4;
     const int vd = g->max_var_deg > 0 ? g->max_var_deg : 1;
     // rows per stage: a check item needs deg (+ deg residual rows for the learned programs) + 1; the sum-product family
     // could do with half, but bigger stages amortise the per-item cost better (variables per item K = rows / (vd + 1)):
     // measured on B200, sum-product / HGP-1600 / T = 50: 15 rows x 2 stages 28.4 ms, 8 rows x 2 / 3 / 4 stages 33.7 / 32.9 / 33.2 ms
-    const int min_rows = (bp ? 1 : 2) * g->max_chk_deg + 1;
     int rows = 2 * g->max_chk_deg + 1;
-    const long long er = opt_int(OPT_SROWS, 0);
-    if (er >= min_rows && er <= 64) rows = (int)er;
     if (rows < vd + 1) rows = vd + 1;
     int K = rows / (vd + 1);
     if (K > 8) K = 8;
@@ -491,23 +485,16 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
         p.ctab_n = (int)(512.0f * p.ctab_R / 3.0f + 0.5f);
         if (p.ctab_n < 512) p.ctab_n = 512;
         p.off_ctab = off; off += p.ctab_n * 16;
-        if (!opt_on(OPT_NO_RTAB)) { p.rtab_n = 2048; p.off_rtab = off; off += p.rtab_n * 16; }
+        p.rtab_n = 2048; p.off_rtab = off; off += p.rtab_n * 16;
     }
     p.off_stage = off;
-    // stages per warp (2..4, GD_SSTAGES): 2 unless deeper still leaves room for all 16 warps at this stage size
+    // stages per warp (2..4): 2 unless deeper still leaves room for all 16 warps at this stage size
     int S = 2;
-    {
-        const long long es = opt_int(OPT_SSTAGES, 0);
-        if (es >= 2 && es <= 4) S = (int)es;
-        else
-            for (int q = 4; q > 2; --q)
-                if ((g->max_smem_optin - off) / (q * stage_bytes) >= 16) { S = q; break; }
-    }
+    for (int q = 4; q > 2; --q)
+        if ((g->max_smem_optin - off) / (q * stage_bytes) >= 16) { S = q; break; }
     p.S = S;
     int Wn = (g->max_smem_optin - off) / (S * stage_bytes);
     if (Wn > 16) Wn = 16;
-    const long long ew = opt_int(OPT_SWARPS, 0);
-    if (ew >= 1 && ew < Wn) Wn = (int)ew;
     if (Wn < 2) return;
     if ((int64_t)Wn * S * rows * tile < 2 * (int64_t)(tile + 2) * 2) return;   // transposition scratch
     p.W = Wn;

@@ -345,7 +345,7 @@ int gd_eval_failures(const gd_graph* g, const uint8_t* logical_dev, int32_t K,
  *      result[0] = units / s over the whole GPU, result[1] = ms of the timed launch. ---- */
 int gd_microbench(int32_t kind, int32_t iters, int device, double* result);
 
-/* ---- library tunables.  Every planner switch (GD_NO_LEAN, GD_FORCE_STREAMED, GD_TILE, ... -- the list is in
+/* ---- library tunables.  Every planner switch (GD_NO_LEAN, GD_FORCE_STREAMED, GD_LEAN_R, ... -- the list is in
  *      gnn_decode_b200/csrc/gd_options.cuh) lives in one table that is filled from the environment ONCE, at first use;
  *      nothing on the launch path reads the environment.  gd_set_option changes an entry at run time (unset != 0:
  *      back to "not given").  Returns GD_ERR_INVALID for an unknown name. ---- */

@@ -1,5 +1,5 @@
-"""Hard-decision agreement and logical error rate of the tabulated (default) vs direct (GD_NO_CTAB=1 GD_NO_VSKIP=1
-GD_NO_DIRECT=1) evaluation paths of the decoder_v2_4 kernel on 2^20 sampled syndromes (rotated d=5, depolarizing)."""
+"""Hard-decision agreement and logical error rate of the tabulated (default) vs direct (GD_NO_CTAB=1 GD_NO_VSKIP=1)
+evaluation paths of the decoder_v2_4 kernel on 2^20 sampled syndromes (rotated d=5, depolarizing)."""
 import os, sys, subprocess, numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 if len(sys.argv) > 1:
@@ -21,7 +21,7 @@ if len(sys.argv) > 1:
     cnt = count_failures(g, err, hard, codes.css_logicals(Hz, Hx)).tolist()
     torch.save({"hard": hard.cpu(), "logit": logit.cpu(), "cnt": cnt}, sys.argv[1])
 else:
-    env_b = dict(os.environ, GD_NO_CTAB="1", GD_NO_VSKIP="1", GD_NO_DIRECT="1")
+    env_b = dict(os.environ, GD_NO_CTAB="1", GD_NO_VSKIP="1")
     subprocess.run([sys.executable, __file__, "/tmp/ler_a.pt"], check=True)
     subprocess.run([sys.executable, __file__, "/tmp/ler_b.pt"], check=True, env=env_b)
     a, b = torch.load("/tmp/ler_a.pt"), torch.load("/tmp/ler_b.pt")

@@ -1,9 +1,11 @@
 """Tiny run of every kernel family, meant to be executed under compute-sanitizer (memcheck / racecheck / synccheck):
     compute-sanitizer --tool racecheck python scripts/sanitize_smoke.py
-Sizes are small; each launch still covers ragged tiles and every phase."""
+Sizes are small; each launch still covers ragged tiles and every phase.  300 syndromes cannot fill the GPU, so the light
+programs take the edge-owner kernel unless GD_FORCE_LIGHT is set, and decoder_v2_4 (below 128 syndromes per SM) takes the
+register-batched streamed kernel under GD_FORCE_STREAMED."""
 import os, sys, numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from gnn_decode_b200 import codes
+from gnn_decode_b200 import codes, options
 from gnn_decode_b200.evaluate import count_failures
 from gnn_decode_b200.graph import TannerGraph
 from gnn_decode_b200.quantum import decoder_v2_4, QGNNI, BP, neural_BP, QGNNNI_ca
@@ -12,7 +14,7 @@ from gnn_decode_b200.sampler import sample_syndromes
 from gnn_decode_b200.train import train_step_grads
 
 dev = torch.device("cuda", 0)
-which = sys.argv[1:] or ["resident", "light", "streamed", "legacy", "train", "misc"]
+which = sys.argv[1:] or ["resident", "light", "streamed", "train", "misc"]
 Hz, Hx = codes.rotated_surface_checks(3)
 pcm = codes.css_pcm(Hz, Hx)
 g = TannerGraph.from_pcm(pcm, dev)
@@ -22,32 +24,24 @@ xt, _ = sample_syndromes(gt, 300, [0.05], noise=0, seed=2)
 torch.manual_seed(0)
 progs = [decoder_v2_4.GNNI(3), QGNNI.GNNI(3), BP.GNNI(3), neural_BP.GNNI(3, n_edges=int(pcm.sum())), QGNNNI_ca.GNNI(3)]
 if "resident" in which:
-    os.environ["GD_NO_LIGHT"] = "1"
     for d in progs:
         d.to(dev).eval().decode(x, graph=g, return_hard=True)
     CGNNI.GNNI(3).to(dev).eval().decode(xt, graph=gt)
-    os.environ.pop("GD_NO_LIGHT")
     print("resident ok", flush=True)
 if "light" in which:
-    os.environ["GD_FORCE_LIGHT"] = "1"
-    for d in (QGNNI.GNNI(3), BP.GNNI(3)):
-        d.to(dev).eval().decode(x, graph=g, return_logits=True)
-    CGNNI.GNNI(3).to(dev).eval().decode(xt, graph=gt)
-    os.environ.pop("GD_FORCE_LIGHT")
+    with options.option("GD_FORCE_LIGHT"):
+        for d in (QGNNI.GNNI(3), BP.GNNI(3)):
+            d.to(dev).eval().decode(x, graph=g, return_logits=True)
+        CGNNI.GNNI(3).to(dev).eval().decode(xt, graph=gt)
     print("light ok", flush=True)
 if "streamed" in which:
-    os.environ["GD_FORCE_STREAMED"] = "1"
-    for d in (QGNNI.GNNI(3), BP.GNNI(3)):
-        d.to(dev).eval().decode(x, graph=g, return_hard=True)
-    CGNNI.GNNI(3).to(dev).eval().decode(xt, graph=gt)
-    print("streamed (TMA) ok", flush=True)
-    if "legacy" in which:
-        os.environ["GD_STREAM_LEGACY"] = "1"
-        for d in (decoder_v2_4.GNNI(2), QGNNI.GNNI(2), BP.GNNI(2)):
+    with options.option("GD_FORCE_STREAMED"):
+        for d in (QGNNI.GNNI(3), BP.GNNI(3)):
             d.to(dev).eval().decode(x, graph=g, return_hard=True)
-        os.environ.pop("GD_STREAM_LEGACY")
+        CGNNI.GNNI(3).to(dev).eval().decode(xt, graph=gt)
+        print("streamed (TMA) ok", flush=True)
+        decoder_v2_4.GNNI(2).to(dev).eval().decode(x, graph=g, return_hard=True)
         print("streamed (register-batched) ok", flush=True)
-    os.environ.pop("GD_FORCE_STREAMED")
 if "train" in which:
     dec = decoder_v2_4.GNNI(3).to(dev).train()
     train_step_grads(dec, g, x, err, codes.css_logicals(Hz, Hx))
