@@ -13,7 +13,7 @@ PROG_NEURAL_BP, PROG_GRU_CA = 5, 6
 PROG_V3_0, PROG_V1_2_2, PROG_V2_4_1 = 7, 8, 9
 FLAG_ALL_ITERS = 1
 PHASE_VAR, PHASE_CHK = 0, 1
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 
 class GdModel(C.Structure):
@@ -55,7 +55,6 @@ _SIGNATURES = {
     "gd_pipeline_wait": (C.c_int, [_p, C.c_int32]),
     "gd_pipeline_drain": (C.c_int, [_p]),
     "gd_decode_host": (C.c_int, [_p, C.POINTER(GdModel), _p, _p, _p, _p, C.c_int64]),
-    "gd_decode_host_last_launches": (C.c_int, [_p]),
     "gd_decode_tables_info": (C.c_int, [_p, C.POINTER(GdModel), C.c_int64, C.POINTER(C.c_int32)]),
     "gd_decode_launch_info": (C.c_int, [_p, C.POINTER(GdModel), C.c_int64, C.POINTER(GdLaunchInfo)]),
     "gd_decode_autotune": (C.c_int, [_p, C.POINTER(GdModel), _p, _p, C.c_int64, C.c_int32, _p, C.POINTER(GdLaunchInfo)]),

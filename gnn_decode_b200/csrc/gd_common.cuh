@@ -104,7 +104,7 @@ struct gd_graph {
     gd::GraphTables t;          // device pointers into blob_dev
     std::vector<int32_t> h_edge_var, h_edge_chk, h_var_ptr, h_var_edges, h_chk_ptr, h_chk_edges, h_vlist;
     // lazily grown scratch (guarded by mu): global edge-state workspace for codes too large
-    // for shared memory, and pinned/device staging for gd_decode_host.
+    // for shared memory, and gd_decode_host's internal pipeline.
     std::mutex mu;
     float* gstate;
     size_t gstate_bytes;

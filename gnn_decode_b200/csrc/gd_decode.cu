@@ -368,10 +368,6 @@ __global__ void __launch_bounds__(MAXT, 1) decode_kernel(const DecodeParams p) {
         const float* xg = p.x + s0 * N;
         const int n_in = nvalid * N;
         const uint32_t bulk_bytes = didx ? 0u : ((uint32_t)n_in * 4u) & ~15u;
-        if (p.gate_in) {   // gated launch: this tile's chunk may still be on its way from the host
-            if (tid == 0) gate_wait(p.gate_in + tix / p.gate_chunk_tiles, p.gate_epoch, p.gate_err);
-            __syncthreads();
-        }
         // ---- input slab: one bulk async copy (TMA) + scalar tail; zero the state ----
         if (tid == 0) {
             fence_proxy_async();  // order earlier generic reads of xs before the async write
@@ -886,13 +882,6 @@ __global__ void __launch_bounds__(MAXT, 1) decode_kernel(const DecodeParams p) {
             }
         }
         if (!((kGRU || kV122) && p.all_iters)) emit(0);
-        if (p.gate_out) {   // gated launch: publish the tile so the chunk's device->host copy can go
-            __syncthreads();
-            if (tid == 0) {
-                __threadfence_system();
-                atomicAdd(p.gate_out + tix / p.gate_chunk_tiles, 1u);
-            }
-        }
     }
 }
 
@@ -1076,16 +1065,12 @@ static int launch_decode(const DecodePlan& pl, cudaStream_t st) {
     return GD_OK;
 }
 
-int edge_decode(const gd_graph* g, const gd_model* model, DecodePlan pl, const DecodeIO& io, cudaStream_t st, const Gate* gate,
+int edge_decode(const gd_graph* g, const gd_model* model, DecodePlan pl, const DecodeIO& io, cudaStream_t st,
                 const DeferList* dl) {
     pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
     pl.p.stash = io.stash; pl.p.hard_bits = io.hard_bits;
     pl.p.aux_prob = io.aux_prob; pl.p.aux_logit = io.aux_logit;
     if (dl) { pl.p.defer_count = dl->count; pl.p.defer_idx = dl->idx; }
-    if (gate) {
-        pl.p.gate_in = gate->in_flags; pl.p.gate_out = gate->out_counts; pl.p.gate_err = gate->err;
-        pl.p.gate_epoch = gate->epoch; pl.p.gate_chunk_tiles = gate->chunk_tiles;
-    }
     switch (model->program) {
         case GD_PROG_CGNNI: return launch_decode<GD_PROG_CGNNI>(pl, st);
         case GD_PROG_QGNNI: return launch_decode<GD_PROG_QGNNI>(pl, st);
@@ -1211,8 +1196,7 @@ int packed_run(void* ctx, const float* x_dev) {
 }
 }  // namespace
 
-int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const DecodeIO& io, int64_t B, cudaStream_t st,
-                  const Gate* gate) {
+int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const DecodeIO& io, int64_t B, cudaStream_t st) {
     switch (r.family) {
         case Family::Lean: {
             bool no_resources = false;
@@ -1222,7 +1206,7 @@ int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const Deco
             // The edge-owner kernel decodes the whole batch instead.
             break;
         }
-        case Family::Light: return light_decode(r.light, model, io, st, gate);
+        case Family::Light: return light_decode(r.light, model, io, st);
         case Family::StreamedTma: return streamed_tma_decode(g, r.tma, model, io, st);
         case Family::Streamed: return streamed_decode(g, r.streamed, model, io, st);
         case Family::EdgeOwner: break;
@@ -1231,7 +1215,7 @@ int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const Deco
         PackedRun run{g, model, &r.edge, &io, st};
         return packed_via_unpack(g, io.prior, io.synd, B, st, packed_run, &run);
     }
-    return edge_decode(g, model, r.edge, io, st, gate);
+    return edge_decode(g, model, r.edge, io, st);
 }
 
 }  // namespace gd

@@ -30,12 +30,6 @@ struct DecodeParams {
     // meets (inputs made like the reference's gen_syn carry one prior per syndrome, drawn from a short list)
     int vtab_n, vtab_k, off_vtab, off_vmeta;
     int off_w, off_tab, off_x, off_node, off_m, off_t;
-    // gated launch (gd_decode_host, see Gate below); all NULL / 0 otherwise
-    const unsigned int* gate_in;
-    unsigned int* gate_out;
-    int* gate_err;
-    unsigned int gate_epoch;
-    int gate_chunk_tiles;
     // deferred pass behind the check-owner table kernel (gd_lean.cu): decode only the listed syndromes (*defer_count > 0),
     // the whole batch (-1) or nothing (0); all NULL otherwise
     const int* defer_count;
@@ -107,31 +101,6 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
 // the per-graph edge-state slab both streamed kernels use, grown to at least `bytes` (NULL and gd_last_error() on failure)
 float* streamed_slab(gd_graph* g, size_t bytes);
 
-// Gated whole-batch launch for gd_decode_host (gd_host.cu): ONE persistent launch over the full batch whose tiles wait for
-// the host->device copy of their chunk (in_flags[k] >= epoch, raised by a stream memory operation behind the copy) and
-// count completed tiles per chunk (out_counts[k]) so the device->host copy of a chunk can start as soon as its last tile is
-// out.  The edge-owner resident kernel and the node-owner kernel support it.
-struct Gate {
-    const unsigned int* in_flags;
-    unsigned int* out_counts;
-    int* err;                    // host-mapped: set to 1 if a chunk never arrived (bounded spin)
-    unsigned int epoch;
-    int chunk_tiles;             // tiles per chunk: chunk of tile t = t / chunk_tiles
-};
-#ifdef __CUDACC__
-// wait until the chunk's host->device copy has landed (flag raised in stream order behind the copy); bounded
-__device__ __forceinline__ void gate_wait(const unsigned int* flag, unsigned int epoch, int* err) {
-    long long spins = 0;
-    while (true) {
-        unsigned int v;
-        asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-        if ((int)(v - epoch) >= 0) break;
-        if (++spins > (1ll << 22)) { *err = 1; break; }   // seconds: the copy never came; do not hang the GPU
-        __nanosleep(100);
-    }
-}
-#endif
-
 // ---- routing ----
 // The buffers of one decode call; NULL where the call does not ask for them.
 struct DecodeIO {
@@ -146,7 +115,7 @@ struct DecodeIO {
 enum class Family { Lean, Light, EdgeOwner, StreamedTma, Streamed };
 
 enum class Use {
-    Infer,      // gd_decode_fwd(_aux), gd_decode_host (its gated launch too), the launch / table queries, the autotuner
+    Infer,      // gd_decode_fwd(_aux), gd_decode_host, the launch / table queries, the autotuner
     Packed,     // gd_decode_packed_fwd: decoder_v2_4 on the resident kernels only
     Train,      // gd_decode_fwd_train
     TrainBwd,   // gd_decode_bwd: the same family as Train; the backward kernels lay out their own shared memory
@@ -165,21 +134,16 @@ struct Route {
 // programs or codes no kernel serves).  Runs on the graph's device: the table kernel's planning uploads metadata.
 int route_decode(const gd_graph* g, const gd_model* model, int64_t B, Use use, Route* out);
 gd_launch_info route_launch_info(const Route& r);
-// A gated whole-batch launch can serve this route (gd_decode_host).
-inline bool route_gated(const Route& r, const gd_model* model) {
-    return model->flags == 0 && (r.family == Family::Light || r.family == Family::EdgeOwner);
-}
 // Launches the routed family on the current device (the graph's).
-int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const DecodeIO& io, int64_t B, cudaStream_t st,
-                  const Gate* gate = nullptr);
+int decode_routed(gd_graph* g, const gd_model* model, const Route& r, const DecodeIO& io, int64_t B, cudaStream_t st);
 
 // ---- the families' launchers: plan + buffers -> gd_status ----
 int edge_decode(const gd_graph* g, const gd_model* model, DecodePlan pl, const DecodeIO& io, cudaStream_t st,
-                const Gate* gate = nullptr, const DeferList* dl = nullptr);
+                const DeferList* dl = nullptr);
 // *no_resources: the table kernel could not get its memory pool or a table set, and enqueued nothing that decodes
 int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>& pls, const DecodePlan& deferred,
                 const DecodeIO& io, int64_t B, cudaStream_t st, bool* no_resources);
-int light_decode(const LightPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st, const Gate* gate = nullptr);
+int light_decode(const LightPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st);
 int streamed_decode(gd_graph* g, const StreamPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st);
 int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st);
 

@@ -146,10 +146,6 @@ __global__ void __launch_bounds__(512, 2) decode_light_kernel(const LightParams 
     for (int tix = blockIdx.x; tix < p.n_tiles; tix += gridDim.x) {
         const long long s0 = (long long)tix * tile;
         const int nvalid = (int)min((long long)tile, p.B - s0);
-        if (p.gate_in) {   // gated launch: this tile's chunk may still be on its way from the host
-            if (tid == 0) gate_wait(p.gate_in + tix / p.gate_chunk_tiles, p.gate_epoch, p.gate_err);
-            __syncthreads();
-        }
         // ---- x[tile][N] (coalesced reads) -> xT[N][tile]; m = 0 ----
         {
             const float* xg = p.x + s0 * N;
@@ -315,10 +311,6 @@ __global__ void __launch_bounds__(512, 2) decode_light_kernel(const LightParams 
             }
         }
         __syncthreads();
-        if (p.gate_out && tid == 0) {   // gated launch: publish the tile so the chunk's device->host copy can go
-            __threadfence_system();
-            atomicAdd(p.gate_out + tix / p.gate_chunk_tiles, 1u);
-        }
     }
 }
 
@@ -364,10 +356,6 @@ __global__ void __launch_bounds__(512, 2) decode_light_ext_kernel(const LightPar
     for (int tix = blockIdx.x; tix < p.n_tiles; tix += gridDim.x) {
         const long long s0 = (long long)tix * tile;
         const int nvalid = (int)min((long long)tile, p.B - s0);
-        if (p.gate_in) {   // gated launch: this tile's chunk may still be on its way from the host
-            if (tid == 0) gate_wait(p.gate_in + tix / p.gate_chunk_tiles, p.gate_epoch, p.gate_err);
-            __syncthreads();
-        }
         {
             const float* xg = p.x + s0 * N;
             const int pitch = N | 1;
@@ -538,10 +526,6 @@ __global__ void __launch_bounds__(512, 2) decode_light_ext_kernel(const LightPar
             }
         }
         __syncthreads();
-        if (p.gate_out && tid == 0) {   // gated launch: publish the tile so the chunk's device->host copy can go
-            __threadfence_system();
-            atomicAdd(p.gate_out + tix / p.gate_chunk_tiles, 1u);
-        }
     }
 }
 
@@ -647,14 +631,10 @@ void plan_light(const gd_graph* g, const gd_model* m, int64_t B, LightPlan* out,
     out->why = nullptr;
 }
 
-int light_decode(const LightPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st, const Gate* gate) {
+int light_decode(const LightPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st) {
     LightPlan pl = plan;
     pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
     pl.p.stash = io.stash;
-    if (gate) {
-        pl.p.gate_in = gate->in_flags; pl.p.gate_out = gate->out_counts; pl.p.gate_err = gate->err;
-        pl.p.gate_epoch = gate->epoch; pl.p.gate_chunk_tiles = gate->chunk_tiles;
-    }
     void (*k)(const LightParams);
     switch (model->program) {
         case GD_PROG_CGNNI:

@@ -1,104 +1,25 @@
 // gd_decode_host: the end-to-end call with HOST buffers.  Replaces the reference's
 // `datas = datas.to(device); pred = decoder(datas)` (quantum/decoder_v2_4.py:332-334) plus the
-// read-back of the prediction.  The batch is cut into chunks that flow through two streams
-// (H2D copy -> fused decode kernel -> D2H copy), so copies of one chunk overlap the kernel of
-// the other and the second kernel's CTAs back-fill the SMs the first one's last wave leaves idle.
-//
-// Gated pipeline (edge-owner resident kernel, the headline path): ONE persistent launch over the whole batch instead of one
-// per chunk.  The copy-in stream raises a device flag behind every chunk's H2D copy with a stream memory operation
-// (cuStreamWriteValue32: executed by the front end, no SM needed, so it can never be starved by the resident CTAs); the
-// kernel's tiles wait for their chunk's flag, and count finished tiles per chunk; the copy-out stream blocks on that
-// count (cuStreamWaitValue32) and then copies the chunk's results back.  No per-chunk prologue (weight staging, table
-// builds), no per-chunk tail, and the chunks can be small: the exposed copies shrink to one small chunk each way.
+// read-back of the prediction.  The batch is cut into chunks that are submitted to one internal gd_pipeline per graph
+// (gd_pipeline.cu), so one chunk's copies overlap the decode of its neighbours; the call then waits for all of them.
 #include "gd_decode.cuh"
-#include "gd_options.cuh"
-#include <cuda.h>
 #include <algorithm>
 
 namespace gd {
 
-typedef CUresult (*StreamMemOp32)(CUstream, CUdeviceptr, cuuint32_t, unsigned int);
-
 struct HostCtx {
-    std::mutex call_mu;              // one gd_decode_host call at a time per graph: the staging buffers, gate flags and epochs are shared
-    cudaStream_t st[3] = {nullptr, nullptr, nullptr};
-    // gated pipeline state
-    StreamMemOp32 write32 = nullptr, wait32 = nullptr;
-    int memops = -1;                 // -1 unknown, 0 unavailable, 1 available
-    unsigned int* gate_dev = nullptr;  // [kMaxGateChunks] in_flags | [kMaxGateChunks] out_counts
-    int* gate_err_host = nullptr;    // pinned, mapped
-    int* gate_err_dev = nullptr;
-    cudaEvent_t ev_ready = nullptr;
-    unsigned int epoch = 0;
-    int last_launches = 0;           // kernel launches of the last gd_decode_host call (benchmark accounting)
-    float* x_dev = nullptr;
-    float* prob_dev = nullptr;
-    uint8_t* hard_dev = nullptr;
-    float* w_dev = nullptr;
-    int64_t cap_B = 0;
-    int64_t cap_w = 0;
+    std::mutex call_mu;              // one gd_decode_host call at a time per graph: the pipeline is shared state
+    gd_pipeline* pipe = nullptr;
+    gd_model model{};                // the pipeline was created for this model ...
+    int64_t max_B = 0;               // ... and chunks of up to max_B syndromes
 };
-
-constexpr int kMaxGateChunks = 32;
-
-// stream memory operations through the driver entry points (no link-time dependency on libcuda); the 32-bit
-// operations are available on every device CUDA 12 supports
-static void probe_memops(HostCtx* c, int device) {
-    c->memops = 0;
-    if (opt_on(OPT_NO_GATED_HOST)) return;
-    cudaDriverEntryPointQueryResult q;
-    void *w = nullptr, *wt = nullptr;
-    if (cudaGetDriverEntryPoint("cuStreamWriteValue32", &w, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) return;
-    if (cudaGetDriverEntryPoint("cuStreamWaitValue32", &wt, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) return;
-    if (!w || !wt) return;
-    if (cudaMalloc((void**)&c->gate_dev, 2 * kMaxGateChunks * sizeof(unsigned int)) != cudaSuccess) return;
-    if (cudaMemset(c->gate_dev, 0, 2 * kMaxGateChunks * sizeof(unsigned int)) != cudaSuccess) return;
-    if (cudaHostAlloc((void**)&c->gate_err_host, sizeof(int), cudaHostAllocMapped) != cudaSuccess) return;
-    *c->gate_err_host = 0;
-    if (cudaHostGetDevicePointer((void**)&c->gate_err_dev, c->gate_err_host, 0) != cudaSuccess) return;
-    if (cudaEventCreateWithFlags(&c->ev_ready, cudaEventDisableTiming) != cudaSuccess) return;
-    c->write32 = reinterpret_cast<StreamMemOp32>(w);
-    c->wait32 = reinterpret_cast<StreamMemOp32>(wt);
-    c->memops = 1;
-}
-
-static cudaError_t ensure(HostCtx* c, const gd_graph* g, int64_t B, int64_t n_w) {
-    cudaError_t e = cudaSuccess;
-    for (int i = 0; i < 3 && e == cudaSuccess; ++i)
-        if (!c->st[i]) e = cudaStreamCreateWithFlags(&c->st[i], cudaStreamNonBlocking);
-    if (e == cudaSuccess && B > c->cap_B) {
-        if (c->x_dev) cudaFree(c->x_dev);
-        if (c->prob_dev) cudaFree(c->prob_dev);
-        if (c->hard_dev) cudaFree(c->hard_dev);
-        c->x_dev = nullptr; c->prob_dev = nullptr; c->hard_dev = nullptr; c->cap_B = 0;
-        e = cudaMalloc((void**)&c->x_dev, (size_t)B * g->N * sizeof(float));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&c->prob_dev, (size_t)B * g->V * sizeof(float));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&c->hard_dev, (size_t)B * g->V);
-        if (e == cudaSuccess) c->cap_B = B;
-    }
-    if (e == cudaSuccess && n_w > c->cap_w) {
-        if (c->w_dev) cudaFree(c->w_dev);
-        c->w_dev = nullptr; c->cap_w = 0;
-        e = cudaMalloc((void**)&c->w_dev, (size_t)n_w * sizeof(float));
-        if (e == cudaSuccess) c->cap_w = n_w;
-    }
-    return e;
-}
 
 }  // namespace gd
 
 void gd_host_ctx_destroy(gd_graph* g) {
     gd::HostCtx* c = static_cast<gd::HostCtx*>(g->host_ctx);
     if (!c) return;
-    for (int i = 0; i < 3; ++i)
-        if (c->st[i]) cudaStreamDestroy(c->st[i]);
-    if (c->gate_dev) cudaFree(c->gate_dev);
-    if (c->gate_err_host) cudaFreeHost(c->gate_err_host);
-    if (c->ev_ready) cudaEventDestroy(c->ev_ready);
-    if (c->x_dev) cudaFree(c->x_dev);
-    if (c->prob_dev) cudaFree(c->prob_dev);
-    if (c->hard_dev) cudaFree(c->hard_dev);
-    if (c->w_dev) cudaFree(c->w_dev);
+    gd_pipeline_destroy(c->pipe);
     delete c;
     g->host_ctx = nullptr;
 }
@@ -121,134 +42,34 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
     gd::Route r;
     int rc = gd::route_decode(g, model, B, gd::Use::Infer, &r);
     if (rc != GD_OK) return rc;
+    // chunks: multiples of 8 syndromes (output alignment); >= 4096 syndromes each, at most 4; the streamed kernels take the
+    // batch in one piece.  GNNI.autotune (message_passing.py) tunes the launch geometry for these chunk sizes: keep the two
+    // in step.
+    int n_chunks = (int)std::min<int64_t>(4, std::max<int64_t>(1, B / 8192));
+    if (r.family == gd::Family::StreamedTma || r.family == gd::Family::Streamed) n_chunks = 1;
+    const int64_t per = ((B + n_chunks - 1) / n_chunks + 7) / 8 * 8;
+
     std::unique_lock<std::mutex> lk(g->mu);
     if (!g->host_ctx) g->host_ctx = new gd::HostCtx();
     gd::HostCtx* c = static_cast<gd::HostCtx*>(g->host_ctx);
     lk.unlock();  // gd_decode_fwd takes the same mutex for the streamed workspace
-    // one call at a time per graph from here on: the staging buffers, streams, gate flags and epochs are shared state
     std::lock_guard<std::mutex> call_lk(c->call_mu);
-    cudaError_t e = gd::ensure(c, g, B, n_w);
-    if (e == cudaSuccess && c->memops < 0) gd::probe_memops(c, g->device);
-    if (e == cudaSuccess && c->memops == 1 && B >= 16384 && gd::route_gated(r, model)) {
-        // ---- gated pipeline: st[0] = kernel, st[1] = copies in, st[2] = copies out ----
-        const gd_launch_info li = gd::route_launch_info(r);
-        const int tile = li.tile, n_tiles = li.n_tiles;
-        // 16 chunks: measured on B200, rotated d=5 B=65536: 4 -> 19.20, 8 -> 19.41, 16 -> 19.55 M syn/s
-        int n_chunks = std::min(16, std::max(1, (int)(B / 4096)));
-        const int chunk_tiles = (n_tiles + n_chunks - 1) / n_chunks;
-        n_chunks = (n_tiles + chunk_tiles - 1) / chunk_tiles;
-        const int64_t per = (int64_t)chunk_tiles * tile;
-        unsigned int* in_flags = c->gate_dev;
-        unsigned int* out_counts = c->gate_dev + gd::kMaxGateChunks;
-        const unsigned int epoch = ++c->epoch;
-        *c->gate_err_host = 0;
-        e = cudaMemsetAsync(out_counts, 0, gd::kMaxGateChunks * sizeof(unsigned int), c->st[0]);
-        if (e == cudaSuccess) e = cudaEventRecord(c->ev_ready, c->st[0]);
-        if (e == cudaSuccess && n_w)
-            e = cudaMemcpyAsync(c->w_dev, weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice, c->st[0]);
-        // Enqueue order.  Fast order: the kernel first (its prologue -- weight staging, table builds -- overlaps the first
-        // copy), then the copies + flag writes.  Under a tool that makes kernel launches block the host (ncu / sanitizer
-        // injection, CUDA_LAUNCH_BLOCKING=1) the copies would then never be queued while the kernel waits for them, so
-        // there every copy-in and flag write goes FIRST (measured: 65.0 vs 68.1 M syndromes/s end to end).  If such a tool
-        // goes undetected the gates time out (seconds), the batch is redone by the chunked pipeline and gating is turned off.
-        // (Nsight Compute marks its target with NV_NSIGHT_INJECTION_PORT_BASE / NV_COMPUTE_PROFILER_PERFWORKS_DIR; other
-        // injectors use CUDA_INJECTION64_PATH)
-        const bool kernel_first = !gd::opt_on(gd::OPT_LAUNCH_BLOCKING);
-        bool memop_failed = false, launched = false;
-        auto launch = [&]() {
-            gd::Gate gate{in_flags, out_counts, c->gate_err_dev, epoch, chunk_tiles};
-            gd::DecodeIO io{};
-            io.weights = c->w_dev; io.x = c->x_dev; io.prob = prob_host ? c->prob_dev : nullptr;
-            io.hard = hard_host ? c->hard_dev : nullptr;
-            rc = gd::decode_routed(g, model, r, io, B, c->st[0], &gate);
-            launched = rc == GD_OK;
-        };
-        if (e == cudaSuccess && kernel_first) launch();
-        for (int k = 0; k < n_chunks && e == cudaSuccess && !memop_failed && rc == GD_OK; ++k) {
-            const int64_t b0 = (int64_t)k * per, nb = std::min<int64_t>(per, B - b0);
-            e = cudaMemcpyAsync(c->x_dev + b0 * g->N, x_host + b0 * g->N, (size_t)nb * g->N * sizeof(float),
-                                cudaMemcpyHostToDevice, c->st[1]);
-            if (e == cudaSuccess &&
-                c->write32((CUstream)c->st[1], (CUdeviceptr)(uintptr_t)(in_flags + k), epoch, CU_STREAM_WRITE_VALUE_DEFAULT) != CUDA_SUCCESS)
-                memop_failed = true;
-        }
-        if (memop_failed && launched) {
-            // a flag write was refused with the kernel already waiting: raise every flag from the host so that it drains
-            // (its results are discarded and the batch is redone below)
-            cudaStreamSynchronize(c->st[1]);
-            std::vector<unsigned int> open(gd::kMaxGateChunks, epoch);
-            cudaMemcpyAsync(in_flags, open.data(), gd::kMaxGateChunks * sizeof(unsigned int), cudaMemcpyHostToDevice, c->st[1]);
-            cudaStreamSynchronize(c->st[1]);
-        }
-        if (e == cudaSuccess && !memop_failed && !kernel_first) launch();
-        if (launched && !memop_failed && e == cudaSuccess) {
-            e = cudaStreamWaitEvent(c->st[2], c->ev_ready, 0);
-            for (int k = 0; k < n_chunks && e == cudaSuccess && !memop_failed; ++k) {
-                const int64_t b0 = (int64_t)k * per, nb = std::min<int64_t>(per, B - b0);
-                const unsigned int tiles_k = (unsigned int)((nb + tile - 1) / tile);
-                if (c->wait32((CUstream)c->st[2], (CUdeviceptr)(uintptr_t)(out_counts + k), tiles_k, CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS) {
-                    memop_failed = true;      // the kernel still drains (all its flags are queued); results are redone below
-                    break;
-                }
-                if (prob_host)
-                    e = cudaMemcpyAsync(prob_host + b0 * g->V, c->prob_dev + b0 * g->V, (size_t)nb * g->V * sizeof(float),
-                                        cudaMemcpyDeviceToHost, c->st[2]);
-                if (e == cudaSuccess && hard_host)
-                    e = cudaMemcpyAsync(hard_host + b0 * g->V, c->hard_dev + b0 * g->V, (size_t)nb * g->V,
-                                        cudaMemcpyDeviceToHost, c->st[2]);
-            }
-        }
-        cudaError_t s0 = cudaStreamSynchronize(c->st[0]);
-        cudaError_t s1 = cudaStreamSynchronize(c->st[1]);
-        cudaError_t s2 = cudaStreamSynchronize(c->st[2]);   // the kernel always drains, so every queued wait is satisfied
-        if (e == cudaSuccess) e = s0 != cudaSuccess ? s0 : (s1 != cudaSuccess ? s1 : s2);
+    const bool same_model = c->model.program == model->program && c->model.hidden == model->hidden &&
+                            c->model.iters == model->iters && c->model.flags == model->flags;
+    if (!c->pipe || per > c->max_B || !same_model) {
+        gd_pipeline_destroy(c->pipe);
+        rc = gd_pipeline_create(g, model, weights_host, per, 4, &c->pipe);
         if (rc != GD_OK) return rc;
-        GD_CUDA(e);
-        c->last_launches = 1;
-        if (!memop_failed && *c->gate_err_host == 0) return GD_OK;
-        // a gate timed out (the copy-in stream was held up behind the kernel) or a memory operation was refused: results
-        // are not trustworthy -> never gate again on this graph and redo the batch with one launch per chunk
-        c->memops = 0;
+        c->model = *model;
+        c->max_B = per;
     }
-    if (e == cudaSuccess && n_w) {
-        e = cudaMemcpyAsync(c->w_dev, weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice, c->st[0]);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->st[0]);
+    rc = gd_pipeline_set_weights(c->pipe, weights_host);
+    for (int64_t b0 = 0; b0 < B && rc == GD_OK; b0 += per) {
+        const int64_t nb = std::min<int64_t>(per, B - b0);
+        rc = gd_pipeline_submit(c->pipe, x_host + b0 * g->N, prob_host ? prob_host + b0 * g->V : nullptr,
+                                hard_host ? hard_host + b0 * g->V : nullptr, nb, nullptr);
     }
-    if (e == cudaSuccess) {
-        // chunks: multiples of 8 syndromes (output alignment); >= 4096 syndromes each, at most 4
-        int n_chunks = (int)std::min<int64_t>(4, std::max<int64_t>(1, B / 8192));
-        if (r.family == gd::Family::StreamedTma || r.family == gd::Family::Streamed) n_chunks = 1;  // one shared slab
-        int64_t per = ((B + n_chunks - 1) / n_chunks + 7) / 8 * 8;
-        c->last_launches = 0;
-        for (int k = 0; k < n_chunks && e == cudaSuccess && rc == GD_OK; ++k) {
-            const int64_t b0 = (int64_t)k * per;
-            const int64_t nb = std::min<int64_t>(per, B - b0);
-            if (nb <= 0) break;
-            cudaStream_t st = c->st[k & 1];
-            e = cudaMemcpyAsync(c->x_dev + b0 * g->N, x_host + b0 * g->N, (size_t)nb * g->N * sizeof(float),
-                                cudaMemcpyHostToDevice, st);
-            if (e != cudaSuccess) break;
-            rc = gd_decode_fwd(g, model, c->w_dev, c->x_dev + b0 * g->N, prob_host ? c->prob_dev + b0 * g->V : nullptr,
-                               nullptr, hard_host ? c->hard_dev + b0 * g->V : nullptr, nb, st);
-            if (rc != GD_OK) break;
-            ++c->last_launches;
-            if (prob_host)
-                e = cudaMemcpyAsync(prob_host + b0 * g->V, c->prob_dev + b0 * g->V, (size_t)nb * g->V * sizeof(float),
-                                    cudaMemcpyDeviceToHost, st);
-            if (e == cudaSuccess && hard_host)
-                e = cudaMemcpyAsync(hard_host + b0 * g->V, c->hard_dev + b0 * g->V, (size_t)nb * g->V,
-                                    cudaMemcpyDeviceToHost, st);
-        }
-        cudaError_t s0 = cudaStreamSynchronize(c->st[0]);
-        cudaError_t s1 = cudaStreamSynchronize(c->st[1]);
-        if (e == cudaSuccess) e = s0 != cudaSuccess ? s0 : s1;
-    }
-    if (rc != GD_OK) return rc;
-    GD_CUDA(e);
-    return GD_OK;
-}
-
-extern "C" int gd_decode_host_last_launches(const gd_graph* g) {
-    if (!g || !g->host_ctx) return 0;
-    return static_cast<const gd::HostCtx*>(g->host_ctx)->last_launches;
+    // drain even after an error: chunks already submitted are still writing into the caller's buffers
+    const int rc_drain = gd_pipeline_drain(c->pipe);
+    return rc != GD_OK ? rc : rc_drain;
 }

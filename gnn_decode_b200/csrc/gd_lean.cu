@@ -1790,7 +1790,7 @@ int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>&
         // training: all rows or none (the header's old_count is 0 or -1), and the edge-owner kernel writes its own stash layout
         const DeferList dl{stash_dev ? &lean_train_hdr(stash_dev, g, model, B)->old_count : &call->defer_count,
                            reinterpret_cast<const int*>(ws + o_defer)};
-        rc = edge_decode(g, model, deferred, dio, st, nullptr, &dl);
+        rc = edge_decode(g, model, deferred, dio, st, &dl);
     }
     cudaError_t ef = cudaFreeAsync(ws, st);
     if (rc != GD_OK) return rc;

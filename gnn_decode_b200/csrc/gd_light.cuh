@@ -17,12 +17,6 @@ struct LightParams {
     int T, V, C, E, N;
     int tile, lanes, R, hid, hp, n_tiles, trows;
     int off_w, off_tab, off_x, off_m, off_t;
-    // gated launch (gd_decode_host, see Gate in gd_decode.cuh); all NULL / 0 otherwise
-    const unsigned int* gate_in;
-    unsigned int* gate_out;
-    int* gate_err;
-    unsigned int gate_epoch;
-    int gate_chunk_tiles;
     // training: m after every iteration, stash[it][E][B] (CGNNI forward with stash), or the stash the backward reads
     float* stash;
 };

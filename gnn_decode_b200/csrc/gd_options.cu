@@ -9,8 +9,8 @@
 namespace gd {
 
 static const char* const kOptNames[OPT_COUNT] = {
-    "GD_NO_CTAB", "GD_NO_VTAB", "GD_FORCE_STREAMED", "GD_NO_VSKIP", "GD_FORCE_LIGHT", "GD_NO_GATED_HOST", "GD_NO_LEAN",
-    "GD_LEAN_R", "GD_LEAN_G", "GD_LEAN_PARTS", "GD_LAUNCH_BLOCKING"};
+    "GD_NO_CTAB", "GD_NO_VTAB", "GD_FORCE_STREAMED", "GD_NO_VSKIP", "GD_FORCE_LIGHT", "GD_NO_LEAN", "GD_LEAN_R", "GD_LEAN_G",
+    "GD_LEAN_PARTS"};
 
 static std::atomic<long long> g_opt[OPT_COUNT];
 static std::once_flag g_opt_once;
@@ -23,12 +23,6 @@ static void load_env() {
         const char* e = getenv(kOptNames[i]);
         g_opt[i].store(e ? atoll(e) : kOptUnset, std::memory_order_relaxed);
     }
-    // tools that make kernel launches block the host (Nsight Compute marks its target with NV_NSIGHT_INJECTION_PORT_BASE /
-    // NV_COMPUTE_PROFILER_PERFWORKS_DIR; other injectors use CUDA_INJECTION64_PATH): the gated host pipeline then queues
-    // its copies before the kernel (gd_host.cu)
-    if (getenv("CUDA_INJECTION64_PATH") || getenv("NV_NSIGHT_INJECTION_PORT_BASE") || getenv("NV_COMPUTE_PROFILER_PERFWORKS_DIR") ||
-        getenv("CUDA_LAUNCH_BLOCKING"))
-        g_opt[OPT_LAUNCH_BLOCKING].store(1, std::memory_order_relaxed);
 }
 
 long long opt_get(Opt o) {

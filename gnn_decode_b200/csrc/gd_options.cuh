@@ -11,12 +11,10 @@ enum Opt {
     OPT_FORCE_STREAMED,   // GD_FORCE_STREAMED take the streamed global-memory kernel even when the state fits on chip
     OPT_NO_VSKIP,         // GD_NO_VSKIP       re-evaluate degree-1 variables every iteration
     OPT_FORCE_LIGHT,      // GD_FORCE_LIGHT    node-owner kernel even where the planner declines
-    OPT_NO_GATED_HOST,    // GD_NO_GATED_HOST  chunked host pipeline instead of the gated single launch
     OPT_NO_LEAN,          // GD_NO_LEAN        decoder_v2_4 on surface/toric codes: skip the table-only check-owner kernel
     OPT_LEAN_R,           // GD_LEAN_R         its owners (warps) per group of 32 syndromes
     OPT_LEAN_G,           // GD_LEAN_G         its groups per CTA
     OPT_LEAN_PARTS,       // GD_LEAN_PARTS     1: decode the graph's connected components in separate launches, 0: never (unset: when that seats more groups)
-    OPT_LAUNCH_BLOCKING,  // (derived) a tool that makes launches block the host is attached (ncu / sanitizer / CUDA_LAUNCH_BLOCKING)
     OPT_COUNT
 };
 

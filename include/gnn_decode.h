@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define GD_ABI_VERSION 1
+#define GD_ABI_VERSION 2
 
 enum gd_status {
     GD_OK = 0,
@@ -193,15 +193,12 @@ int gd_decode_packed_fwd(const gd_graph* g, const gd_model* model, const float* 
                          const uint32_t* synd_dev, float* prob_dev, uint32_t* hard_bits_dev, int64_t B, void* stream);
 
 /* Same computation with HOST buffers: host->device copy of x, the kernel, device->host copy of
- * the requested outputs, pipelined in chunks over internal streams; returns when the outputs
- * are complete.  Calls on one graph are serialised internally (they share its staging buffers); use one gd_pipeline
- * per caller for concurrency.  Replaces `datas.to(device); pred = decoder(datas)` (decoder_v2_4.py:332-334)
- * followed by reading the prediction back. weights_host is the packed buffer on the host. */
+ * the requested outputs.  The batch is cut into up to 4 chunks that run through an internal gd_pipeline (below) kept
+ * per graph; returns when the outputs are complete.  Calls on one graph are serialised internally (they share that
+ * pipeline); use one gd_pipeline per caller for concurrency.  Replaces `datas.to(device); pred = decoder(datas)`
+ * (decoder_v2_4.py:332-334) followed by reading the prediction back. weights_host is the packed buffer on the host. */
 int gd_decode_host(const gd_graph* g, const gd_model* model, const float* weights_host,
                    const float* x_host, float* prob_host, uint8_t* hard_host, int64_t B);
-/* Decode-kernel launches the last gd_decode_host call on this graph made: 1 for the gated single-launch pipeline, one per chunk
- * otherwise (benchmark accounting; streamed codes count one per gd_decode_fwd call). */
-int gd_decode_host_last_launches(const gd_graph* g);
 
 /* ---- the same end-to-end call as an ASYNCHRONOUS PIPELINE for callers that stream batches: batch k+1 is copied in
  *      while batch k decodes and batch k-1 is copied out (three internal streams chained by events, `depth` slots of

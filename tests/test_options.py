@@ -4,14 +4,16 @@ import pytest
 
 from gnn_decode_b200 import _cabi, options
 
-KEPT = ["GD_NO_LEAN", "GD_FORCE_STREAMED", "GD_FORCE_LIGHT", "GD_NO_CTAB", "GD_NO_VTAB", "GD_NO_VSKIP", "GD_NO_GATED_HOST",
-        "GD_LEAN_PARTS", "GD_LEAN_R", "GD_LEAN_G"]
+KEPT = ["GD_NO_LEAN", "GD_FORCE_STREAMED", "GD_FORCE_LIGHT", "GD_NO_CTAB", "GD_NO_VTAB", "GD_NO_VSKIP", "GD_LEAN_PARTS",
+        "GD_LEAN_R", "GD_LEAN_G"]
 
 # tuning experiments whose measured winner is now the only value (DESIGN.md keeps the numbers)
 RETIRED = ["GD_CPS", "GD_NO_PWL", "GD_NO_RTAB", "GD_RTAB_N", "GD_CTAB_N", "GD_VTAB_N", "GD_VTAB_K", "GD_TILE", "GD_R", "GD_EB",
            "GD_NPOLY", "GD_NO_DIRECT", "GD_NO_LIGHT", "GD_LTILE", "GD_LR", "GD_GATE_CHUNKS", "GD_GATE_COPIES_FIRST", "GD_STILE",
            "GD_STHREADS", "GD_STREAM_LEGACY", "GD_SROWS", "GD_SSTAGES", "GD_SWARPS", "GD_NO_BWD_CTAB", "GD_LEAN_VTAB_N",
-           "GD_LEAN_CTAB_N", "GD_LEAN_RTAB_N", "GD_NO_PDL"]
+           "GD_LEAN_CTAB_N", "GD_LEAN_RTAB_N", "GD_NO_PDL",
+           # switches of gd_decode_host's gated single launch, which is gone (the call runs on gd_pipeline)
+           "GD_NO_GATED_HOST", "GD_LAUNCH_BLOCKING"]
 
 
 @pytest.mark.parametrize("name", KEPT)

@@ -307,10 +307,10 @@ def test_autotuned_geometry_gives_identical_results():
     assert isinstance(info0, dict)
 
 
-def test_decode_host_gated_pipeline(gd_opt):
-    """gd_decode_host's gated single-launch pipeline (chunk flags raised by stream memory operations, per-chunk tile
-    counters releasing the copies back): bit-identical to the device path and to the one-launch-per-chunk pipeline, on
-    ragged batch sizes, repeated calls (epoch reuse), changing batch sizes and either output alone."""
+def test_decode_host_pipeline(gd_opt):
+    """gd_decode_host (chunks through the graph's internal gd_pipeline): bit-identical to the device path on ragged batch
+    sizes, repeated and changing batch sizes, either output alone, pageable input, a fresh graph context, the edge-owner
+    kernel, the streamed kernel (one chunk), and a second decoder with another T on the same graph (a new pipeline)."""
     from gnn_decode_b200.graph import TannerGraph
     from gnn_decode_b200.sampler import sample_syndromes
     g = Golden("v2_4_toricL4_epoch1")
@@ -323,11 +323,15 @@ def test_decode_host_gated_pipeline(gd_opt):
     ref_p, ref_h = dec.decode(x_all, return_hard=True)
     ref_p, ref_h = ref_p.cpu(), ref_h.cpu()
     xh_all = x_all.cpu().pin_memory()
-    for B in (40000, 16384, 20001, 33333, 40000):
-        xh = xh_all[:B]
+
+    def both(dec, B, graph=None):
         prob_h = torch.zeros(B, g.V, dtype=torch.float32).pin_memory()
         hard_h = torch.full((B, g.V), 7, dtype=torch.uint8).pin_memory()
-        dec.decode_host(xh, prob_h, hard_h)
+        dec.decode_host(xh_all[:B], prob_h, hard_h, graph=graph)
+        return prob_h, hard_h
+
+    for B in (40000, 16384, 20001, 33333, 40000):
+        prob_h, hard_h = both(dec, B)
         assert torch.equal(prob_h, ref_p[:B]) and torch.equal(hard_h, ref_h[:B]), B
     only_h = dec.decode_host(xh_all, hard_out=torch.empty(40000, g.V, dtype=torch.uint8).pin_memory())
     assert torch.equal(only_h, ref_h)
@@ -335,16 +339,27 @@ def test_decode_host_gated_pipeline(gd_opt):
     assert torch.equal(only_p, ref_p)
     pageable = dec.decode_host(x_all.cpu()[:17000].clone())                                # pageable host memory works too
     assert torch.equal(pageable, ref_p[:17000])
-    # the one-launch-per-chunk pipeline (gating disabled for a fresh graph context) gives the same bits
-    gd_opt.set("GD_NO_GATED_HOST")
-    tg2 = TannerGraph(g.edge_index, g.V, g.C, dev)
+    tg2 = TannerGraph(g.edge_index, g.V, g.C, dev)                                         # a fresh graph context
     p2 = dec.decode_host(xh_all, graph=tg2)
     assert torch.equal(p2, ref_p)
+    for opt, B in (("GD_NO_LEAN", 40000), ("GD_FORCE_STREAMED", 20001)):                   # edge-owner; streamed: one chunk
+        gd_opt.set(opt)
+        p_d, h_d = dec.decode(x_all[:B], return_hard=True)
+        prob_h, hard_h = both(dec, B)
+        gd_opt.unset(opt)
+        assert torch.equal(prob_h, p_d.cpu()) and torch.equal(hard_h, h_d.cpu()), opt
+    dec_t = mod.GNNI(g.T + 2)                                                              # another model on the same graph
+    dec_t.load_state_dict(g.weights, strict=True)
+    dec_t = dec_t.to(dev).eval()
+    p_t, h_t = dec_t.decode(x_all, graph=tg, return_hard=True)
+    prob_h, hard_h = both(dec_t, 40000, graph=tg)
+    assert torch.equal(prob_h, p_t.cpu()) and torch.equal(hard_h, h_t.cpu())
+    assert not torch.equal(p_t.cpu(), ref_p)
 
 
 @pytest.mark.parametrize("name", ["qgnni_toricL4_seeded", "cgnni_bch_seeded", "bp_quantum_toricL4", "cgnni_ldpc_epoch18"])
-def test_decode_host_gated_pipeline_light_programs(name):
-    """The gated pipeline through the node-owner (light) kernels: same bits as the device path."""
+def test_decode_host_pipeline_light_programs(name):
+    """gd_decode_host through the node-owner (light) kernels: same bits as the device path."""
     from gnn_decode_b200.graph import TannerGraph
     g = Golden(name)
     dev = _dev()
