@@ -2,8 +2,9 @@
 // w.r.t. the 10h+3 MLP weights, given dL/dlogit [B, V].  Replaces autograd through the reference's
 // T x 2 x ~12 eager ops (quantum/decoder_v2_4.py:280-292, loss.backward() at :335).
 //
-// Structure per tile of syndromes (edge arrays [E][tile] fp32 in shared memory), iterations in
-// reverse, activations (m_it, a_it) re-read from the stash the training forward wrote:
+// Structure per tile of syndromes (edge arrays [E][tile] fp32 in shared memory -- or, for codes whose arrays do not fit
+// there, in a per-CTA slab of the caller's workspace: the same kernel body, see WORK_GLOBAL), iterations in reverse,
+// activations (m_it, a_it) re-read from the stash the training forward wrote:
 //   * "sum over siblings minus self" is self-adjoint, so the gather-of-gradients is the same
 //     deterministic segmented sum as the forward reduce;
 //   * the per-edge MLP backward is the expensive part and is mapped DIFFERENTLY from the forward:
@@ -46,6 +47,9 @@ struct BwdParams {
     // n_static = E - n_vact edges of degree-1 variables see ext == 0 in every iteration, so their upstream
     // gradients are summed over the iterations (off_gacc) and pushed through the MLP once per tile
     int n_vact, off_gacc;
+    // WORK_GLOBAL: the per-tile work arrays (off_x .. off_gacc, byte offsets) live at slab + blockIdx.x * slab_floats
+    float* slab;
+    long long slab_floats;
 };
 
 constexpr int kPairs = kUPL / 2;
@@ -194,6 +198,10 @@ __device__ __forceinline__ void store_acc(float* dst, const LaneAcc& A, int h, b
     if (lane == 0) dst[(two_in ? 4 : 3) * h] = A.b2;
 }
 
+// WORK_GLOBAL = false: every per-tile array in shared memory (tile limited by its size).  WORK_GLOBAL = true: the per-tile work
+// arrays (xs .. GA) in this CTA's slab of the workspace, for codes too large for the first form (HGP [[1600,64]]: ~390 KB per
+// syndrome); the graph tables, the check table and its adjoint bins stay in shared memory, the bins as 64-bit integers (below).
+template <bool WORK_GLOBAL>
 __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdParams p) {
     extern __shared__ __align__(128) unsigned char smem[];
     pdl_enter();
@@ -202,17 +210,18 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
     const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5, n_warps = nthr >> 5;
     const int s = tid % tile, r = tid / tile;
     const bool ew = r < R;                      // threads beyond R*tile only take part in the MLP phases
-    float* xs = reinterpret_cast<float*>(smem + p.off_x);
-    float* node = reinterpret_cast<float*>(smem + p.off_node);
-    float* DM = reinterpret_cast<float*>(smem + p.off_dm);
-    float* A_ = reinterpret_cast<float*>(smem + p.off_a);
-    float* XI = reinterpret_cast<float*>(smem + p.off_xin);
-    float* X1 = reinterpret_cast<float*>(smem + p.off_x1);
-    float* MB = reinterpret_cast<float*>(smem + p.off_mb);
-    float* AB = reinterpret_cast<float*>(smem + p.off_ab);
-    float* node2 = reinterpret_cast<float*>(smem + p.off_node2);
-    float* G_ = reinterpret_cast<float*>(smem + p.off_g);
-    float* DX = reinterpret_cast<float*>(smem + p.off_dx);
+    unsigned char* const wk = WORK_GLOBAL ? reinterpret_cast<unsigned char*>(p.slab + (size_t)blockIdx.x * p.slab_floats) : smem;
+    float* xs = reinterpret_cast<float*>(wk + p.off_x);
+    float* node = reinterpret_cast<float*>(wk + p.off_node);
+    float* DM = reinterpret_cast<float*>(wk + p.off_dm);
+    float* A_ = reinterpret_cast<float*>(wk + p.off_a);
+    float* XI = reinterpret_cast<float*>(wk + p.off_xin);
+    float* X1 = reinterpret_cast<float*>(wk + p.off_x1);
+    float* MB = reinterpret_cast<float*>(wk + p.off_mb);
+    float* AB = reinterpret_cast<float*>(wk + p.off_ab);
+    float* node2 = reinterpret_cast<float*>(wk + p.off_node2);
+    float* G_ = reinterpret_cast<float*>(wk + p.off_g);
+    float* DX = reinterpret_cast<float*>(wk + p.off_dx);
     uint16_t* tab = reinterpret_cast<uint16_t*>(smem + p.off_tab);
     uint16_t* edge_var = tab;
     uint16_t* edge_chk = edge_var + E;
@@ -223,7 +232,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
     uint16_t* vpos = chk_edges + E;                      // position of edge e in vlist order
     for (int i = tid; i < E; i += nthr) vpos[p.tb.vlist[i]] = (uint16_t)i;
     const int n_act = p.n_vact, n_static = E - n_act;
-    float* GA = reinterpret_cast<float*>(smem + p.off_gacc);
+    float* GA = reinterpret_cast<float*>(wk + p.off_gacc);
     for (int i = tid; i < E; i += nthr) {
         edge_var[i] = (uint16_t)p.tb.edge_var[i];
         edge_chk[i] = (uint16_t)p.tb.edge_chk[i];
@@ -247,13 +256,17 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
     //                its Hermite interpolant gives  sum_j [ A_j phi(x_j) + D_j h phi'(x_j) ]  with the ADJOINT bins
     //                A_j = sum_i g_i h00/h01(t_i), D_j = sum_i g_i h10/h11(t_i): four scatter-adds per item now, and one
     //                pass over (nodes x hidden units) at the very end, instead of h x 3 MUFU per item.
-    // The bins are accumulated as 32-bit FIXED-POINT integers (scale from the phase's max |g|: integer adds commute,
-    // so shared-memory atomics stay bit-reproducible) and flushed into double master bins after every phase.
+    // The bins are accumulated as FIXED-POINT integers (scale from the phase's max |g|: integer adds commute, so shared-memory
+    // atomics stay bit-reproducible) and flushed into double master bins after every phase.  The scale keeps
+    // n_items * max|g| below 2^30 in 32-bit bins; with WORK_GLOBAL, n_items = E * tile is large (HGP: ~3e5) and 32 bits would
+    // leave ~3e3 units for the largest item, so that variant takes 64-bit bins and 2^62: every item keeps the float
+    // product's own precision.
     CubicTab ctab{};
     bool use_ctab = false;
     unsigned int* bins = reinterpret_cast<unsigned int*>(smem + p.off_bins);      // [2][n+1]
+    unsigned long long* bins64 = reinterpret_cast<unsigned long long*>(smem + p.off_bins);
     double* mbins = reinterpret_cast<double*>(smem + p.off_mbins);                // [2][n+1]
-    unsigned int* gmax_bits = bins + 2 * (p.ctab_n + 1);
+    unsigned int* gmax_bits = WORK_GLOBAL ? reinterpret_cast<unsigned int*>(bins64 + 2 * (p.ctab_n + 1)) : bins + 2 * (p.ctab_n + 1);
     if (p.ctab_n > 0 && E * tile >= p.ctab_n + 8) {
         float* w2s = reinterpret_cast<float*>(smem + p.off_w2s);
         const int hp = (h + 7) / 8 * 8;
@@ -272,7 +285,11 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
             float4* cdst = reinterpret_cast<float4*>(smem + p.off_ctab);
             cubic_tab_build(W2s, hp, p.ctab_R, p.ctab_n, cdst, DM, tid, nthr);    // DM is idle scratch here
             ctab = CubicTab{cdst, 1.0f / step, p.ctab_R / step, (float)p.ctab_n - 0.001f};
-            for (int j = tid; j < 2 * (p.ctab_n + 1); j += nthr) { bins[j] = 0u; mbins[j] = 0.0; }
+            for (int j = tid; j < 2 * (p.ctab_n + 1); j += nthr) {
+                if constexpr (WORK_GLOBAL) bins64[j] = 0ull;
+                else bins[j] = 0u;
+                mbins[j] = 0.0;
+            }
             if (tid == 0) *gmax_bits = 0u;
         }
     }
@@ -293,8 +310,13 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
             const float* st_m = p.stash + (size_t)it * 2 * EB_ + s0 + s;
             const float* st_a = st_m + EB_;
             for (int e = r; e < E; e += R) {
-                cp_async4(MB + e * tile + s, st_m + (size_t)e * p.B);
-                cp_async4(AB + e * tile + s, st_a + (size_t)e * p.B);
+                if constexpr (WORK_GLOBAL) {        // (the same thread reads them back, behind the same barriers)
+                    MB[e * tile + s] = __ldcs(st_m + (size_t)e * p.B);
+                    AB[e * tile + s] = __ldcs(st_a + (size_t)e * p.B);
+                } else {
+                    cp_async4(MB + e * tile + s, st_m + (size_t)e * p.B);
+                    cp_async4(AB + e * tile + s, st_a + (size_t)e * p.B);
+                }
             }
         }
         cp_async_commit();
@@ -349,8 +371,8 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
                 if (lane == 0) atomicMax(gmax_bits, __float_as_uint(gm));
                 __syncthreads();
                 const float gmax = __uint_as_float(*gmax_bits);
-                // |sum over a bin| <= n_items * gmax: keep it below 2^30
-                const float scale = gmax > 0.f ? 1073741824.0f / (gmax * (float)n_items) : 0.f;
+                // |sum over a bin| <= n_items * gmax: keep it below 2^30 (32-bit bins) / 2^62 (64-bit bins)
+                const float scale = gmax > 0.f ? (WORK_GLOBAL ? 4611686018427387904.0f : 1073741824.0f) / (gmax * (float)n_items) : 0.f;
                 for (int i = tid; i < n_items; i += nthr) {
                     const float xv = XI[i], gv = G_[i];
                     float u = fmaf(xv, ctab.inv_h, ctab.off);
@@ -363,18 +385,30 @@ __global__ void __launch_bounds__(kBwdThreads, 1) decode_bwd_kernel(const BwdPar
                     if (gv != 0.f) {
                         const float t2 = t * t, t3 = t2 * t, gs = gv * scale;
                         const float h01 = 3.0f * t2 - 2.0f * t3;
-                        atomicAdd(bins + j, (unsigned int)__float2int_rn(gs * (1.0f - h01)));
-                        atomicAdd(bins + j + 1, (unsigned int)__float2int_rn(gs * h01));
-                        atomicAdd(bins + nb + j, (unsigned int)__float2int_rn(gs * (t3 - 2.0f * t2 + t)));
-                        atomicAdd(bins + nb + j + 1, (unsigned int)__float2int_rn(gs * (t3 - t2)));
+                        if constexpr (WORK_GLOBAL) {
+                            atomicAdd(bins64 + j, (unsigned long long)__float2ll_rn(gs * (1.0f - h01)));
+                            atomicAdd(bins64 + j + 1, (unsigned long long)__float2ll_rn(gs * h01));
+                            atomicAdd(bins64 + nb + j, (unsigned long long)__float2ll_rn(gs * (t3 - 2.0f * t2 + t)));
+                            atomicAdd(bins64 + nb + j + 1, (unsigned long long)__float2ll_rn(gs * (t3 - t2)));
+                        } else {
+                            atomicAdd(bins + j, (unsigned int)__float2int_rn(gs * (1.0f - h01)));
+                            atomicAdd(bins + j + 1, (unsigned int)__float2int_rn(gs * h01));
+                            atomicAdd(bins + nb + j, (unsigned int)__float2int_rn(gs * (t3 - 2.0f * t2 + t)));
+                            atomicAdd(bins + nb + j + 1, (unsigned int)__float2int_rn(gs * (t3 - t2)));
+                        }
                     }
                 }
                 __syncthreads();
                 if (scale > 0.f) {
                     const double inv = 1.0 / (double)scale;
                     for (int j = tid; j < 2 * nb; j += nthr) {
-                        mbins[j] += (double)(int)bins[j] * inv;
-                        bins[j] = 0u;
+                        if constexpr (WORK_GLOBAL) {
+                            mbins[j] += (double)(long long)bins64[j] * inv;
+                            bins64[j] = 0ull;
+                        } else {
+                            mbins[j] += (double)(int)bins[j] * inv;
+                            bins[j] = 0u;
+                        }
                     }
                 }
                 if (tid == 0) *gmax_bits = 0u;
@@ -494,8 +528,11 @@ static int align_up_b(int x, int a) { return (x + a - 1) / a * a; }
 struct BwdPlan {
     BwdParams p;
     int threads, grid, smem, n_rows;
+    bool work_global;        // decode_bwd_kernel<true>: the work arrays in a slab of grid * p.slab_floats workspace floats
 };
 
+// The shared-memory form when at least 4 syndromes' work arrays fit there (and GD_FORCE_STREAMED is not set), the
+// global-memory form otherwise.
 static int plan_bwd(const gd_graph* g, const gd_model* m, int64_t B, BwdPlan* out) {
     BwdParams& p = out->p;
     memset(&p, 0, sizeof(p));
@@ -504,40 +541,55 @@ static int plan_bwd(const gd_graph* g, const gd_model* m, int64_t B, BwdPlan* ou
     p.B = B; p.T = m->iters; p.V = V; p.C = C; p.E = E; p.N = N; p.hid = m->hidden; p.maxvc = maxvc;
     p.tb = g->t;
     p.np_pad = align_up_b((int)gd_weights_size(m), 32);
-    const int tab_bytes = (5 * E + V + C + 2) * 2;
-    int fixed = align_up_b(tab_bytes, 128);
-    p.n_vact = opt_on(OPT_NO_VSKIP) ? E : g->n_vact;
-    if (!opt_on(OPT_NO_CTAB)) {
-        p.ctab_n = kCtabN;
-        p.ctab_R = (float)(g->max_chk_deg > 1 ? g->max_chk_deg - 1 : 1);
-        const int hp = (m->hidden + 7) / 8 * 8;
-        p.off_ctab = fixed; fixed += p.ctab_n * 16;
-        p.off_w2s = fixed; fixed += 4 * hp * 4;
-        p.off_mbins = fixed; fixed += 2 * (p.ctab_n + 1) * 8;
-        p.off_bins = fixed; fixed += (2 * (p.ctab_n + 1) + 4) * 4;
-        fixed = align_up_b(fixed, 128);
-    }
-    const int64_t per_syn = ((int64_t)N + 2LL * maxvc + 8LL * E + (E - p.n_vact)) * 4;
-    const int64_t tmax = (g->max_smem_optin - fixed) / per_syn;
-    if (g->E >= 65536 || tmax < 4) {
-        set_error("gd_decode_bwd: code too large for the shared-memory backward kernel (E=%lld)", (long long)g->E);
+    if (g->E >= 65536) {
+        set_error("gd_decode_bwd: E=%lld edges; the backward's graph tables hold 16-bit edge ids (E < 65536)", (long long)g->E);
         return GD_ERR_UNSUPPORTED;
     }
-    // tile: multiple of 8 dividing the work evenly over the SMs (same criterion as the forward)
+    const int64_t per_syn = ((int64_t)N + 2LL * maxvc + 8LL * E + (E - (opt_on(OPT_NO_VSKIP) ? E : g->n_vact))) * 4;
+    const int tab_bytes = (5 * E + V + C + 2) * 2;
+    // the form is decided before the layout: the global-memory form's bins are 64-bit
+    int64_t tmax = 0;
+    bool work_global = opt_on(OPT_FORCE_STREAMED);
+    for (int pass = 0; pass < 2; ++pass) {
+        int fixed = align_up_b(tab_bytes, 128);
+        p.n_vact = opt_on(OPT_NO_VSKIP) ? E : g->n_vact;
+        if (!opt_on(OPT_NO_CTAB)) {
+            p.ctab_n = kCtabN;
+            p.ctab_R = (float)(g->max_chk_deg > 1 ? g->max_chk_deg - 1 : 1);
+            const int hp = (m->hidden + 7) / 8 * 8;
+            p.off_ctab = fixed; fixed += p.ctab_n * 16;
+            p.off_w2s = fixed; fixed += 4 * hp * 4;
+            p.off_mbins = fixed; fixed += 2 * (p.ctab_n + 1) * 8;
+            p.off_bins = fixed; fixed += work_global ? 2 * (p.ctab_n + 1) * 8 + 16 : (2 * (p.ctab_n + 1) + 4) * 4;
+            fixed = align_up_b(fixed, 128);
+        }
+        out->smem = fixed;
+        tmax = (g->max_smem_optin - fixed) / per_syn;
+        if (work_global) break;
+        if (tmax >= 4) break;
+        work_global = true;
+    }
+    if (work_global && out->smem > g->max_smem_optin) {
+        set_error("gd_decode_bwd: the graph tables (%d bytes) do not fit shared memory", out->smem);
+        return GD_ERR_UNSUPPORTED;
+    }
+    out->work_global = work_global;
+    // tile: multiple of 4 dividing the work evenly over the SMs (same criterion as the forward); the global-memory form is not
+    // limited by shared memory and takes the larger tile on a tie (longer contiguous rows)
     int tile = 4;
     double best = -1.0;
-    for (int t = 4; t <= tmax && t <= 128; t += 4) {
+    for (int t = 4; (work_global || t <= tmax) && t <= 128; t += 4) {
         const int64_t n_t = (B + t - 1) / t;
         const int64_t rounds = (n_t + g->sm_count - 1) / g->sm_count;
         const double eff = (double)B / ((double)rounds * g->sm_count * t);
-        if (eff > best + 1e-9) { best = eff; tile = t; }
+        if (eff > best + 1e-9 || (work_global && eff > best - 1e-9)) { best = eff; tile = t; }
     }
     p.tile = tile;
     p.R = kBwdThreads / tile;
     if (p.R > E) p.R = E;
     if (p.R < 1) p.R = 1;
     int o = 0;
-    p.off_tab = o; o = fixed;
+    p.off_tab = o; o = work_global ? 0 : out->smem;
     p.off_x = o; o += tile * N * 4; o = align_up_b(o, 16);
     p.off_node = o; o += maxvc * tile * 4;
     p.off_node2 = o; o += maxvc * tile * 4;
@@ -550,12 +602,18 @@ static int plan_bwd(const gd_graph* g, const gd_model* m, int64_t B, BwdPlan* ou
     p.off_mb = o; o += E * tile * 4;
     p.off_ab = o; o += E * tile * 4;
     p.off_gacc = o; o += (E - p.n_vact) * tile * 4;
-    out->smem = o;
+    if (work_global) p.slab_floats = align_up_b(o, 16) / 4;
+    else out->smem = o;
     out->threads = kBwdThreads;
     p.n_tiles = (int)((B + tile - 1) / tile);
     out->grid = p.n_tiles < g->sm_count ? p.n_tiles : g->sm_count;
     out->n_rows = out->grid * (kBwdThreads / 32);
     return GD_OK;
+}
+
+// workspace: per-warp partials | the table backward's adjoint bins (gd_lean.cu) | the global-memory form's slab
+static int64_t bwd_slab_offset(const gd_graph* g, const gd_model* m, const BwdPlan& pl) {
+    return ((int64_t)pl.n_rows * pl.p.np_pad + lean_bwd_bins_floats(g, m) + 4 + 3) & ~(int64_t)3;
 }
 
 }  // namespace gd
@@ -569,7 +627,9 @@ extern "C" int64_t gd_bwd_workspace_floats(const gd_graph* g, const gd_model* mo
     }
     gd::BwdPlan pl;
     if (gd::plan_bwd(g, model, B, &pl) != GD_OK) return -1;
-    // per-warp partial gradient vectors of the edge-owner backward, then the adjoint bins of the table backward (gd_lean.cu)
+    // per-warp partial gradient vectors of the edge-owner backward, then the adjoint bins of the table backward (gd_lean.cu),
+    // then the per-CTA work slabs of the global-memory form
+    if (pl.work_global) return gd::bwd_slab_offset(g, model, pl) + (int64_t)pl.grid * pl.p.slab_floats;
     return (int64_t)pl.n_rows * pl.p.np_pad + gd::lean_bwd_bins_floats(g, model) + 4;
 }
 
@@ -602,6 +662,7 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
     if (rc != GD_OK) return rc;
     pl.p.x = x_dev; pl.p.stash = stash_dev; pl.p.grad_logit = grad_logit_dev; pl.p.weights = weights_dev;
     pl.p.partials = workspace_dev;
+    if (pl.work_global) pl.p.slab = workspace_dev + gd::bwd_slab_offset(g, model, pl);
     if (r.family == gd::Family::Lean) {
         // decoder_v2_4 on surface / toric codes: when the table forward wrote the stash (its header says so, on the device), the
         // table backward produces the gradient and the two kernels below return at once; otherwise the other way round
@@ -611,8 +672,9 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
         if (rc != GD_OK) return rc;
         pl.p.run_flag = &gd::lean_train_hdr(const_cast<float*>(stash_dev), g, model, B)->old_count;
     }
-    GD_CUDA(cudaFuncSetAttribute(gd::decode_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
-    GD_CUDA(gd::pdl_launch(gd::decode_bwd_kernel, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, pl.p));
+    void (*k)(const gd::BwdParams) = pl.work_global ? gd::decode_bwd_kernel<true> : gd::decode_bwd_kernel<false>;
+    GD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));
+    GD_CUDA(gd::pdl_launch(k, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, pl.p));
     GD_CUDA(gd::pdl_launch(gd::reduce_partials_kernel, dim3((n_params + 127) / 128), dim3(128), 0, st, workspace_dev, pl.n_rows,
                            pl.p.np_pad, n_params, grad_weights_dev, accumulate ? 1 : 0, pl.p.run_flag));
     return GD_OK;

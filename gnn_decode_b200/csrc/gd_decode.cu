@@ -1100,18 +1100,35 @@ int route_decode(const gd_graph* gc, const gd_model* m, int64_t B, Use use, Rout
             }
             return GD_OK;
         }
-        // decoder_v2_4: the table kernel over the whole graph when it plans, and the edge-owner pair in any case -- the header
-        // at the end of the stash tells the device which of them runs (gd_lean.cuh).  The backward plans the table kernel as
-        // the forward did; the edge-owner backward has its own planner (gd_backward.cu).
-        if (use == Use::Train) {
-            const int rc = plan_decode(g, m, B, &r->edge);
-            if (rc != GD_OK) return rc;
-            if (!r->edge.resident) {
-                set_error("gd_decode_fwd_train: code too large for the resident kernel (training needs it)");
+        // decoder_v2_4: where the edge-owner kernel is resident, the table kernel over the whole graph when it plans, and the
+        // edge-owner pair in any case -- the header at the end of the stash tells the device which of them runs (gd_lean.cuh).
+        // Elsewhere (and under GD_FORCE_STREAMED) the TMA-staged streamed kernel writes the edge-owner stash layout.  The
+        // backward plans the table kernel as the forward did; the edge-owner backward has its own planner (gd_backward.cu),
+        // which takes its shared-memory or its global-memory variant independently of the forward.
+        if (opt_on(OPT_FORCE_STREAMED)) {
+            r->family = Family::StreamedTma;
+        } else {
+            const bool lean = lean_plan(g, m, B, &r->lean, true);
+            if (lean || use == Use::Train) {         // the table kernel needs the resident edge-owner kernel (its deferred pass)
+                const int rc = plan_decode(g, m, B, &r->edge);
+                if (rc != GD_OK) return rc;
+                r->family = !r->edge.resident ? Family::StreamedTma : lean ? Family::Lean : Family::EdgeOwner;
+            } else {
+                r->family = Family::EdgeOwner;
+            }
+        }
+        if (use == Use::Train && r->family == Family::StreamedTma) {
+            if (g->E >= 65536) {
+                set_error("gd_decode_fwd_train: E=%lld edges; the backward's graph tables hold 16-bit edge ids (E < 65536)",
+                          (long long)g->E);
+                return GD_ERR_UNSUPPORTED;
+            }
+            plan_streamed_tma(g, m, B, &r->tma, true);
+            if (!r->tma.ok) {
+                set_error("gd_decode_fwd_train: the streamed training forward cannot take this graph: %s", r->tma.why);
                 return GD_ERR_UNSUPPORTED;
             }
         }
-        r->family = lean_plan(g, m, B, &r->lean, true) ? Family::Lean : Family::EdgeOwner;
         return GD_OK;
     }
     if (m->program == GD_PROG_V2_4_1) {

@@ -88,16 +88,20 @@ struct StreamTmaParams {
     int off_w, off_stage;    // shared-memory byte offsets (mbarriers sit at 0)
     int off_ctab, off_rtab, ctab_n, rtab_n;   // decoder_v2_4: cubic tables of the check-phase and read-out MLPs (0: none)
     float ctab_R;
+    float* stash;            // training (decoder_v2_4): [(T+1)][2][E][B], the edge-owner kernel's layout (gnn_decode.h)
 };
 
 struct StreamTmaPlan {
     StreamTmaParams p;
     int threads, grid, smem, npad;
     bool ok;                 // false: the register-batched kernel takes the call (plan_streamed_tma says why)
+    const char* why;         // the reason when !ok
 };
 
 int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* out);
-void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out);
+// train: decoder_v2_4's training forward (the kernel also writes the stash); no batch-size gate, training has no other
+// streamed kernel
+void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out, bool train = false);
 // the per-graph edge-state slab both streamed kernels use, grown to at least `bytes` (NULL and gd_last_error() on failure)
 float* streamed_slab(gd_graph* g, size_t bytes);
 

@@ -44,10 +44,8 @@ struct NodeMath {
     // variable phase: ext = (sum of siblings) - own, prior -> the value the check phase sums
     __device__ __forceinline__ void var_update(const float (&ext)[4], const float (&pr)[4], float (&out)[4]) const {
         if constexpr (PROG == GD_PROG_V2_4) {
-            float oo[4];
-            mlp_softplus_x2<4, true, 2>(W1, hp, ext, pr, oo);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) out[j] = tanh_half_fast(oo[j]);
+            float a[4];
+            var_update_a(ext, pr, a, out);
         } else if constexpr (kIsBP) {
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
@@ -59,6 +57,13 @@ struct NodeMath {
 #pragma unroll
             for (int j = 0; j < 4; ++j) out[j] = tanh_half_fast(ext[j] + pr[j]);
         }
+    }
+    // decoder_v2_4's variable phase that also returns a = mlp(ext, prior), the value before tanh(a/2): the training stash keeps it
+    __device__ __forceinline__ void var_update_a(const float (&ext)[4], const float (&pr)[4], float (&a)[4],
+                                                 float (&out)[4]) const {
+        mlp_softplus_x2<4, true, 2>(W1, hp, ext, pr, a);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) out[j] = tanh_half_fast(a[j]);
     }
     // check phase (learned programs): mlp(ext)
     __device__ __forceinline__ void chk_mlp(const float (&ext)[4], float (&oo)[4]) const {

@@ -62,8 +62,11 @@ __device__ __forceinline__ void wait(uint64_t* bar, uint32_t parity) {
 }
 }  // namespace tma
 
-template <int PROG, int NPAD>
+// STASH: decoder_v2_4's training forward -- also writes (m_it, a_it) of every edge and iteration and the final m into
+// p.stash, in the edge-owner kernel's layout [(T+1)][2][E][B], so either backward kernel (gd_backward.cu) can take it.
+template <int PROG, int NPAD, bool STASH = false>
 __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const StreamTmaParams p) {
+    static_assert(!STASH || PROG == GD_PROG_V2_4, "the training stash exists for decoder_v2_4 only");
     extern __shared__ __align__(128) unsigned char smem[];
     using NM = NodeMath<PROG, NPAD>;
     constexpr bool kIsBP = NM::kIsBP;
@@ -197,6 +200,16 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
         tma::wait(bar0 + sidx, (parbits >> sidx) & 1u);
         parbits ^= 1u << sidx;
     };
+    // training: this lane's float4 of stash row `row` (syndromes s0 + l4 ..); past s0 + nvalid the row runs into the next one
+    const bool stash_vec = STASH && (p.B & 3) == 0 && ((uintptr_t)p.stash & 15) == 0;
+    auto stash4 = [&](size_t row, long long s0, int nvalid, const float (&v)[4]) {
+        float* d = p.stash + row * (size_t)p.B + s0 + l4;
+        if (stash_vec) {
+            if (l4 < nvalid) __stcg(reinterpret_cast<float4*>(d), make_float4(v[0], v[1], v[2], v[3]));
+        } else {
+            for (int j = 0; j < 4 && l4 + j < nvalid; ++j) __stcg(d + j, v[j]);
+        }
+    };
 
     for (int tix = blockIdx.x; tix < p.n_tiles; tix += gridDim.x) {
         const long long s0 = (long long)tix * tile;
@@ -250,6 +263,7 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
                                         const float4 mv = lds4(rows + k * tile);
                                         if constexpr (PROG == GD_PROG_V2_4) {     // per-EDGE read-out MLP, then the sum
                                             float xi[4] = {mv.x, mv.y, mv.z, mv.w}, oo[4];
+                                            if constexpr (STASH) stash4((size_t)p.T * 2 * E + b + k, s0, nvalid, xi);   // m_T
                                             nm.readout_edge(xi, oo);
 #pragma unroll
                                             for (int j = 0; j < 4; ++j) acc[j] += oo[j];
@@ -260,13 +274,39 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
                                 } else if constexpr (PROG == GD_PROG_V2_4) {      // T == 0: mlp(0) per edge
                                     float xi[4] = {0.f, 0.f, 0.f, 0.f}, oo[4];
                                     mlp_softplus_x2<4, false, 2>(nm.W3, nm.hp, xi, xi, oo);
-                                    for (int k = 0; k < d; ++k)
+                                    for (int k = 0; k < d; ++k) {
+                                        if constexpr (STASH) stash4((size_t)b + k, s0, nvalid, xi);
 #pragma unroll
                                         for (int j = 0; j < 4; ++j) acc[j] += oo[j];
+                                    }
                                 }
                                 float lg[4] = {acc[0] + pr.x, acc[1] + pr.y, acc[2] + pr.z, acc[3] + pr.w};
                                 nm.readout_mlp(lg);
                                 stg4(lg_st + (size_t)v * tile + l4, lg);
+                            } else if constexpr (STASH) {
+                                // training: the generic loop of the inference path below, with (m_it, a_it) of every edge
+                                // (edge id b + k: canonical order) into the stash
+                                float* tout = t_st + (size_t)b * tile + l4;
+                                float acc[4] = {0.f, 0.f, 0.f, 0.f};
+                                if (with_m)
+                                    for (int k = 0; k < d; ++k) {      // ascending edge id
+                                        const float4 mv = lds4(rows + k * tile);
+                                        acc[0] += mv.x; acc[1] += mv.y; acc[2] += mv.z; acc[3] += mv.w;
+                                    }
+                                const float prv[4] = {pr.x, pr.y, pr.z, pr.w};
+                                for (int k = 0; k < d; ++k) {
+                                    float mo[4] = {0.f, 0.f, 0.f, 0.f};
+                                    if (with_m) {
+                                        const float4 mv = lds4(rows + k * tile);
+                                        mo[0] = mv.x; mo[1] = mv.y; mo[2] = mv.z; mo[3] = mv.w;
+                                    }
+                                    const float ext[4] = {acc[0] - mo[0], acc[1] - mo[1], acc[2] - mo[2], acc[3] - mo[3]};
+                                    float a[4], out[4];
+                                    nm.var_update_a(ext, prv, a, out);
+                                    stg4(tout + k * tile, out);
+                                    stash4((size_t)it * 2 * E + b + k, s0, nvalid, mo);
+                                    stash4((size_t)(it * 2 + 1) * E + b + k, s0, nvalid, a);
+                                }
                             } else {
                                 float* tout = t_st + (size_t)b * tile + l4;
 #define GD_VAR_CALL(D) nm.template var_node<D>(rows, tile, pr, tout)
@@ -431,14 +471,16 @@ _Pragma("unroll")
 
 static int align_up_i(int x, int a) { return (x + a - 1) / a * a; }
 
-// Returns ok == false when the graph does not qualify (edges not in variable-sorted order, or a
+// Returns ok == false (and out->why) when the graph does not qualify (edges not in variable-sorted order, or a
 // node's rows do not fit a pipeline stage): the caller then takes the register-batched kernel.
-void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out) {
+void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out, bool train) {
     StreamTmaParams& p = out->p;
     memset(&p, 0, sizeof(p));
     out->ok = false;
+    out->why = "edges are not in the canonical variable-sorted order (H.to_sparse())";
     for (size_t i = 0; i < g->h_var_edges.size(); ++i)
         if (g->h_var_edges[i] != (int32_t)i) return;
+    out->why = "a node's rows do not fit a pipeline stage in shared memory";
     const bool bp = m->program == GD_PROG_BP_QUANTUM || m->program == GD_PROG_BP_CLASSICAL;
     p.B = B; p.T = m->iters; p.V = g->V; p.C = g->C; p.E = (int)g->E; p.N = g->N;
     p.hid = bp ? 0 : m->hidden;
@@ -447,7 +489,10 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
     const int n_slots = bp ? 0 : (m->program == GD_PROG_V2_4 ? 3 : 2);
     // The Softplus program is MUFU-bound, not HBM-bound: four syndromes per lane only pay when the
     // batch fills all 32 lanes of every SM; smaller batches take the register-batched kernel.
-    if (m->program == GD_PROG_V2_4 && B < (int64_t)128 * g->sm_count) return;
+    if (m->program == GD_PROG_V2_4 && !train && B < (int64_t)128 * g->sm_count) {
+        out->why = "batch too small to fill the SMs";
+        return;
+    }
     out->npad = 0;
     if ((m->program == GD_PROG_CGNNI || m->program == GD_PROG_QGNNI) && m->hidden < 32)
         out->npad = m->hidden < 16 ? 16 : 32;
@@ -509,9 +554,14 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
 int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st) {
     StreamTmaPlan pl = plan;
     pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
+    pl.p.stash = io.stash;
     pl.p.slab = streamed_slab(g, (size_t)pl.grid * (size_t)pl.p.slab_floats * sizeof(float));
     if (!pl.p.slab) return GD_ERR_CUDA;
     void (*k)(const StreamTmaParams);
+    if (io.stash && model->program != GD_PROG_V2_4) {
+        set_error("gd_decode_fwd_train: the streamed kernel writes a training stash for GD_PROG_V2_4 only");
+        return GD_ERR_UNSUPPORTED;
+    }
     switch (model->program) {
         case GD_PROG_CGNNI:
             k = pl.npad == 16 ? decode_streamed_tma_kernel<GD_PROG_CGNNI, 16>
@@ -521,7 +571,9 @@ int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& plan, const gd_model* 
             k = pl.npad == 16 ? decode_streamed_tma_kernel<GD_PROG_QGNNI, 16>
                 : pl.npad == 32 ? decode_streamed_tma_kernel<GD_PROG_QGNNI, 32> : decode_streamed_tma_kernel<GD_PROG_QGNNI, 0>;
             break;
-        case GD_PROG_V2_4: k = decode_streamed_tma_kernel<GD_PROG_V2_4, 0>; break;
+        case GD_PROG_V2_4:
+            k = io.stash ? decode_streamed_tma_kernel<GD_PROG_V2_4, 0, true> : decode_streamed_tma_kernel<GD_PROG_V2_4, 0>;
+            break;
         case GD_PROG_BP_QUANTUM: k = decode_streamed_tma_kernel<GD_PROG_BP_QUANTUM, 0>; break;
         default: k = decode_streamed_tma_kernel<GD_PROG_BP_CLASSICAL, 0>; break;
     }

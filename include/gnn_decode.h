@@ -229,6 +229,11 @@ int gd_pipeline_drain(gd_pipeline* p);   /* wait for every batch submitted so fa
  *      gd_stash_floats() floats:
  *        GD_PROG_V2_4 : [(iters+1)][2][E][B] (+ a header of the table kernel, gd_lean.cuh);
  *        GD_PROG_CGNNI: [iters][E][B], m after every iteration (the backward recomputes the rest).
+ *      GD_PROG_V2_4 trains on any code the library decodes: where the edge state does not fit shared memory
+ *      (or under GD_FORCE_STREAMED) the forward is the TMA-staged streamed kernel writing the same stash
+ *      layout, and where the backward's per-tile arrays do not fit shared memory its work arrays go to the
+ *      workspace; the two choices are independent.  There, graphs in another edge order than the canonical
+ *      variable-sorted one, and graphs with E >= 65536, return GD_ERR_UNSUPPORTED.
  *      GD_PROG_CGNNI trains on the node-owner kernel only: graphs in another edge order than the canonical
  *      variable-sorted one, and codes whose edge state does not fit shared memory, return GD_ERR_UNSUPPORTED.
  *      gd_decode_bwd takes dL/dlogit [B,V], the gradient w.r.t. the logit BEFORE the clamp the classical
@@ -236,7 +241,9 @@ int gd_pipeline_drain(gd_pipeline* p);   /* wait for every batch submitted so fa
  *      prob = clamp(s, 1e-7, 1-1e-7), s = sigmoid(-logit): -dL/dprob * s * (1 - s) where 1e-7 <= s <= 1-1e-7,
  *      else 0) and writes (accumulate == 0) or adds (accumulate != 0) dL/dweights in the packed order of
  *      gd_model.  workspace_dev: gd_bwd_workspace_floats() floats (8-byte aligned) of per-warp partial sums
- *      (GD_PROG_V2_4) or per-CTA fixed-point bins (GD_PROG_CGNNI), reduced in a fixed order ->
+ *      (GD_PROG_V2_4; where the backward does not fit shared memory also one work slab per CTA, about
+ *      390 KB per syndrome of the CTA's tile at HGP [[1600,64]]) or per-CTA fixed-point bins
+ *      (GD_PROG_CGNNI), reduced in a fixed order ->
  *      bit-reproducible gradients; gd_bwd_workspace_floats returns -1 for other programs. ---- */
 int64_t gd_stash_floats(const gd_graph* g, const gd_model* model, int64_t B);
 int gd_decode_fwd_train(const gd_graph* g, const gd_model* model, const float* weights_dev,
