@@ -77,33 +77,30 @@ extern "C" int gd_microbench(int32_t kind, int32_t iters, int device, double* re
     GD_CUDA(dg.status());
     cudaDeviceProp prop;
     GD_CUDA(cudaGetDeviceProperties(&prop, device));
-    float* out = nullptr;
-    GD_CUDA(cudaMalloc((void**)&out, 4));
+    gd::DeviceBuffer<float> out;
+    GD_CUDA(gd::device_alloc(out, 4));
     const int grid = kind == 7 ? prop.multiProcessorCount : prop.multiProcessorCount * 4, threads = kind == 7 ? 1024 : 512;
-    cudaEvent_t e0, e1;
-    cudaEventCreate(&e0);
-    cudaEventCreate(&e1);
+    gd::Event e0, e1;
+    GD_CUDA(gd::create(e0, cudaEventCreateWithFlags, cudaEventDefault));
+    GD_CUDA(gd::create(e1, cudaEventCreateWithFlags, cudaEventDefault));
     float ms = 0.f;
     for (int rep = 0; rep < 3; ++rep) {   // first two are warm-up
-        cudaEventRecord(e0);
+        cudaEventRecord(e0.get());
         switch (kind) {
-            case 0: gd::ubench_kernel<0><<<grid, threads>>>(out, iters); break;
-            case 1: gd::ubench_kernel<1><<<grid, threads>>>(out, iters); break;
-            case 2: gd::ubench_kernel<2><<<grid, threads>>>(out, iters); break;
-            case 3: gd::ubench_kernel<3><<<grid, threads>>>(out, iters); break;
-            case 4: gd::ubench_kernel<4><<<grid, threads>>>(out, iters); break;
-            case 5: gd::ubench_kernel<5><<<grid, threads>>>(out, iters); break;
-            case 7: gd::lds_bench_kernel<<<grid, threads>>>(out, iters); break;
-            default: gd::ubench_kernel<6><<<grid, threads>>>(out, iters); break;
+            case 0: gd::ubench_kernel<0><<<grid, threads>>>(out.get(), iters); break;
+            case 1: gd::ubench_kernel<1><<<grid, threads>>>(out.get(), iters); break;
+            case 2: gd::ubench_kernel<2><<<grid, threads>>>(out.get(), iters); break;
+            case 3: gd::ubench_kernel<3><<<grid, threads>>>(out.get(), iters); break;
+            case 4: gd::ubench_kernel<4><<<grid, threads>>>(out.get(), iters); break;
+            case 5: gd::ubench_kernel<5><<<grid, threads>>>(out.get(), iters); break;
+            case 7: gd::lds_bench_kernel<<<grid, threads>>>(out.get(), iters); break;
+            default: gd::ubench_kernel<6><<<grid, threads>>>(out.get(), iters); break;
         }
-        cudaEventRecord(e1);
-        cudaEventSynchronize(e1);
-        cudaEventElapsedTime(&ms, e0, e1);
+        cudaEventRecord(e1.get());
+        cudaEventSynchronize(e1.get());
+        cudaEventElapsedTime(&ms, e0.get(), e1.get());
     }
     cudaError_t e = cudaGetLastError();
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    cudaFree(out);
     GD_CUDA(e);
     // kind 7: units = 128-byte shared-memory wavefronts (a warp-wide 128-bit load is 4 of them)
     const double units = (double)grid * threads * (double)iters * 8.0 * (kind == 7 ? 4.0 / 32.0 : 1.0);

@@ -6,7 +6,10 @@
 #include <stdarg.h>
 #include <string.h>
 #include <vector>
+#include <memory>
 #include <mutex>
+#include <type_traits>
+#include <utility>
 
 #include "../../include/gnn_decode.h"
 
@@ -56,6 +59,67 @@ private:
     cudaError_t err_ = cudaSuccess;
 };
 
+// Owners of device memory and CUDA handles: each releases what it holds when it goes out of scope or is reset, so the
+// library's host code frees nothing by hand.  Fill them with device_alloc / create, which leave them empty on failure.
+template <class H, cudaError_t (*Free)(H)> struct Release { void operator()(H h) const { Free(h); } };
+template <class T> using DeviceBuffer = std::unique_ptr<T, Release<void*, cudaFree>>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, Release<cudaEvent_t, cudaEventDestroy>>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, Release<cudaStream_t, cudaStreamDestroy>>;
+using MemPool = std::unique_ptr<std::remove_pointer_t<cudaMemPool_t>, Release<cudaMemPool_t, cudaMemPoolDestroy>>;
+
+// frees what `buf` holds first, so a buffer that grows never holds both sizes at once
+template <class T> cudaError_t device_alloc(DeviceBuffer<T>& buf, size_t bytes) {
+    buf.reset();
+    void* p = nullptr;
+    const cudaError_t e = cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) buf.reset(static_cast<T*>(p));
+    return e;
+}
+// create(ev, cudaEventCreateWithFlags, flags): runs a CUDA create call and gives the handle it made to the owner
+template <class Owner, class... P, class... A>
+cudaError_t create(Owner& owner, cudaError_t (*make)(typename Owner::pointer*, P...), A... args) {
+    typename Owner::pointer h = nullptr;
+    const cudaError_t e = make(&h, args...);
+    owner.reset(e == cudaSuccess ? h : nullptr);
+    return e;
+}
+
+// A stream-ordered allocation from a memory pool, returned with cudaFreeAsync on the stream it was made for.  The success
+// path calls release() and checks what it returns; on any other return the destructor frees it.
+template <class T> class PoolAlloc {
+public:
+    explicit PoolAlloc(cudaStream_t st) : st_(st) {}
+    ~PoolAlloc() { release(); }
+    PoolAlloc(const PoolAlloc&) = delete;
+    PoolAlloc& operator=(const PoolAlloc&) = delete;
+    cudaError_t alloc(size_t bytes, cudaMemPool_t pool) {
+        const cudaError_t e = cudaMallocFromPoolAsync(&p_, bytes, pool, st_);
+        if (e != cudaSuccess) p_ = nullptr;
+        return e;
+    }
+    T* get() const { return p_; }
+    cudaError_t release() {
+        T* p = std::exchange(p_, nullptr);
+        return p ? cudaFreeAsync(p, st_) : cudaSuccess;
+    }
+
+private:
+    T* p_ = nullptr;
+    cudaStream_t st_;
+};
+
+// Deleter of the graph's lazily made state (HostCtx: gd_host.cu, LeanCtx: gd_lean.cu).  Each type is complete only in its own
+// file, so that file instantiates the deleter (`template struct gd::Delete<T>;`) and every other file links to it.
+template <class T> struct Delete { void operator()(T* p) const; };
+template <class T> void Delete<T>::operator()(T* p) const { delete p; }
+struct HostCtx;
+struct LeanCtx;
+extern template struct Delete<HostCtx>;
+extern template struct Delete<LeanCtx>;
+
+// the per-graph edge-state slab both streamed kernels use, grown to at least `bytes` (NULL and gd_last_error() on failure)
+float* streamed_slab(gd_graph* g, size_t bytes);
+
 // Device blob layout (int32 words): all tables of one Tanner graph, uploaded once.
 struct GraphTables {
     const int32_t* edge_var;   // [E]   variable endpoint of edge e
@@ -100,16 +164,16 @@ struct gd_graph {
     int sm_count;
     int max_smem_optin;
     int max_smem_sm;
-    int32_t* blob_dev;          // single allocation holding all tables
+    gd::DeviceBuffer<int32_t> blob_dev;   // single allocation holding all tables
     gd::GraphTables t;          // device pointers into blob_dev
     std::vector<int32_t> h_edge_var, h_edge_chk, h_var_ptr, h_var_edges, h_chk_ptr, h_chk_edges, h_vlist;
-    // lazily grown scratch (guarded by mu): global edge-state workspace for codes too large
-    // for shared memory, and gd_decode_host's internal pipeline.
+    // made on first use (guarded by mu).  Members are destroyed in reverse order, so teardown runs: gd_decode_host's pipeline
+    // (batches in flight decode through the rest), the table cache (each table set waits for its last use), the slab, blob_dev.
     std::mutex mu;
-    float* gstate;
-    size_t gstate_bytes;
-    void* host_ctx;             // gd_decode_host pipeline state (see gd_host.cu)
-    void* lean_ctx;             // check-owner table kernel: per-(R) metadata, workspace pool (see gd_lean.cu)
+    gd::DeviceBuffer<float> gstate;   // global edge-state slab of the streamed kernels, for codes too large for shared memory
+    size_t gstate_bytes = 0;
+    std::unique_ptr<gd::LeanCtx, gd::Delete<gd::LeanCtx>> lean_ctx;   // table kernel: metadata, table sets, pool (gd_lean.cu)
+    std::unique_ptr<gd::HostCtx, gd::Delete<gd::HostCtx>> host_ctx;   // gd_decode_host's internal pipeline (gd_host.cu)
     // geometries measured by gd_decode_autotune (guarded by mu): key = {program, hidden, iters, flags, B}
     struct TunedGeom { int32_t program, hidden, iters, flags; int64_t B; int32_t tile, R, eb; };
     std::vector<TunedGeom> tuned;

@@ -1389,11 +1389,11 @@ extern "C" int gd_decode_autotune(const gd_graph* gc, const gd_model* model, con
         if (!dup) pick.push_back(c);
         if ((int)pick.size() >= K) break;
     }
-    float* prob = nullptr;
-    cudaError_t e = cudaMalloc((void**)&prob, (size_t)B * g->V * sizeof(float));
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (e == cudaSuccess) e = cudaEventCreate(&e0);
-    if (e == cudaSuccess) e = cudaEventCreate(&e1);
+    gd::DeviceBuffer<float> prob;
+    gd::Event e0, e1;
+    cudaError_t e = gd::device_alloc(prob, (size_t)B * g->V * sizeof(float));
+    if (e == cudaSuccess) e = gd::create(e0, cudaEventCreateWithFlags, cudaEventDefault);
+    if (e == cudaSuccess) e = gd::create(e1, cudaEventCreateWithFlags, cudaEventDefault);
     gd::GeomCand best{0, 0, 0, 0.0};
     float best_ms = 1e30f;
     for (size_t i = 0; i < pick.size() && e == cudaSuccess && rc == GD_OK; ++i) {
@@ -1410,19 +1410,16 @@ extern "C" int gd_decode_autotune(const gd_graph* gc, const gd_model* model, con
         }
         float ms = 1e30f;
         for (int rep = 0; rep < 3 && rc == GD_OK && e == cudaSuccess; ++rep) {       // first launch warms up
-            cudaEventRecord(e0, st);
-            rc = gd_decode_fwd(g, model, weights_dev, x_dev, prob, nullptr, nullptr, B, st);
-            cudaEventRecord(e1, st);
-            e = cudaEventSynchronize(e1);
+            cudaEventRecord(e0.get(), st);
+            rc = gd_decode_fwd(g, model, weights_dev, x_dev, prob.get(), nullptr, nullptr, B, st);
+            cudaEventRecord(e1.get(), st);
+            e = cudaEventSynchronize(e1.get());
             float t = 0.f;
-            if (e == cudaSuccess) cudaEventElapsedTime(&t, e0, e1);
+            if (e == cudaSuccess) cudaEventElapsedTime(&t, e0.get(), e1.get());
             if (rep > 0 && t < ms) ms = t;
         }
         if (ms < best_ms) { best_ms = ms; best = pick[i]; }
     }
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    if (prob) cudaFree(prob);
     if (best.tile) {
         std::lock_guard<std::mutex> lk(g->mu);
         for (size_t q = 0; q < g->tuned.size(); ++q)

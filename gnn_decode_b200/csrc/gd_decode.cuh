@@ -102,8 +102,6 @@ int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* o
 // train: decoder_v2_4's training forward (the kernel also writes the stash); no batch-size gate, training has no other
 // streamed kernel
 void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out, bool train = false);
-// the per-graph edge-state slab both streamed kernels use, grown to at least `bytes` (NULL and gd_last_error() on failure)
-float* streamed_slab(gd_graph* g, size_t bytes);
 
 // ---- routing ----
 // The buffers of one decode call; NULL where the call does not ask for them.

@@ -75,10 +75,10 @@ extern "C" int gd_graph_create(const int64_t* ei, int64_t E, int32_t V, int32_t 
     GD_CUDA(cudaGetDeviceCount(&n_dev));
     GD_CHECK_ARG(device >= 0 && device < n_dev, "gd_graph_create: device %d not in [0,%d)", device, n_dev);
 
-    gd_graph* g = new (std::nothrow) gd_graph();
+    gd::DeviceGuard dg(device);                     // also for the release of the graph's storage if creation fails
+    std::unique_ptr<gd_graph> g(new (std::nothrow) gd_graph());
     GD_CHECK_ARG(g != nullptr, "gd_graph_create: out of host memory");
     g->V = V; g->C = C; g->N = V + C; g->E = E; g->device = device;
-    g->gstate = nullptr; g->gstate_bytes = 0; g->host_ctx = nullptr; g->lean_ctx = nullptr; g->blob_dev = nullptr;
     g->h_edge_var.resize((size_t)E);
     g->h_edge_chk.resize((size_t)E);
     for (int64_t e = 0; e < E; ++e) {
@@ -113,48 +113,49 @@ extern "C" int gd_graph_create(const int64_t* ei, int64_t E, int32_t V, int32_t 
     put(g->h_edge_var, o_ev); put(g->h_edge_chk, o_ec); put(g->h_var_ptr, o_vp);
     put(g->h_var_edges, o_ve); put(g->h_chk_ptr, o_cp); put(g->h_chk_edges, o_ce); put(g->h_vlist, o_vl);
 
-    cudaError_t e;
     cudaDeviceProp prop;
-    {
-        gd::DeviceGuard dg(device);
-        e = dg.status();
-        if (e == cudaSuccess) e = cudaMalloc((void**)&g->blob_dev, words * sizeof(int32_t));
-        if (e == cudaSuccess) e = cudaMemcpy(g->blob_dev, blob.data(), words * sizeof(int32_t), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, device);
-    }
+    cudaError_t e = dg.status();
+    if (e == cudaSuccess) e = gd::device_alloc(g->blob_dev, words * sizeof(int32_t));
+    if (e == cudaSuccess) e = cudaMemcpy(g->blob_dev.get(), blob.data(), words * sizeof(int32_t), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaGetDeviceProperties(&prop, device);
     if (e != cudaSuccess) {
         gd::set_error("gd_graph_create: CUDA failure: %s", cudaGetErrorString(e));
-        if (g->blob_dev) cudaFree(g->blob_dev);
-        delete g;
         return GD_ERR_CUDA;
     }
     g->sm_count = prop.multiProcessorCount;
     g->max_smem_optin = (int)prop.sharedMemPerBlockOptin;
     g->max_smem_sm = (int)prop.sharedMemPerMultiprocessor;
-    g->t.edge_var = g->blob_dev + o_ev;
-    g->t.edge_chk = g->blob_dev + o_ec;
-    g->t.var_ptr = g->blob_dev + o_vp;
-    g->t.var_edges = g->blob_dev + o_ve;
-    g->t.chk_ptr = g->blob_dev + o_cp;
-    g->t.chk_edges = g->blob_dev + o_ce;
-    g->t.vlist = g->blob_dev + o_vl;
-    *out = g;
+    g->t.edge_var = g->blob_dev.get() + o_ev;
+    g->t.edge_chk = g->blob_dev.get() + o_ec;
+    g->t.var_ptr = g->blob_dev.get() + o_vp;
+    g->t.var_edges = g->blob_dev.get() + o_ve;
+    g->t.chk_ptr = g->blob_dev.get() + o_cp;
+    g->t.chk_edges = g->blob_dev.get() + o_ce;
+    g->t.vlist = g->blob_dev.get() + o_vl;
+    *out = g.release();
     return GD_OK;
 }
 
-void gd_host_ctx_destroy(gd_graph* g);  // gd_host.cu
-void gd_lean_ctx_destroy(gd_graph* g);  // gd_lean.cu
-
 extern "C" void gd_graph_destroy(gd_graph* g) {
     if (!g) return;
-    {
-        gd::DeviceGuard dg(g->device);
-        gd_host_ctx_destroy(g);
-        gd_lean_ctx_destroy(g);
-        if (g->gstate) cudaFree(g->gstate);
-        if (g->blob_dev) cudaFree(g->blob_dev);
+    gd::DeviceGuard dg(g->device);
+    std::unique_ptr<gd_graph> owned(g);          // released on the graph's device, in the order gd_graph declares
+}
+
+// The slab is per graph: concurrent streamed decodes of one graph on different streams must be serialised by the caller
+// (documented in include/gnn_decode.h).
+float* gd::streamed_slab(gd_graph* g, size_t bytes) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (bytes > g->gstate_bytes) {
+        g->gstate_bytes = 0;
+        cudaError_t e = device_alloc(g->gstate, bytes);
+        if (e != cudaSuccess) {
+            set_error("gd_decode_fwd: cudaMalloc of the %zu-byte streamed edge-state slab failed: %s", bytes, cudaGetErrorString(e));
+            return nullptr;
+        }
+        g->gstate_bytes = bytes;
     }
-    delete g;
+    return g->gstate.get();
 }
 
 extern "C" int gd_graph_dims(const gd_graph* g, int32_t* V, int32_t* C, int64_t* E, int32_t* max_var_deg,
@@ -214,21 +215,20 @@ extern "C" int gd_graph_check_batched(const gd_graph* g, const int64_t* ei_dev, 
     cudaStream_t st = (cudaStream_t)stream;
     gd::DeviceGuard dg(g->device);
     GD_CUDA(dg.status());
-    unsigned long long* bad = nullptr;
-    cudaError_t e = cudaMalloc((void**)&bad, sizeof(unsigned long long));
-    if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0, sizeof(unsigned long long), st);
+    gd::DeviceBuffer<unsigned long long> bad;
+    cudaError_t e = gd::device_alloc(bad, sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMemsetAsync(bad.get(), 0, sizeof(unsigned long long), st);
     if (e == cudaSuccess) {
         const int64_t total = g->E * B;
         int blocks = (int)((total + 255) / 256);
         if (blocks > g->sm_count * 8) blocks = g->sm_count * 8;
         check_batched_kernel<<<blocks, 256, 0, st>>>(ei_dev, g->t.edge_var, g->t.edge_chk, g->E, B, g->N,
-                                                     chk_offset, bad);
+                                                     chk_offset, bad.get());
         e = cudaGetLastError();
     }
     unsigned long long h = 0;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&h, bad, sizeof(h), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&h, bad.get(), sizeof(h), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (bad) cudaFree(bad);
     GD_CUDA(e);
     *mismatches_host = (int64_t)h;
     return GD_OK;

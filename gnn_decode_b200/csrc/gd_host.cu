@@ -12,17 +12,11 @@ struct HostCtx {
     gd_pipeline* pipe = nullptr;
     gd_model model{};                // the pipeline was created for this model ...
     int64_t max_B = 0;               // ... and chunks of up to max_B syndromes
+    ~HostCtx() { gd_pipeline_destroy(pipe); }
 };
+template struct Delete<HostCtx>;
 
 }  // namespace gd
-
-void gd_host_ctx_destroy(gd_graph* g) {
-    gd::HostCtx* c = static_cast<gd::HostCtx*>(g->host_ctx);
-    if (!c) return;
-    gd_pipeline_destroy(c->pipe);
-    delete c;
-    g->host_ctx = nullptr;
-}
 
 extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const float* weights_host,
                               const float* x_host, float* prob_host, uint8_t* hard_host, int64_t B) {
@@ -50,8 +44,8 @@ extern "C" int gd_decode_host(const gd_graph* gc, const gd_model* model, const f
     const int64_t per = ((B + n_chunks - 1) / n_chunks + 7) / 8 * 8;
 
     std::unique_lock<std::mutex> lk(g->mu);
-    if (!g->host_ctx) g->host_ctx = new gd::HostCtx();
-    gd::HostCtx* c = static_cast<gd::HostCtx*>(g->host_ctx);
+    if (!g->host_ctx) g->host_ctx.reset(new gd::HostCtx());
+    gd::HostCtx* c = g->host_ctx.get();
     lk.unlock();  // gd_decode_fwd takes the same mutex for the streamed workspace
     std::lock_guard<std::mutex> call_lk(c->call_mu);
     const bool same_model = c->model.program == model->program && c->model.hidden == model->hidden &&

@@ -1179,7 +1179,7 @@ struct LeanSub {
 struct LeanMeta {
     int sub = -1;
     int R = 0, NCH = 0;
-    uint32_t* dev = nullptr;
+    DeviceBuffer<uint32_t> dev;
     size_t bytes = 0;
     int off_ms = 0, off_mi = 0, off_var = 0;   // byte offsets inside the blob (me at 0)
     double balance = 0.0;
@@ -1194,26 +1194,35 @@ struct LeanEntry {
     cudaStream_t st = nullptr;
     const float* w = nullptr;
     int T = 0, hid = 0, ct_n = 0, rt_n = 0, vt_n = 0;
-    unsigned char* dev = nullptr;          // header | ctab | rtab | vtab
+    DeviceBuffer<unsigned char> dev;       // header | ctab | rtab | vtab
     size_t o_ct = 0, o_rt = 0, o_vt = 0;
-    cudaEvent_t ev = nullptr;
+    Event ev;                              // recorded after each use of the tables
     unsigned long long last_use = 0;
     unsigned long long calls = 0;          // decode calls enqueued on this entry: selects the header's LeanCall
+    ~LeanEntry() { if (ev) cudaEventSynchronize(ev.get()); }   // the blob goes only after its last use
 };
 constexpr int kMaxEntries = 4;
 struct LeanCtx {
-    std::vector<LeanMeta*> metas;          // one per (part, R) ever planned (stable addresses)
-    std::vector<LeanSub*> subs;            // [0] = the whole graph, [1 ..] = its connected components (when they can be decoded apart)
+    std::vector<std::unique_ptr<LeanMeta>> metas;   // one per (part, R) ever planned (stable addresses: plans point at them)
+    std::vector<std::unique_ptr<LeanSub>> subs;     // [0] = the whole graph, [1 ..] = its connected components (when they can be decoded apart)
     bool subs_done = false;
     long long mode_epoch = -1;             // parts decision per option set: [0] inference, [1] training (whole graph only)
     int mode[2] = {-2, -2}, mode_ri[2] = {-1, -1};
     std::vector<LeanGeom> geoms;           // geometry search results per tiles-per-CTA count, redone when an option changes
     std::vector<LeanBwdGeom> bwd;          // ... of the training backward
-    cudaMemPool_t pool = nullptr;
+    MemPool pool;
     std::mutex enq;                        // one call at a time enqueues on a graph (entries are shared state)
-    std::vector<LeanEntry*> entries;
+    std::vector<std::unique_ptr<LeanEntry>> entries;   // destroyed first: each waits for its last use
     unsigned long long tick = 0;
 };
+template struct Delete<LeanCtx>;
+
+// the graph's table-kernel state, made on first use
+static LeanCtx* lean_ctx_of(gd_graph* g) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    if (!g->lean_ctx) g->lean_ctx.reset(new LeanCtx());
+    return g->lean_ctx.get();
+}
 
 static int align_up_i(int x, int a) { return (x + a - 1) / a * a; }
 
@@ -1245,18 +1254,17 @@ static void assign_owners(const gd_graph* g, const LeanSub* sub, int R, std::vec
 
 // parts of the graph: [0] the whole graph; [1 ..] its connected components, kept only when there are several, each holds a
 // contiguous range of variables (the output rows are written range by range) and at least one check
-static const std::vector<LeanSub*>& lean_subs(gd_graph* g) {
+static const std::vector<std::unique_ptr<LeanSub>>& lean_subs(gd_graph* g) {
+    LeanCtx* ctx = lean_ctx_of(g);
     std::lock_guard<std::mutex> lk(g->mu);
-    if (!g->lean_ctx) g->lean_ctx = new LeanCtx();
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
     if (ctx->subs_done) return ctx->subs;
     const int E = (int)g->E, V = g->V, C = g->C;
-    LeanSub* whole = new LeanSub();
+    auto whole = std::make_unique<LeanSub>();
     whole->v_lo = 0; whole->nv = V; whole->E = E;
     for (int c = 0; c < C; ++c) whole->checks.push_back(c);
     whole->edge_local.resize(E);
     for (int e = 0; e < E; ++e) whole->edge_local[e] = e;
-    ctx->subs.push_back(whole);
+    ctx->subs.push_back(std::move(whole));
     // union-find over the nodes (variables 0 .. V-1, checks V .. V+C-1)
     std::vector<int> parent(V + C);
     for (int i = 0; i < V + C; ++i) parent[i] = i;
@@ -1266,12 +1274,12 @@ static const std::vector<LeanSub*>& lean_subs(gd_graph* g) {
         if (a != b) parent[std::max(a, b)] = std::min(a, b);
     }
     std::vector<int> comp_of(V + C, -1);
-    std::vector<LeanSub*> comps;
+    std::vector<std::unique_ptr<LeanSub>> comps;
     bool ok = true;
     for (int c = 0; c < C; ++c) {
         if (g->h_chk_ptr[c + 1] == g->h_chk_ptr[c]) continue;   // an empty check belongs nowhere (and does nothing)
         const int root = find(V + c);
-        if (comp_of[root] < 0) { comp_of[root] = (int)comps.size(); comps.push_back(new LeanSub()); comps.back()->edge_local.assign(E, -1); }
+        if (comp_of[root] < 0) { comp_of[root] = (int)comps.size(); comps.push_back(std::make_unique<LeanSub>()); comps.back()->edge_local.assign(E, -1); }
         comps[comp_of[root]]->checks.push_back(c);
     }
     std::vector<int> vmin(comps.size(), V), vmax(comps.size(), -1), vcnt(comps.size(), 0);
@@ -1286,29 +1294,26 @@ static const std::vector<LeanSub*>& lean_subs(gd_graph* g) {
     for (size_t k = 0; k < comps.size() && ok; ++k) ok = vcnt[k] > 0 && vmax[k] - vmin[k] + 1 == vcnt[k];
     if (ok && comps.size() >= 2 && comps.size() <= 8) {
         for (size_t k = 0; k < comps.size(); ++k) {
-            LeanSub* s = comps[k];
+            LeanSub* s = comps[k].get();
             s->id = (int)k; s->v_lo = vmin[k]; s->nv = vcnt[k];
             int n = 0;
             for (int e = 0; e < E; ++e)
                 if (comp_of[find(V + g->h_edge_chk[e])] == (int)k) s->edge_local[e] = n++;
             s->E = n;
-            ctx->subs.push_back(s);
+            ctx->subs.push_back(std::move(comps[k]));
         }
-    } else {
-        for (LeanSub* s : comps) delete s;
     }
     ctx->subs_done = true;
     return ctx->subs;
 }
 
 static const LeanMeta* get_meta(gd_graph* g, const LeanSub* sub, int R) {
+    LeanCtx* ctx = lean_ctx_of(g);
     std::lock_guard<std::mutex> lk(g->mu);
-    if (!g->lean_ctx) g->lean_ctx = new LeanCtx();
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
-    for (const LeanMeta* q : ctx->metas)
-        if (q->R == R && q->sub == sub->id) return q->dev ? q : nullptr;
-    LeanMeta* mp = new LeanMeta();
-    LeanMeta& m = *mp;
+    for (const auto& q : ctx->metas)
+        if (q->R == R && q->sub == sub->id) return q->dev ? q.get() : nullptr;
+    ctx->metas.push_back(std::make_unique<LeanMeta>());
+    LeanMeta& m = *ctx->metas.back();
     m.R = R;
     m.sub = sub->id;
     std::vector<std::vector<int>> own;
@@ -1354,14 +1359,11 @@ static const LeanMeta* get_meta(gd_graph* g, const LeanSub* sub, int R) {
         var[2 * i] = d > 0 ? (uint32_t)loc[g->h_var_edges[b]] * 256u : kNone;
         var[2 * i + 1] = d > 1 ? (uint32_t)loc[g->h_var_edges[b + 1]] * 256u : kNone;
     }
-    if (cudaMalloc((void**)&m.dev, m.bytes) != cudaSuccess ||
-        cudaMemcpy(m.dev, blob.data(), m.bytes, cudaMemcpyHostToDevice) != cudaSuccess) {
-        if (m.dev) cudaFree(m.dev);
-        m.dev = nullptr;
+    if (device_alloc(m.dev, m.bytes) != cudaSuccess || cudaMemcpy(m.dev.get(), blob.data(), m.bytes, cudaMemcpyHostToDevice) != cudaSuccess) {
+        m.dev.reset();
         cudaGetLastError();
     }
-    ctx->metas.push_back(mp);
-    return mp->dev ? mp : nullptr;
+    return m.dev ? &m : nullptr;
 }
 
 static bool lean_applicable(const gd_graph* g, const gd_model* m) {
@@ -1467,7 +1469,7 @@ static bool lean_fill(gd_graph* g, const LeanSub* sub, const gd_model* m, int64_
     p.v_lo = sub->v_lo; p.nv = sub->nv; p.part = sub->id >= 0 ? 1 : 0;
     p.R = best.R; p.G = best.G; p.NCH = meta->NCH;
     p.ct_n = kLeanCtN; p.rt_n = best.rt_n; p.vt_n = kLeanVtN;
-    p.meta = meta->dev;
+    p.meta = meta->dev.get();
     p.off_me = 0; p.off_ms = meta->off_ms; p.off_mi = meta->off_mi; p.off_var = meta->off_var;
     p.off_ct = (int)meta->bytes;
     p.off_rt = p.off_ct + (kLeanCtN + 2) * 128;
@@ -1492,10 +1494,10 @@ static bool lean_fill(gd_graph* g, const LeanSub* sub, const gd_model* m, int64_
 bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>* out, bool whole_only) {
     out->clear();
     if (!lean_applicable(g, m)) return false;
-    const std::vector<LeanSub*>& subs = lean_subs(g);
+    const std::vector<std::unique_ptr<LeanSub>>& subs = lean_subs(g);
     // tiles of 32 syndromes a CTA will see (one CTA per SM; large batches: the quantisation no longer matters)
     const int tpc = (int)std::min<long long>(64, std::max<long long>(1, ((B + 31) / 32 + g->sm_count - 1) / g->sm_count));
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
+    LeanCtx* ctx = lean_ctx_of(g);
     // which parts, and the read-out table they share (cached per option set)
     int mode = -2, ri = -1;                                    // mode: 0 whole graph, 1 components, -1 neither fits
     {
@@ -1505,8 +1507,9 @@ bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>*
     if (mode == -2) {
         int modes[2], ris[2];
         // (nv | 1) <= E: the staged logits reuse the free message buffer
-        const int ri_whole = (subs[0]->nv | 1) <= subs[0]->E ? lean_rt_choice(g, {subs[0]}) : -1;
-        std::vector<const LeanSub*> comps(subs.begin() + 1, subs.end());
+        const int ri_whole = (subs[0]->nv | 1) <= subs[0]->E ? lean_rt_choice(g, {subs[0].get()}) : -1;
+        std::vector<const LeanSub*> comps;
+        for (size_t i = 1; i < subs.size(); ++i) comps.push_back(subs[i].get());
         bool comps_ok = !comps.empty();
         for (const LeanSub* c : comps) comps_ok = comps_ok && (c->nv | 1) <= c->E;
         const int ri_comps = comps_ok ? lean_rt_choice(g, comps) : -1;
@@ -1522,7 +1525,7 @@ bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>*
     if (mode < 0) return false;
     const size_t first = mode == 0 ? 0 : 1, last = mode == 0 ? 1 : subs.size();
     for (size_t si = first; si < last; ++si) {
-        const LeanSub* sub = subs[si];
+        const LeanSub* sub = subs[si].get();
         LeanGeom geom;
         {
             std::lock_guard<std::mutex> lk(g->mu);
@@ -1551,9 +1554,8 @@ bool lean_plan(gd_graph* g, const gd_model* m, int64_t B, std::vector<LeanPlan>*
 }
 
 static cudaMemPool_t lean_pool(gd_graph* g) {
+    LeanCtx* ctx = lean_ctx_of(g);
     std::lock_guard<std::mutex> lk(g->mu);
-    if (!g->lean_ctx) g->lean_ctx = new LeanCtx();
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
     if (!ctx->pool) {
         cudaMemPoolProps props;
         memset(&props, 0, sizeof(props));
@@ -1561,21 +1563,20 @@ static cudaMemPool_t lean_pool(gd_graph* g) {
         props.handleTypes = cudaMemHandleTypeNone;
         props.location.type = cudaMemLocationTypeDevice;
         props.location.id = g->device;
-        if (cudaMemPoolCreate(&ctx->pool, &props) != cudaSuccess) {
-            ctx->pool = nullptr;
+        if (create(ctx->pool, cudaMemPoolCreate, &props) != cudaSuccess) {
             cudaGetLastError();
             return nullptr;
         }
         unsigned long long keep = ~0ull;                          // never hand the workspace back between calls
-        cudaMemPoolSetAttribute(ctx->pool, cudaMemPoolAttrReleaseThreshold, &keep);
+        cudaMemPoolSetAttribute(ctx->pool.get(), cudaMemPoolAttrReleaseThreshold, &keep);
     }
-    return ctx->pool;
+    return ctx->pool.get();
 }
 
 // Training backward geometry (cached per graph, option set and tiles per CTA): three [E][32] arrays per group, one copy of each
 // table, the bins.
 static bool lean_bwd_geom(gd_graph* g, const LeanParams& fp, LeanBwdGeom* out) {
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
+    LeanCtx* ctx = lean_ctx_of(g);
     const int tpc = (int)std::min<long long>(64, std::max<long long>(1, ((fp.B + 31) / 32 + g->sm_count - 1) / g->sm_count));
     {
         std::lock_guard<std::mutex> lk(g->mu);
@@ -1604,7 +1605,7 @@ static bool lean_bwd_geom(gd_graph* g, const LeanParams& fp, LeanBwdGeom* out) {
         std::vector<std::vector<int>> own;
         int nch;
         double bal;
-        assign_owners(g, lean_subs(g)[0], R, own, &nch, &bal);
+        assign_owners(g, lean_subs(g)[0].get(), R, own, &nch, &bal);
         if (nch == 0 || nch > 32) continue;
         const int meta = align_up_i(align_up_i(2 * R * nch * 16 + R * nch * 4, 16) + g->V * 8, 16);
         nchs[R] = nch; metas[R] = meta; mxs[R] = bal > 0.0 ? (int)std::lround((double)E / ((double)R * bal)) : 0;
@@ -1640,43 +1641,37 @@ static bool lean_bwd_geom(gd_graph* g, const LeanParams& fp, LeanBwdGeom* out) {
 static LeanEntry* lean_entry(gd_graph* g, LeanCtx* ctx, const LeanParams& p, const gd_model* model, const float* w, cudaStream_t st) {
     LeanEntry* hit = nullptr;
     LeanEntry* lru = nullptr;
-    for (LeanEntry* e : ctx->entries) {
+    for (const auto& e : ctx->entries) {
         if (e->st == st && e->w == w && e->T == model->iters && e->hid == model->hidden && e->ct_n == p.ct_n && e->rt_n == p.rt_n &&
             e->vt_n == p.vt_n)
-            hit = e;
-        if (!lru || e->last_use < lru->last_use) lru = e;
+            hit = e.get();
+        if (!lru || e->last_use < lru->last_use) lru = e.get();
     }
     if (!hit) {
         const bool same_shape = lru && lru->ct_n == p.ct_n && lru->rt_n == p.rt_n && lru->vt_n == p.vt_n;
         if ((int)ctx->entries.size() < kMaxEntries || !same_shape) {
-            if ((int)ctx->entries.size() >= kMaxEntries) {          // table sizes changed (options): drop the oldest entry
-                cudaEventSynchronize(lru->ev);
-                cudaFree(lru->dev);
-                cudaEventDestroy(lru->ev);
-                ctx->entries.erase(std::find(ctx->entries.begin(), ctx->entries.end(), lru));
-                delete lru;
-            }
-            hit = new LeanEntry();
+            if ((int)ctx->entries.size() >= kMaxEntries)            // table sizes changed (options): drop the oldest entry
+                ctx->entries.erase(std::find_if(ctx->entries.begin(), ctx->entries.end(), [&](const auto& e) { return e.get() == lru; }));
+            auto fresh = std::make_unique<LeanEntry>();
             size_t off = 0;
             auto take = [&](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
             take(kHdrBytes);
-            hit->o_ct = take((size_t)(p.ct_n + 2) * 16);
-            hit->o_rt = take((size_t)(p.rt_n + 2) * 16);
-            hit->o_vt = take((size_t)kMaxSlots * (8 * p.vt_n + 2) * 16);   // room for the finest tables (8 x the base pieces)
-            if (cudaMalloc((void**)&hit->dev, off) != cudaSuccess || cudaMemsetAsync(hit->dev, 0, kHdrBytes, st) != cudaSuccess ||
-                cudaMemsetAsync(hit->dev + offsetof(LeanHeader, slot_bits), 0xFF, sizeof(LeanHeader::slot_bits), st) != cudaSuccess ||
-                cudaEventCreateWithFlags(&hit->ev, cudaEventDisableTiming) != cudaSuccess) {
-                if (hit->dev) cudaFree(hit->dev);
-                delete hit;
+            fresh->o_ct = take((size_t)(p.ct_n + 2) * 16);
+            fresh->o_rt = take((size_t)(p.rt_n + 2) * 16);
+            fresh->o_vt = take((size_t)kMaxSlots * (8 * p.vt_n + 2) * 16);   // room for the finest tables (8 x the base pieces)
+            if (device_alloc(fresh->dev, off) != cudaSuccess || cudaMemsetAsync(fresh->dev.get(), 0, kHdrBytes, st) != cudaSuccess ||
+                cudaMemsetAsync(fresh->dev.get() + offsetof(LeanHeader, slot_bits), 0xFF, sizeof(LeanHeader::slot_bits), st) != cudaSuccess ||
+                create(fresh->ev, cudaEventCreateWithFlags, cudaEventDisableTiming) != cudaSuccess) {
                 cudaGetLastError();
                 return nullptr;
             }
-            ctx->entries.push_back(hit);
+            hit = fresh.get();
+            ctx->entries.push_back(std::move(fresh));
         } else {
             hit = lru;                                            // recycle: back to the state of a new entry, after its last use
-            if (hit->st != st && cudaStreamWaitEvent(st, hit->ev, 0) != cudaSuccess) return nullptr;
-            if (cudaMemsetAsync(hit->dev, 0, kHdrBytes, st) != cudaSuccess ||
-                cudaMemsetAsync(hit->dev + offsetof(LeanHeader, slot_bits), 0xFF, sizeof(LeanHeader::slot_bits), st) != cudaSuccess)
+            if (hit->st != st && cudaStreamWaitEvent(st, hit->ev.get(), 0) != cudaSuccess) return nullptr;
+            if (cudaMemsetAsync(hit->dev.get(), 0, kHdrBytes, st) != cudaSuccess ||
+                cudaMemsetAsync(hit->dev.get() + offsetof(LeanHeader, slot_bits), 0xFF, sizeof(LeanHeader::slot_bits), st) != cudaSuccess)
                 return nullptr;
             hit->calls = 0;
         }
@@ -1702,7 +1697,7 @@ int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>&
     const long long prep_blocks = (B + prep_rows - 1) / prep_rows;
     GD_CHECK_ARG(prep_blocks < (1ll << 30), "gd_decode_fwd: batch too large for the table kernel's prep pass");
     cudaMemPool_t pool = lean_pool(g);
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
+    LeanCtx* ctx = lean_ctx_of(g);
     std::lock_guard<std::mutex> enq(ctx->enq);
     LeanEntry* ent = pool ? lean_entry(g, ctx, p, model, weights_dev, st) : nullptr;
     if (!ent) {
@@ -1716,15 +1711,16 @@ int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>&
     const size_t o_slot = take((size_t)B * 2), o_pos = take((size_t)B * 4), o_idx = take((size_t)B * 4);
     const size_t o_sgn = take(x_dev ? (size_t)B * p.nw * 4 : 0);
     const size_t o_defer = take((size_t)B * 4), o_x = take(x_dev ? 0 : (size_t)B * N * 4);
-    unsigned char* ws = nullptr;
-    GD_CUDA(cudaMallocFromPoolAsync((void**)&ws, off, pool, st));
-    LeanHeader* hdr = reinterpret_cast<LeanHeader*>(ent->dev);
+    PoolAlloc<unsigned char> wsa(st);
+    GD_CUDA(wsa.alloc(off, pool));
+    unsigned char* ws = wsa.get();
+    LeanHeader* hdr = reinterpret_cast<LeanHeader*>(ent->dev.get());
     LeanCall* call = &hdr->calls[ent->calls & 1];
     LeanCall* next_call = &hdr->calls[(ent->calls + 1) & 1];
     ++ent->calls;
-    float4* ctab = reinterpret_cast<float4*>(ent->dev + ent->o_ct);
-    float4* rtab = reinterpret_cast<float4*>(ent->dev + ent->o_rt);
-    float4* vtab = reinterpret_cast<float4*>(ent->dev + ent->o_vt);
+    float4* ctab = reinterpret_cast<float4*>(ent->dev.get() + ent->o_ct);
+    float4* rtab = reinterpret_cast<float4*>(ent->dev.get() + ent->o_rt);
+    float4* vtab = reinterpret_cast<float4*>(ent->dev.get() + ent->o_vt);
     int rc = GD_OK;
     cudaError_t e = cudaSuccess;
     {
@@ -1776,7 +1772,7 @@ int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>&
         e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem);
         if (e == cudaSuccess) e = pdl_launch(kern, dim3(pl.grid), dim3(pl.threads), (size_t)pl.smem, st, q);
     }
-    cudaEventRecord(ent->ev, st);                                // the entry's tables are free again after this point of the stream
+    cudaEventRecord(ent->ev.get(), st);                          // the entry's tables are free again after this point of the stream
     // the syndromes the tables could not serve: edge-owner kernel, direct evaluation, per item
     DecodeIO dio = io;
     if (e == cudaSuccess && !x_dev) {
@@ -1792,7 +1788,7 @@ int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>&
                            reinterpret_cast<const int*>(ws + o_defer)};
         rc = edge_decode(g, model, deferred, dio, st, &dl);
     }
-    cudaError_t ef = cudaFreeAsync(ws, st);
+    cudaError_t ef = wsa.release();
     if (rc != GD_OK) return rc;
     GD_CUDA(e);
     GD_CUDA(ef);
@@ -1808,12 +1804,12 @@ int packed_via_unpack(gd_graph* g, const float* prior_dev, const uint32_t* synd_
         set_error("gd_decode_packed_fwd: no memory pool on device %d", g->device);
         return GD_ERR_CUDA;
     }
-    float* xw = nullptr;
-    GD_CUDA(cudaMallocFromPoolAsync((void**)&xw, (size_t)B * g->N * sizeof(float), pool, st));
-    lean_unpack_kernel<<<g->sm_count * 4, 256, 0, st>>>(prior_dev, synd_dev, nullptr, nullptr, xw, B, g->V, g->C, (g->C + 31) / 32);
+    PoolAlloc<float> xw(st);
+    GD_CUDA(xw.alloc((size_t)B * g->N * sizeof(float), pool));
+    lean_unpack_kernel<<<g->sm_count * 4, 256, 0, st>>>(prior_dev, synd_dev, nullptr, nullptr, xw.get(), B, g->V, g->C, (g->C + 31) / 32);
     cudaError_t e = cudaGetLastError();
-    int rc = e == cudaSuccess ? run(ctx, xw) : GD_OK;
-    cudaError_t ef = cudaFreeAsync(xw, st);
+    int rc = e == cudaSuccess ? run(ctx, xw.get()) : GD_OK;
+    cudaError_t ef = xw.release();
     if (rc != GD_OK) return rc;
     GD_CUDA(e);
     GD_CUDA(ef);
@@ -1832,14 +1828,14 @@ int64_t lean_bwd_bins_floats(const gd_graph* g, const gd_model* model) {
 int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const float* weights_dev, const float* x_dev,
                   const float* stash_dev, const float* grad_logit_dev, float* grad_weights_dev, float* bins_dev, int accumulate,
                   int64_t B, cudaStream_t st) {
-    LeanCtx* ctx = static_cast<LeanCtx*>(g->lean_ctx);
+    LeanCtx* ctx = lean_ctx_of(g);
     std::lock_guard<std::mutex> enq(ctx->enq);
     // the table set the forward of this step used (same stream, same weights): it is not touched in between
     LeanEntry* ent = nullptr;
-    for (LeanEntry* e : ctx->entries)
+    for (const auto& e : ctx->entries)
         if (e->st == st && e->w == weights_dev && e->T == model->iters && e->hid == model->hidden && e->ct_n == fwd.p.ct_n &&
             e->rt_n == fwd.p.rt_n && e->vt_n == fwd.p.vt_n)
-            ent = e;
+            ent = e.get();
     if (!ent) {
         set_error("gd_decode_bwd: no table set of a matching gd_decode_fwd_train on this stream (call the forward first)");
         return GD_ERR_INVALID;
@@ -1850,17 +1846,17 @@ int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const
     LeanBwdGeom bg;
     if (!lean_bwd_geom(g, fwd.p, &bg)) return GD_OK;           // the forward saw the same answer and left the stash to the edge-owner kernel
     const int bestR = bg.R, bestG = bg.G;
-    const LeanMeta* meta = get_meta(g, lean_subs(g)[0], bestR);
+    const LeanMeta* meta = get_meta(g, lean_subs(g)[0].get(), bestR);
     if (!meta) {
         set_error("gd_decode_bwd: could not upload the table backward's metadata on device %d", g->device);
         return GD_ERR_CUDA;
     }
     const LeanTrainHdr* hdr = lean_train_hdr(const_cast<float*>(stash_dev), g, model, B);
     p.x = x_dev; p.stash = stash_dev; p.train = hdr; p.grad_logit = grad_logit_dev;
-    p.ctab = reinterpret_cast<const float4*>(ent->dev + ent->o_ct);
-    p.rtab = reinterpret_cast<const float4*>(ent->dev + ent->o_rt);
-    p.vtab = reinterpret_cast<const float4*>(ent->dev + ent->o_vt);
-    p.meta = meta->dev; p.bins = reinterpret_cast<long long*>(bins_dev);
+    p.ctab = reinterpret_cast<const float4*>(ent->dev.get() + ent->o_ct);
+    p.rtab = reinterpret_cast<const float4*>(ent->dev.get() + ent->o_rt);
+    p.vtab = reinterpret_cast<const float4*>(ent->dev.get() + ent->o_vt);
+    p.meta = meta->dev.get(); p.bins = reinterpret_cast<long long*>(bins_dev);
     p.B = B; p.T = model->iters; p.V = g->V; p.C = g->C; p.E = E; p.N = g->N; p.R = bestR; p.G = bestG; p.NCH = meta->NCH;
     p.ct_n = ct_n; p.rt_n = rt_n; p.vt_n = vt_n;
     p.off_me = 0; p.off_ms = meta->off_ms; p.off_mi = meta->off_mi; p.off_var = meta->off_var;
@@ -1879,21 +1875,3 @@ int lean_backward(gd_graph* g, const gd_model* model, const LeanPlan& fwd, const
 }
 
 }  // namespace gd
-
-void gd_lean_ctx_destroy(gd_graph* g) {
-    gd::LeanCtx* ctx = static_cast<gd::LeanCtx*>(g->lean_ctx);
-    if (!ctx) return;
-    for (gd::LeanMeta* m : ctx->metas) {
-        if (m->dev) cudaFree(m->dev);
-        delete m;
-    }
-    for (gd::LeanSub* sb : ctx->subs) delete sb;
-    for (gd::LeanEntry* e : ctx->entries) {
-        if (e->ev) { cudaEventSynchronize(e->ev); cudaEventDestroy(e->ev); }
-        if (e->dev) cudaFree(e->dev);
-        delete e;
-    }
-    if (ctx->pool) cudaMemPoolDestroy(ctx->pool);
-    delete ctx;
-    g->lean_ctx = nullptr;
-}

@@ -17,54 +17,38 @@ struct gd_pipeline {
     int64_t max_B = 0;
     int depth = 0;
     int nw = 0, vw = 0;
-    cudaStream_t s_in = nullptr, s_comp = nullptr, s_out = nullptr;
-    float* w_dev = nullptr;
+    gd::DeviceBuffer<float> w_dev;
+    gd::Stream s_in, s_comp, s_out;
     struct Slot {
-        float* x = nullptr;          // [max_B, N]   (unpacked submissions)
-        float* prior = nullptr;      // [max_B]
-        uint32_t* synd = nullptr;    // [max_B, nw]
-        float* prob = nullptr;       // [max_B, V]
-        uint8_t* hard = nullptr;     // [max_B, V]
-        uint32_t* bits = nullptr;    // [max_B, vw]
-        cudaEvent_t ev_in = nullptr, ev_comp = nullptr, ev_out = nullptr;
+        gd::DeviceBuffer<float> x;          // [max_B, N]   (unpacked submissions)
+        gd::DeviceBuffer<float> prior;      // [max_B]
+        gd::DeviceBuffer<uint32_t> synd;    // [max_B, nw]
+        gd::DeviceBuffer<float> prob;       // [max_B, V]
+        gd::DeviceBuffer<uint8_t> hard;     // [max_B, V]
+        gd::DeviceBuffer<uint32_t> bits;    // [max_B, vw]
+        gd::Event ev_in, ev_comp, ev_out;
         bool in_flight = false;
         int rc = GD_OK;
     };
     std::vector<Slot> slots;
     long long submitted = 0;         // tickets handed out so far; ticket t lives in slot t % depth
     std::mutex mu;
+    // batches in flight still use the slots' buffers: wait for them, then the members go (slots before streams)
+    ~gd_pipeline() {
+        for (auto& s : slots)
+            if (s.in_flight) cudaEventSynchronize(s.ev_out.get());
+    }
 };
 
-namespace {
-
-void pipeline_free(gd_pipeline* p) {
-    if (!p) return;
-    gd::DeviceGuard dg(p->g->device);
-    for (auto& s : p->slots) {
-        if (s.ev_out && s.in_flight) cudaEventSynchronize(s.ev_out);
-        cudaFree(s.x); cudaFree(s.prior); cudaFree(s.synd); cudaFree(s.prob); cudaFree(s.hard); cudaFree(s.bits);
-        if (s.ev_in) cudaEventDestroy(s.ev_in);
-        if (s.ev_comp) cudaEventDestroy(s.ev_comp);
-        if (s.ev_out) cudaEventDestroy(s.ev_out);
-    }
-    if (p->s_in) cudaStreamDestroy(p->s_in);
-    if (p->s_comp) cudaStreamDestroy(p->s_comp);
-    if (p->s_out) cudaStreamDestroy(p->s_out);
-    cudaFree(p->w_dev);
-    delete p;
-}
-
 // make slot `i` reusable: its previous batch must have left the device
-int slot_acquire(gd_pipeline* p, int i) {
+static int slot_acquire(gd_pipeline* p, int i) {
     gd_pipeline::Slot& s = p->slots[i];
     if (s.in_flight) {
-        GD_CUDA(cudaEventSynchronize(s.ev_out));
+        GD_CUDA(cudaEventSynchronize(s.ev_out.get()));
         s.in_flight = false;
     }
     return GD_OK;
 }
-
-}  // namespace
 
 extern "C" int gd_pipeline_create(const gd_graph* g, const gd_model* model, const float* weights_host, int64_t max_B,
                                   int32_t depth, gd_pipeline** out) {
@@ -78,33 +62,36 @@ extern "C" int gd_pipeline_create(const gd_graph* g, const gd_model* model, cons
     GD_CHECK_ARG(n_w == 0 || weights_host, "gd_pipeline_create: weights is NULL");
     gd::DeviceGuard dg(g->device);
     GD_CUDA(dg.status());
-    gd_pipeline* p = new gd_pipeline();
+    std::unique_ptr<gd_pipeline> p(new gd_pipeline());
     p->g = g; p->model = *model; p->max_B = max_B; p->depth = depth;
     p->nw = (g->C + 31) / 32; p->vw = (g->V + 31) / 32;
     p->slots.resize(depth);
-    cudaError_t e = cudaStreamCreateWithFlags(&p->s_in, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->s_comp, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&p->s_out, cudaStreamNonBlocking);
-    if (e == cudaSuccess && n_w) e = cudaMalloc((void**)&p->w_dev, (size_t)n_w * sizeof(float));
-    if (e == cudaSuccess && n_w) e = cudaMemcpy(p->w_dev, weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice);
+    cudaError_t e = gd::create(p->s_in, cudaStreamCreateWithFlags, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = gd::create(p->s_comp, cudaStreamCreateWithFlags, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = gd::create(p->s_out, cudaStreamCreateWithFlags, cudaStreamNonBlocking);
+    if (e == cudaSuccess && n_w) e = gd::device_alloc(p->w_dev, (size_t)n_w * sizeof(float));
+    if (e == cudaSuccess && n_w) e = cudaMemcpy(p->w_dev.get(), weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice);
     for (auto& s : p->slots) {
-        if (e == cudaSuccess) e = cudaMalloc((void**)&s.prior, (size_t)max_B * sizeof(float));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&s.synd, (size_t)max_B * p->nw * sizeof(uint32_t));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&s.bits, (size_t)max_B * p->vw * sizeof(uint32_t));
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_in, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_comp, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_out, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = gd::device_alloc(s.prior, (size_t)max_B * sizeof(float));
+        if (e == cudaSuccess) e = gd::device_alloc(s.synd, (size_t)max_B * p->nw * sizeof(uint32_t));
+        if (e == cudaSuccess) e = gd::device_alloc(s.bits, (size_t)max_B * p->vw * sizeof(uint32_t));
+        if (e == cudaSuccess) e = gd::create(s.ev_in, cudaEventCreateWithFlags, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = gd::create(s.ev_comp, cudaEventCreateWithFlags, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = gd::create(s.ev_out, cudaEventCreateWithFlags, cudaEventDisableTiming);
     }
     if (e != cudaSuccess) {
         gd::set_error("gd_pipeline_create: %s", cudaGetErrorString(e));
-        pipeline_free(p);
         return GD_ERR_CUDA;
     }
-    *out = p;
+    *out = p.release();
     return GD_OK;
 }
 
-extern "C" void gd_pipeline_destroy(gd_pipeline* p) { pipeline_free(p); }
+extern "C" void gd_pipeline_destroy(gd_pipeline* p) {
+    if (!p) return;
+    gd::DeviceGuard dg(p->g->device);
+    std::unique_ptr<gd_pipeline> owned(p);       // released on the graph's device
+}
 
 extern "C" int gd_pipeline_set_weights(gd_pipeline* p, const float* weights_host) {
     GD_CHECK_ARG(p != nullptr, "gd_pipeline_set_weights: pipeline is NULL");
@@ -115,7 +102,7 @@ extern "C" int gd_pipeline_set_weights(gd_pipeline* p, const float* weights_host
     gd::DeviceGuard dg(p->g->device);
     GD_CUDA(dg.status());
     // in compute-stream order: batches already submitted keep the old weights (pageable source: staged before the call returns)
-    cudaError_t e = cudaMemcpyAsync(p->w_dev, weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice, p->s_comp);
+    cudaError_t e = cudaMemcpyAsync(p->w_dev.get(), weights_host, (size_t)n_w * sizeof(float), cudaMemcpyHostToDevice, p->s_comp.get());
     GD_CUDA(e);
     return GD_OK;
 }
@@ -145,22 +132,23 @@ extern "C" int gd_pipeline_submit_packed(gd_pipeline* p, const float* prior_host
     gd_pipeline::Slot& s = p->slots[i];
     int rc = slot_acquire(p, i);
     cudaError_t e = cudaSuccess;
-    if (rc == GD_OK && prob_host && !s.prob) e = cudaMalloc((void**)&s.prob, (size_t)p->max_B * g->V * sizeof(float));
+    if (rc == GD_OK && prob_host && !s.prob) e = gd::device_alloc(s.prob, (size_t)p->max_B * g->V * sizeof(float));
     if (rc == GD_OK && e == cudaSuccess) {
-        e = cudaMemcpyAsync(s.prior, prior_host, (size_t)B * sizeof(float), cudaMemcpyHostToDevice, p->s_in);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(s.synd, synd_host, (size_t)B * p->nw * sizeof(uint32_t), cudaMemcpyHostToDevice, p->s_in);
-        if (e == cudaSuccess) e = cudaEventRecord(s.ev_in, p->s_in);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(p->s_comp, s.ev_in, 0);
+        e = cudaMemcpyAsync(s.prior.get(), prior_host, (size_t)B * sizeof(float), cudaMemcpyHostToDevice, p->s_in.get());
         if (e == cudaSuccess)
-            rc = gd_decode_packed_fwd(g, &p->model, p->w_dev, s.prior, s.synd, prob_host ? s.prob : nullptr,
-                                      hard_bits_host ? s.bits : nullptr, B, (void*)p->s_comp);
-        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_comp, p->s_comp);
-        if (rc == GD_OK && e == cudaSuccess) e = cudaStreamWaitEvent(p->s_out, s.ev_comp, 0);
+            e = cudaMemcpyAsync(s.synd.get(), synd_host, (size_t)B * p->nw * sizeof(uint32_t), cudaMemcpyHostToDevice, p->s_in.get());
+        if (e == cudaSuccess) e = cudaEventRecord(s.ev_in.get(), p->s_in.get());
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(p->s_comp.get(), s.ev_in.get(), 0);
+        if (e == cudaSuccess)
+            rc = gd_decode_packed_fwd(g, &p->model, p->w_dev.get(), s.prior.get(), s.synd.get(), prob_host ? s.prob.get() : nullptr,
+                                      hard_bits_host ? s.bits.get() : nullptr, B, (void*)p->s_comp.get());
+        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_comp.get(), p->s_comp.get());
+        if (rc == GD_OK && e == cudaSuccess) e = cudaStreamWaitEvent(p->s_out.get(), s.ev_comp.get(), 0);
         if (rc == GD_OK && e == cudaSuccess && hard_bits_host)
-            e = cudaMemcpyAsync(hard_bits_host, s.bits, (size_t)B * p->vw * sizeof(uint32_t), cudaMemcpyDeviceToHost, p->s_out);
+            e = cudaMemcpyAsync(hard_bits_host, s.bits.get(), (size_t)B * p->vw * sizeof(uint32_t), cudaMemcpyDeviceToHost, p->s_out.get());
         if (rc == GD_OK && e == cudaSuccess && prob_host)
-            e = cudaMemcpyAsync(prob_host, s.prob, (size_t)B * g->V * sizeof(float), cudaMemcpyDeviceToHost, p->s_out);
-        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_out, p->s_out);
+            e = cudaMemcpyAsync(prob_host, s.prob.get(), (size_t)B * g->V * sizeof(float), cudaMemcpyDeviceToHost, p->s_out.get());
+        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_out.get(), p->s_out.get());
     }
     return pipeline_finish(p, s, rc, e, ticket);
 }
@@ -179,23 +167,23 @@ extern "C" int gd_pipeline_submit(gd_pipeline* p, const float* x_host, float* pr
     gd_pipeline::Slot& s = p->slots[i];
     int rc = slot_acquire(p, i);
     cudaError_t e = cudaSuccess;
-    if (rc == GD_OK && !s.x) e = cudaMalloc((void**)&s.x, (size_t)p->max_B * g->N * sizeof(float));
-    if (rc == GD_OK && e == cudaSuccess && prob_host && !s.prob) e = cudaMalloc((void**)&s.prob, (size_t)p->max_B * g->V * sizeof(float));
-    if (rc == GD_OK && e == cudaSuccess && hard_host && !s.hard) e = cudaMalloc((void**)&s.hard, (size_t)p->max_B * g->V);
+    if (rc == GD_OK && !s.x) e = gd::device_alloc(s.x, (size_t)p->max_B * g->N * sizeof(float));
+    if (rc == GD_OK && e == cudaSuccess && prob_host && !s.prob) e = gd::device_alloc(s.prob, (size_t)p->max_B * g->V * sizeof(float));
+    if (rc == GD_OK && e == cudaSuccess && hard_host && !s.hard) e = gd::device_alloc(s.hard, (size_t)p->max_B * g->V);
     if (rc == GD_OK && e == cudaSuccess) {
-        e = cudaMemcpyAsync(s.x, x_host, (size_t)B * g->N * sizeof(float), cudaMemcpyHostToDevice, p->s_in);
-        if (e == cudaSuccess) e = cudaEventRecord(s.ev_in, p->s_in);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(p->s_comp, s.ev_in, 0);
+        e = cudaMemcpyAsync(s.x.get(), x_host, (size_t)B * g->N * sizeof(float), cudaMemcpyHostToDevice, p->s_in.get());
+        if (e == cudaSuccess) e = cudaEventRecord(s.ev_in.get(), p->s_in.get());
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(p->s_comp.get(), s.ev_in.get(), 0);
         if (e == cudaSuccess)
-            rc = gd_decode_fwd(g, &p->model, p->w_dev, s.x, prob_host ? s.prob : nullptr, nullptr, hard_host ? s.hard : nullptr, B,
-                               (void*)p->s_comp);
-        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_comp, p->s_comp);
-        if (rc == GD_OK && e == cudaSuccess) e = cudaStreamWaitEvent(p->s_out, s.ev_comp, 0);
+            rc = gd_decode_fwd(g, &p->model, p->w_dev.get(), s.x.get(), prob_host ? s.prob.get() : nullptr, nullptr,
+                               hard_host ? s.hard.get() : nullptr, B, (void*)p->s_comp.get());
+        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_comp.get(), p->s_comp.get());
+        if (rc == GD_OK && e == cudaSuccess) e = cudaStreamWaitEvent(p->s_out.get(), s.ev_comp.get(), 0);
         if (rc == GD_OK && e == cudaSuccess && prob_host)
-            e = cudaMemcpyAsync(prob_host, s.prob, (size_t)B * g->V * sizeof(float), cudaMemcpyDeviceToHost, p->s_out);
+            e = cudaMemcpyAsync(prob_host, s.prob.get(), (size_t)B * g->V * sizeof(float), cudaMemcpyDeviceToHost, p->s_out.get());
         if (rc == GD_OK && e == cudaSuccess && hard_host)
-            e = cudaMemcpyAsync(hard_host, s.hard, (size_t)B * g->V, cudaMemcpyDeviceToHost, p->s_out);
-        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_out, p->s_out);
+            e = cudaMemcpyAsync(hard_host, s.hard.get(), (size_t)B * g->V, cudaMemcpyDeviceToHost, p->s_out.get());
+        if (rc == GD_OK && e == cudaSuccess) e = cudaEventRecord(s.ev_out.get(), p->s_out.get());
     }
     return pipeline_finish(p, s, rc, e, ticket);
 }
@@ -212,7 +200,7 @@ extern "C" int gd_pipeline_wait(gd_pipeline* p, int32_t ticket) {
         if (newest - t >= p->depth) return GD_OK;                 // its slot was reused since: submit() already waited for it
         gd_pipeline::Slot& s = p->slots[(int)(t % p->depth)];
         if (!s.in_flight) return GD_OK;
-        ev = s.ev_out;
+        ev = s.ev_out.get();
     }
     GD_CUDA(cudaEventSynchronize(ev));                            // outside the lock: other threads may keep submitting
     return GD_OK;
@@ -223,7 +211,7 @@ extern "C" int gd_pipeline_drain(gd_pipeline* p) {
     std::lock_guard<std::mutex> lk(p->mu);
     for (auto& s : p->slots)
         if (s.in_flight) {
-            GD_CUDA(cudaEventSynchronize(s.ev_out));
+            GD_CUDA(cudaEventSynchronize(s.ev_out.get()));
             s.in_flight = false;
         }
     return GD_OK;

@@ -325,23 +325,6 @@ int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* o
     return GD_OK;
 }
 
-float* streamed_slab(gd_graph* g, size_t bytes) {
-    // The slab is per graph: concurrent streamed decodes of one graph on different streams
-    // must be serialised by the caller (documented in include/gnn_decode.h).
-    std::lock_guard<std::mutex> lk(g->mu);
-    if (bytes > g->gstate_bytes) {
-        if (g->gstate) cudaFree(g->gstate);
-        g->gstate = nullptr; g->gstate_bytes = 0;
-        cudaError_t e = cudaMalloc((void**)&g->gstate, bytes);
-        if (e != cudaSuccess) {
-            set_error("gd_decode_fwd: cudaMalloc of the %zu-byte streamed edge-state slab failed: %s", bytes, cudaGetErrorString(e));
-            return nullptr;
-        }
-        g->gstate_bytes = bytes;
-    }
-    return g->gstate;
-}
-
 int streamed_decode(gd_graph* g, const StreamPlan& plan, const gd_model* model, const DecodeIO& io, cudaStream_t st) {
     StreamPlan pl = plan;
     pl.p.x = io.x; pl.p.prob = io.prob; pl.p.logit = io.logit; pl.p.hard = io.hard; pl.p.weights = io.weights;
