@@ -1148,8 +1148,8 @@ int route_decode(const gd_graph* gc, const gd_model* m, int64_t B, Use use, Rout
             set_error("gd_decode_packed_fwd: this code's edge state does not fit shared memory (streamed path has no packed form)");
             return GD_ERR_UNSUPPORTED;
         }
-        if (m->program == GD_PROG_NEURAL_BP || m->program == GD_PROG_GRU_CA || m->program == GD_PROG_V3_0 ||
-            m->program == GD_PROG_V1_2_2 || m->program == GD_PROG_V2_4_1) {
+        if (m->program == GD_PROG_GRU_CA || m->program == GD_PROG_V3_0 || m->program == GD_PROG_V1_2_2 ||
+            m->program == GD_PROG_V2_4_1) {
             set_error("gd_decode_fwd: program %d has a resident kernel only and this code's edge state does not fit "
                       "shared memory", m->program);
             return GD_ERR_UNSUPPORTED;
@@ -1158,6 +1158,11 @@ int route_decode(const gd_graph* gc, const gd_model* m, int64_t B, Use use, Rout
         if (r->tma.ok) {
             r->family = Family::StreamedTma;
             return GD_OK;
+        }
+        if (m->program == GD_PROG_NEURAL_BP) {       // the register-batched kernel (gd_streamed.cu) has no neural BP program
+            set_error("gd_decode_fwd: neural BP on a code whose edge state does not fit shared memory needs the TMA-staged "
+                      "streamed kernel, which cannot take this graph: %s", r->tma.why);
+            return GD_ERR_UNSUPPORTED;
         }
         r->family = Family::Streamed;
         return plan_streamed(g, m, B, &r->streamed);

@@ -29,9 +29,12 @@ template <int PROG, int NPAD>
 struct NodeMath {
     static constexpr bool kIsBP = (PROG == GD_PROG_BP_QUANTUM || PROG == GD_PROG_BP_CLASSICAL);
     static constexpr bool kSoftplus = (PROG == GD_PROG_V2_4);
-    static constexpr bool kSign = (PROG == GD_PROG_QGNNI || PROG == GD_PROG_V2_4 || PROG == GD_PROG_BP_QUANTUM);
-    static constexpr float kLogEps1 = PROG == GD_PROG_BP_QUANTUM ? -46.0517019f : -16.1180957f;
-    static constexpr float kEps2 = PROG == GD_PROG_BP_QUANTUM ? 1e-12f : 1e-7f;
+    // neural BP (quantum/neural_BP.py): the BP_QUANTUM check phase with eps1 = 1e-20, eps2 = 1e-15 and a residual alpha * m;
+    // its per-edge weights are read by the kernel from global memory, not staged
+    static constexpr bool kNBP = (PROG == GD_PROG_NEURAL_BP);
+    static constexpr bool kSign = (PROG == GD_PROG_QGNNI || PROG == GD_PROG_V2_4 || PROG == GD_PROG_BP_QUANTUM || kNBP);
+    static constexpr float kLogEps1 = (PROG == GD_PROG_BP_QUANTUM || kNBP) ? -46.0517019f : -16.1180957f;
+    static constexpr float kEps2 = PROG == GD_PROG_BP_QUANTUM ? 1e-12f : kNBP ? 1e-15f : 1e-7f;
     MlpSmem W1, W2, W3;
     PwlSmem P2, P3;
     int hp;
@@ -40,6 +43,7 @@ struct NodeMath {
     CubicTab ctab, rtab;
     bool use_ctab, use_rtab;
     float rtab_R;
+    float alpha;     // neural BP's residual weight
 
     // variable phase: ext = (sum of siblings) - own, prior -> the value the check phase sums
     __device__ __forceinline__ void var_update(const float (&ext)[4], const float (&pr)[4], float (&out)[4]) const {
@@ -183,6 +187,88 @@ struct NodeMath {
                 out[3] = fmaf(oo[3], sg[3], mo.w);
             }
             stg4(m_out + (size_t)e[k] * tile, out);
+        }
+    }
+
+    // Neural BP, one check: st rows [0,d) = t, then (res: residual rows present) [d,2d) = m, then the sign row.  t carries
+    // log|tanh| <= 0 with the sign flag in its sign bit.  Each edge's sum over its siblings is formed without subtracting its
+    // own term: a message without input clamp saturates, its log|tanh| (down to log 1e-20 = -46) would swamp the tiny terms
+    // of saturated siblings in fp32 (sum - own loses them), and those terms set the output's magnitude.
+    __device__ __forceinline__ void nbp_chk_out(const float (&ext)[4], const float (&t4)[4], const int (&cnt)[4], const float* st,
+                                                int tile, int d, int k, bool res, float* dst) const {
+        float out[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int q = cnt[j] - (t4[j] > 0.f ? 1 : 0);
+            out[j] = bp_check_out(ext[j], q & 1, kEps2);
+        }
+        if (res) {                                    // neural_BP.py:304: + alpha * m_p (m == 0 in the first iteration)
+            const float4 mo = lds4(st + (d + k) * tile);
+            out[0] = fmaf(alpha, mo.x, out[0]);
+            out[1] = fmaf(alpha, mo.y, out[1]);
+            out[2] = fmaf(alpha, mo.z, out[2]);
+            out[3] = fmaf(alpha, mo.w, out[3]);
+        }
+        stg4(dst, out);
+    }
+    // the syndrome sign's share of the parity (the row after the t rows, and after the m rows when they are present)
+    __device__ __forceinline__ void nbp_sign_count(const float* st, int tile, int d, bool res, int (&cnt)[4]) const {
+        const float4 s4 = lds4(st + (res ? 2 * d : d) * tile);
+        cnt[0] = s4.x < 0.f ? 1 : 0; cnt[1] = s4.y < 0.f ? 1 : 0; cnt[2] = s4.z < 0.f ? 1 : 0; cnt[3] = s4.w < 0.f ? 1 : 0;
+    }
+    // degree D, unrolled: exclusive sums as prefix + suffix, in registers
+    template <int D>
+    __device__ __forceinline__ void nbp_chk_node(const float* st, int tile, const int32_t* edges, float* m_out, bool res) const {
+        float4 tv[D];
+#pragma unroll
+        for (int k = 0; k < D; ++k) tv[k] = lds4(st + k * tile);
+        int cnt[4];
+        nbp_sign_count(st, tile, D, res, cnt);
+        float ext[D][4], run[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            const float t4[4] = {tv[k].x, tv[k].y, tv[k].z, tv[k].w};
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                ext[k][j] = run[j];
+                run[j] -= fabsf(t4[j]);
+                cnt[j] += t4[j] > 0.f ? 1 : 0;
+            }
+        }
+        run[0] = run[1] = run[2] = run[3] = 0.f;
+#pragma unroll
+        for (int k = D - 1; k >= 0; --k) {
+            const float t4[4] = {tv[k].x, tv[k].y, tv[k].z, tv[k].w};
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                ext[k][j] += run[j];
+                run[j] -= fabsf(t4[j]);
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            const float t4[4] = {tv[k].x, tv[k].y, tv[k].z, tv[k].w};
+            nbp_chk_out(ext[k], t4, cnt, st, tile, D, k, res, m_out + (size_t)__ldg(edges + k) * tile);
+        }
+    }
+    // any degree (past the unrolled ones): each exclusive sum directly from shared memory, O(d^2)
+    __device__ __forceinline__ void nbp_chk_any(const float* st, int tile, const int32_t* edges, float* m_out, int d, bool res) const {
+        int cnt[4];
+        nbp_sign_count(st, tile, d, res, cnt);
+        for (int k = 0; k < d; ++k) {
+            const float4 tv = lds4(st + k * tile);
+            cnt[0] += tv.x > 0.f ? 1 : 0; cnt[1] += tv.y > 0.f ? 1 : 0; cnt[2] += tv.z > 0.f ? 1 : 0; cnt[3] += tv.w > 0.f ? 1 : 0;
+        }
+        for (int k = 0; k < d; ++k) {
+            float ext[4] = {0.f, 0.f, 0.f, 0.f};
+            for (int i = 0; i < d; ++i) {
+                if (i == k) continue;
+                const float4 tv = lds4(st + i * tile);
+                ext[0] -= fabsf(tv.x); ext[1] -= fabsf(tv.y); ext[2] -= fabsf(tv.z); ext[3] -= fabsf(tv.w);
+            }
+            const float4 tv = lds4(st + k * tile);
+            const float t4[4] = {tv.x, tv.y, tv.z, tv.w};
+            nbp_chk_out(ext, t4, cnt, st, tile, d, k, res, m_out + (size_t)__ldg(edges + k) * tile);
         }
     }
 };

@@ -1,7 +1,7 @@
 // Streamed decoder, TMA-staged (the default path for codes whose edge state does not fit shared
 // memory -- BASELINE config 5: hypergraph-product [[1600,64]], V = 3200, C = 1536, E = 10752).
 // Same arithmetic as gd_decode.cu (reference GNNI.forward: quantum/decoder_v2_4.py:272-294,
-// quantum/QGNNI.py:228-252, quantum/BP.py:199-219, classical/CGNNI.py:259-284,
+// quantum/QGNNI.py:228-252, quantum/BP.py:199-219, quantum/neural_BP.py:263-314, classical/CGNNI.py:259-284,
 // classical/BP.py:239-259); what differs is the data movement, which is what bounds this path:
 //
 //   * each persistent CTA owns a slab in HBM   xT[N][tile] | m[E][tile] | t[E][tile] | lg[V][tile]
@@ -18,9 +18,10 @@
 //     alternates load bursts with compute and stalls 45% of its cycles on long_scoreboard);
 //   * results leave as 128-bit coalesced stores straight from registers; no node-sum arrays, two
 //     CTA barriers per iteration;
-//   * HBM traffic per edge and iteration (fp32): learned programs 20 B (m: R,R,W; t: W,R),
+//   * HBM traffic per edge and iteration (fp32): learned programs and neural BP 20 B (m: R,R,W; t: W,R),
 //     sum-product 16 B -- log|tanh| <= 0 always, so the sign flag the check phase needs rides in
-//     the sign bit of the stored value instead of a second array.
+//     the sign bit of the stored value instead of a second array.  Neural BP's per-edge weights
+//     (2 E floats per layer) are read through L2, not staged.
 #include "gd_common.cuh"
 #include "gd_math.cuh"
 #include "gd_options.cuh"
@@ -70,6 +71,7 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
     extern __shared__ __align__(128) unsigned char smem[];
     using NM = NodeMath<PROG, NPAD>;
     constexpr bool kIsBP = NM::kIsBP;
+    constexpr bool kNBP = NM::kNBP;
     constexpr bool kSoftplus = NM::kSoftplus;
     constexpr bool kSign = NM::kSign;
     constexpr bool kClamp = (PROG == GD_PROG_CGNNI || PROG == GD_PROG_BP_CLASSICAL);
@@ -95,7 +97,8 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
 
     NM nm{};
     nm.hp = p.hp;
-    if constexpr (!kIsBP) {
+    if constexpr (kNBP) nm.alpha = __ldg(p.weights + (size_t)(2 * p.T + 2) * E);   // (include/gnn_decode.h: weight layout)
+    if constexpr (!kIsBP && !kNBP) {
         float* wsm = reinterpret_cast<float*>(smem + p.off_w);
         const float* wt = p.weights;
         const int h = p.hid, hp = p.hp;
@@ -256,7 +259,52 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
                             const int b_next = __ldg(tb.var_ptr + v + 1), d = b_next - b;
                             const float4 pr = lds4(st + (p.vrows + v - v0) * tile);
                             const float* rows = st + (b - e0) * tile;
-                            if (readout) {
+                            if constexpr (kNBP) {
+                                // neural_BP.py:244-258 (a = sum of m W - own m W + prior W_p, then log|tanh(a/2)| with no clamp,
+                                // the sign of a in the sign bit) and :308-312 (read-out sum of m W + sum of prior W_p, no bare prior).
+                                // In the canonical order this variable's edges are b .. b + d - 1, so are its weights: warp-uniform
+                                // reads of W_l | W_p,l of this layer, or of the read-out's W | W_p.  Every edge has its own W_p, so the
+                                // first iteration computes each edge's value (no one-value shortcut).
+                                const float* wl = p.weights + (size_t)(readout ? p.T : it) * 2 * E + b;
+                                const float prv[4] = {pr.x, pr.y, pr.z, pr.w};
+                                float acc[4] = {0.f, 0.f, 0.f, 0.f};
+                                if (with_m)
+                                    for (int k = 0; k < d; ++k) {      // ascending edge id
+                                        const float4 mv = lds4(rows + k * tile);
+                                        const float wk = __ldg(wl + k);
+                                        acc[0] = fmaf(mv.x, wk, acc[0]); acc[1] = fmaf(mv.y, wk, acc[1]);
+                                        acc[2] = fmaf(mv.z, wk, acc[2]); acc[3] = fmaf(mv.w, wk, acc[3]);
+                                    }
+                                if (readout) {
+                                    float accp[4] = {0.f, 0.f, 0.f, 0.f};
+                                    for (int k = 0; k < d; ++k) {
+                                        const float wpk = __ldg(wl + E + k);
+#pragma unroll
+                                        for (int j = 0; j < 4; ++j) accp[j] = fmaf(prv[j], wpk, accp[j]);
+                                    }
+                                    const float lg[4] = {acc[0] + accp[0], acc[1] + accp[1], acc[2] + accp[2], acc[3] + accp[3]};
+                                    stg4(lg_st + (size_t)v * tile + l4, lg);
+                                } else {
+                                    float* tout = t_st + (size_t)b * tile + l4;
+                                    for (int k = 0; k < d; ++k) {
+                                        const float wk = __ldg(wl + k), wpk = __ldg(wl + E + k);
+                                        float4 mv = make_float4(0.f, 0.f, 0.f, 0.f);
+                                        if (with_m) mv = lds4(rows + k * tile);
+                                        const float m4[4] = {mv.x, mv.y, mv.z, mv.w};
+                                        float out[4];
+#pragma unroll
+                                        for (int j = 0; j < 4; ++j) {
+                                            const float a = acc[j] - m4[j] * wk + prv[j] * wpk;
+                                            // No input clamp here: past |a| ~ 87 exp(-|a|) underflows and log|tanh| would be 0, whose
+                                            // negation is not > 0, so the sign of a would be lost.  -FLT_MIN keeps it strictly negative
+                                            // (far below any rounding of the sums it enters).
+                                            const float tv = fminf(bp_log_abs_tanh_half<false>(a, NM::kLogEps1), -1.17549435e-38f);
+                                            out[j] = a < 0.f ? -tv : tv;
+                                        }
+                                        stg4(tout + k * tile, out);
+                                    }
+                                }
+                            } else if (readout) {
                                 float acc[4] = {0.f, 0.f, 0.f, 0.f};
                                 if (with_m) {
                                     for (int k = 0; k < d; ++k) {
@@ -358,7 +406,10 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
                         float* m_out = m_st + l4;
                         const int32_t* edges = tb.chk_edges + b;
 #define GD_CHK_CALL(D) nm.template chk_node<D>(st, tile, edges, m_out)
-                        if (ld_m || kIsBP) {
+#define GD_NBP_CHK_CALL(D) nm.template nbp_chk_node<D>(st, tile, edges, m_out, ld_m)
+                        if constexpr (kNBP) {
+                            GD_DEGREE_SWITCH(d, GD_NBP_CHK_CALL, nm.nbp_chk_any(st, tile, edges, m_out, d, ld_m))
+                        } else if (ld_m || kIsBP) {
                             GD_DEGREE_SWITCH(d, GD_CHK_CALL, {
                                 float sg[4] = {1.f, 1.f, 1.f, 1.f};
                                 if constexpr (kSign) {
@@ -433,6 +484,7 @@ _Pragma("unroll")
                             }
                             }
                         }
+#undef GD_NBP_CHK_CALL
 #undef GD_CHK_CALL
                     }
                     __syncwarp();
@@ -472,7 +524,8 @@ _Pragma("unroll")
 static int align_up_i(int x, int a) { return (x + a - 1) / a * a; }
 
 // Returns ok == false (and out->why) when the graph does not qualify (edges not in variable-sorted order, or a
-// node's rows do not fit a pipeline stage): the caller then takes the register-batched kernel.
+// node's rows do not fit a pipeline stage): the caller then takes the register-batched kernel, or refuses the call for a
+// program that kernel does not have (neural BP).
 void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out, bool train) {
     StreamTmaParams& p = out->p;
     memset(&p, 0, sizeof(p));
@@ -481,7 +534,8 @@ void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTm
     for (size_t i = 0; i < g->h_var_edges.size(); ++i)
         if (g->h_var_edges[i] != (int32_t)i) return;
     out->why = "a node's rows do not fit a pipeline stage in shared memory";
-    const bool bp = m->program == GD_PROG_BP_QUANTUM || m->program == GD_PROG_BP_CLASSICAL;
+    // neural BP is a sum-product program without MLP slots: its per-edge weights (model.hidden == E) are read from global memory
+    const bool bp = m->program == GD_PROG_BP_QUANTUM || m->program == GD_PROG_BP_CLASSICAL || m->program == GD_PROG_NEURAL_BP;
     p.B = B; p.T = m->iters; p.V = g->V; p.C = g->C; p.E = (int)g->E; p.N = g->N;
     p.hid = bp ? 0 : m->hidden;
     p.hp = align_up_i(p.hid, m->program == GD_PROG_V2_4 ? 8 : 4);
@@ -575,6 +629,7 @@ int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& plan, const gd_model* 
             k = io.stash ? decode_streamed_tma_kernel<GD_PROG_V2_4, 0, true> : decode_streamed_tma_kernel<GD_PROG_V2_4, 0>;
             break;
         case GD_PROG_BP_QUANTUM: k = decode_streamed_tma_kernel<GD_PROG_BP_QUANTUM, 0>; break;
+        case GD_PROG_NEURAL_BP: k = decode_streamed_tma_kernel<GD_PROG_NEURAL_BP, 0>; break;
         default: k = decode_streamed_tma_kernel<GD_PROG_BP_CLASSICAL, 0>; break;
     }
     GD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));

@@ -47,7 +47,9 @@ enum gd_program {
     GD_PROG_V2_4 = 2,         /* quantum/decoder_v2_4.py:230-294 hidden 128 Softplus         */
     GD_PROG_BP_QUANTUM = 3,   /* quantum/BP.py:101-124,191-219   sum-product, syndrome sign  */
     GD_PROG_BP_CLASSICAL = 4, /* classical/BP.py:99-123,231-259  sum-product                 */
-    /* the "next" update programs (SURVEY.md 8(f)-3); resident kernel only: */
+    /* the "next" update programs (SURVEY.md 8(f)-3).  GD_PROG_NEURAL_BP also decodes codes whose edge state does not fit
+       shared memory (the TMA-staged streamed kernel; edges in the canonical variable-sorted order there, GD_ERR_UNSUPPORTED
+       otherwise); programs 6-9 have a resident kernel only: */
     GD_PROG_NEURAL_BP = 5,    /* quantum/neural_BP.py:236-314    sum-product + per-edge learned weights,
                                  2*Nc un-tied layers, gated residual alpha * m_p, weighted read-out */
     GD_PROG_GRU_CA = 6,       /* quantum/QGNNNI_ca.py:177-251    hidden 20 ReLU MLPs + GRUCell(1,1) updates,
