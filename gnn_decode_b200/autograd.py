@@ -1,6 +1,9 @@
 """Training path: torch.autograd.Function around the hand-written forward-with-stash and backward
-kernels (gd_decode_fwd_train / gd_decode_bwd) of decoder_v2_4 and CGNNI.  Gradients flow to the
-decoder's MLP parameters (the reference never differentiates w.r.t. its inputs)."""
+kernels (gd_decode_fwd_train / gd_decode_bwd) of decoder_v2_4, CGNNI and neural BP (quantum/neural_BP.py,
+and decoder_v1_1, whose per-edge weights are gathered from its type tables).  Gradients flow to the
+decoder's parameters (the reference never differentiates w.r.t. its inputs).  Neural BP trains on the
+TMA-staged streamed kernel on every code; a graph outside the canonical edge order (H.to_sparse()) is
+refused with GdError."""
 import ctypes as ct
 
 import torch
@@ -51,7 +54,7 @@ class _DecodeFn(torch.autograd.Function):
             s = torch.sigmoid(-logit)
             grad_logit = torch.where((s >= 1e-7) & (s <= 1.0 - 1e-7), -g * s * (1.0 - s), torch.zeros_like(s)).contiguous()
         else:
-            # prob = sigmoid(-logit)  ->  dL/dlogit = -dL/dprob * prob * (1 - prob)
+            # prob = sigmoid(-logit) (decoder_v2_4, neural BP: no clamp)  ->  dL/dlogit = -dL/dprob * prob * (1 - prob)
             grad_logit = (-g * prob * (1.0 - prob)).contiguous()
         n_ws = lib.gd_bwd_workspace_floats(graph.handle, ct.byref(model), B)
         if n_ws < 0:
@@ -73,8 +76,8 @@ class _DecodeFn(torch.autograd.Function):
 
 
 def decode_with_grad(decoder, graph, x, return_logits=False, return_hard=False):
-    if decoder._gd_program not in (_cabi.PROG_V2_4, _cabi.PROG_CGNNI):
-        raise _cabi.GdError("training (backward) kernels exist for the decoder_v2_4 and CGNNI programs only; "
+    if decoder._gd_program not in (_cabi.PROG_V2_4, _cabi.PROG_CGNNI, _cabi.PROG_NEURAL_BP):
+        raise _cabi.GdError("training (backward) kernels exist for the decoder_v2_4, CGNNI and neural BP programs only; "
                             "call .eval() or wrap inference in torch.no_grad()")
     x32 = x.detach().to(torch.float32).contiguous()
     if x32.data_ptr() % 16:

@@ -8,7 +8,7 @@ CSRC = os.path.join(_PKG, "csrc")
 LIB_DIR = os.path.join(_PKG, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libgnn_decode_b200.so")
 SOURCES = ["gd_graph.cu", "gd_options.cu", "gd_lean.cu", "gd_decode.cu", "gd_decode_light.cu", "gd_streamed.cu", "gd_streamed_tma.cu", "gd_propagate.cu", "gd_host.cu", "gd_pipeline.cu", "gd_sampler.cu", "gd_eval.cu",
-           "gd_backward.cu", "gd_backward_light.cu", "gd_loss.cu", "gd_p2p.cu", "gd_optim.cu", "gd_bench.cu"]
+           "gd_backward.cu", "gd_backward_light.cu", "gd_backward_nbp.cu", "gd_loss.cu", "gd_p2p.cu", "gd_optim.cu", "gd_bench.cu"]
 # GD_EXTRA_NVCC: extra flags for developer builds (e.g. -DGD_VTAB_DEBUG, -Xptxas -v)
 NVCC_FLAGS = os.environ.get("GD_EXTRA_NVCC", "").split() + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3",
                                                              "-std=c++17", "-Xcompiler", "-fPIC", "-shared"]

@@ -620,9 +620,11 @@ static int64_t bwd_slab_offset(const gd_graph* g, const gd_model* m, const BwdPl
 
 extern "C" int64_t gd_bwd_workspace_floats(const gd_graph* g, const gd_model* model, int64_t B) {
     if (g && gd_model_valid(model) && model->program == GD_PROG_CGNNI && B > 0) return gd::light_bwd_workspace_floats(g, model, B);
+    if (g && gd_model_valid(model) && model->program == GD_PROG_NEURAL_BP && model->hidden == g->E && B > 0)
+        return gd::nbp_bwd_workspace_floats(g, model, B);
     if (!g || !gd_model_valid(model) || model->program != GD_PROG_V2_4 || model->hidden > 32 * gd::kUPL || B <= 0) {
-        gd::set_error("gd_bwd_workspace_floats: unsupported model (need GD_PROG_V2_4 with hidden <= %d, or GD_PROG_CGNNI)",
-                      32 * gd::kUPL);
+        gd::set_error("gd_bwd_workspace_floats: unsupported model (need GD_PROG_V2_4 with hidden <= %d, GD_PROG_CGNNI, or "
+                      "GD_PROG_NEURAL_BP with hidden == E)", 32 * gd::kUPL);
         return -1;
     }
     gd::BwdPlan pl;
@@ -637,9 +639,13 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
                              const float* stash_dev, const float* grad_logit_dev, float* grad_weights_dev,
                              float* workspace_dev, int32_t accumulate, int64_t B, void* stream) {
     GD_CHECK_ARG(g != nullptr, "gd_decode_bwd: graph is NULL");
-    GD_CHECK_ARG(gd_model_valid(model) && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI),
-                 "gd_decode_bwd: only GD_PROG_V2_4 and GD_PROG_CGNNI have a backward kernel");
-    GD_CHECK_ARG(model->hidden <= 32 * gd::kUPL, "gd_decode_bwd: hidden=%d > %d unsupported", model->hidden, 32 * gd::kUPL);
+    GD_CHECK_ARG(gd_model_valid(model) && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI ||
+                                           model->program == GD_PROG_NEURAL_BP),
+                 "gd_decode_bwd: only GD_PROG_V2_4, GD_PROG_CGNNI and GD_PROG_NEURAL_BP have a backward kernel");
+    GD_CHECK_ARG(model->program != GD_PROG_NEURAL_BP || model->hidden == g->E,
+                 "gd_decode_bwd: GD_PROG_NEURAL_BP needs model.hidden == E (%lld per-edge weights), got %d", (long long)g->E,
+                 model->hidden);
+    GD_CHECK_ARG(model->program == GD_PROG_NEURAL_BP || model->hidden <= 32 * gd::kUPL, "gd_decode_bwd: hidden=%d > %d unsupported", model->hidden, 32 * gd::kUPL);
     GD_CHECK_ARG(B >= 0, "gd_decode_bwd: negative B");
     GD_CHECK_ARG(grad_weights_dev != nullptr, "gd_decode_bwd: grad_weights is NULL");
     const int n_params = (int)gd_weights_size(model);
@@ -654,6 +660,9 @@ extern "C" int gd_decode_bwd(const gd_graph* g, const gd_model* model, const flo
     gd::Route r;
     int rc = gd::route_decode(g, model, B, gd::Use::TrainBwd, &r);
     if (rc != GD_OK) return rc;
+    if (model->program == GD_PROG_NEURAL_BP)
+        return gd::nbp_backward(g, model, weights_dev, x_dev, stash_dev, grad_logit_dev, grad_weights_dev, workspace_dev, accumulate,
+                                B, st);
     if (r.family == gd::Family::Light)
         return gd::light_backward(g, model, weights_dev, x_dev, stash_dev, grad_logit_dev, grad_weights_dev, workspace_dev,
                                   accumulate, B, st);

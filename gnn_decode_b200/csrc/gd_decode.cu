@@ -1088,7 +1088,22 @@ int edge_decode(const gd_graph* g, const gd_model* model, DecodePlan pl, const D
 int route_decode(const gd_graph* gc, const gd_model* m, int64_t B, Use use, Route* r) {
     gd_graph* g = const_cast<gd_graph*>(gc);
     r->lean.clear();
-    if (use == Use::Train || use == Use::TrainBwd) {     // (the callers take GD_PROG_V2_4 and GD_PROG_CGNNI only)
+    if (use == Use::Train || use == Use::TrainBwd) {     // (the callers take GD_PROG_V2_4, GD_PROG_CGNNI and GD_PROG_NEURAL_BP)
+        if (m->program == GD_PROG_NEURAL_BP) {
+            // the TMA-staged streamed forward on every code (its exclusive sums are the accurate arithmetic); its backward
+            // (gd_backward_nbp.cu) plans its own layout.  A graph the planner declines is refused, nothing falls back.
+            GD_CHECK_ARG(m->hidden == g->E, "%s: GD_PROG_NEURAL_BP needs model.hidden == E (%lld per-edge weights), got %d",
+                         use == Use::Train ? "gd_decode_fwd_train" : "gd_decode_bwd", (long long)g->E, m->hidden);
+            r->family = Family::StreamedTma;
+            if (use == Use::TrainBwd) return GD_OK;
+            plan_streamed_tma(g, m, B, &r->tma, true);
+            if (!r->tma.ok) {
+                set_error("gd_decode_fwd_train: neural BP trains on the streamed kernel, which cannot take this graph: %s",
+                          r->tma.why);
+                return GD_ERR_UNSUPPORTED;
+            }
+            return GD_OK;
+        }
         if (m->program == GD_PROG_CGNNI) {
             // the node-owner kernel is the only one with a CGNNI backward; that backward plans its own layout
             r->family = Family::Light;
@@ -1346,15 +1361,16 @@ extern "C" int64_t gd_stash_floats(const gd_graph* g, const gd_model* model, int
         gd::set_error("gd_stash_floats: invalid argument");
         return -1;
     }
-    if (model->program == GD_PROG_CGNNI) return (int64_t)model->iters * g->E * B;          // m after every iteration (gd_light.cuh)
+    // m after every iteration (gd_light.cuh; neural BP: the streamed forward, gd_streamed_tma.cu)
+    if (model->program == GD_PROG_CGNNI || model->program == GD_PROG_NEURAL_BP) return (int64_t)model->iters * g->E * B;
     return (int64_t)(model->iters + 1) * 2 * g->E * B + gd::kLeanTrainTailFloats + B;   // + the header and sorted list of gd_lean.cuh
 }
 
 extern "C" int gd_decode_fwd_train(const gd_graph* gc, const gd_model* model, const float* weights_dev,
                                    const float* x_dev, float* prob_dev, float* logit_dev, float* stash_dev, int64_t B,
                                    void* stream) {
-    GD_CHECK_ARG(model && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI),
-                 "gd_decode_fwd_train: only GD_PROG_V2_4 and GD_PROG_CGNNI have a backward kernel");
+    GD_CHECK_ARG(model && (model->program == GD_PROG_V2_4 || model->program == GD_PROG_CGNNI || model->program == GD_PROG_NEURAL_BP),
+                 "gd_decode_fwd_train: only GD_PROG_V2_4, GD_PROG_CGNNI and GD_PROG_NEURAL_BP have a backward kernel");
     GD_CHECK_ARG(stash_dev != nullptr || B == 0, "gd_decode_fwd_train: stash is NULL");
     gd::DecodeIO io{};
     io.weights = weights_dev; io.x = x_dev; io.prob = prob_dev; io.logit = logit_dev; io.stash = stash_dev;

@@ -88,7 +88,7 @@ struct StreamTmaParams {
     int off_w, off_stage;    // shared-memory byte offsets (mbarriers sit at 0)
     int off_ctab, off_rtab, ctab_n, rtab_n;   // decoder_v2_4: cubic tables of the check-phase and read-out MLPs (0: none)
     float ctab_R;
-    float* stash;            // training (decoder_v2_4): [(T+1)][2][E][B], the edge-owner kernel's layout (gnn_decode.h)
+    float* stash;            // training: decoder_v2_4 [(T+1)][2][E][B], the edge-owner kernel's layout; neural BP [T][E][B]
 };
 
 struct StreamTmaPlan {
@@ -99,8 +99,8 @@ struct StreamTmaPlan {
 };
 
 int plan_streamed(const gd_graph* g, const gd_model* m, int64_t B, StreamPlan* out);
-// train: decoder_v2_4's training forward (the kernel also writes the stash); no batch-size gate, training has no other
-// streamed kernel
+// train: the training forward of decoder_v2_4 or neural BP (the kernel also writes the stash); no batch-size gate, training
+// has no other streamed kernel
 void plan_streamed_tma(const gd_graph* g, const gd_model* m, int64_t B, StreamTmaPlan* out, bool train = false);
 
 // ---- routing ----
@@ -148,5 +148,11 @@ int lean_decode(gd_graph* g, const gd_model* model, const std::vector<LeanPlan>&
 int light_decode(const LightPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st);
 int streamed_decode(gd_graph* g, const StreamPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st);
 int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& pl, const gd_model* model, const DecodeIO& io, cudaStream_t st);
+
+// ---- neural BP's training backward (gd_backward_nbp.cu): the streamed forward's stash [T][E][B] -> the weight gradients ----
+int64_t nbp_bwd_workspace_floats(const gd_graph* g, const gd_model* model, int64_t B);
+int nbp_backward(const gd_graph* g, const gd_model* model, const float* weights_dev, const float* x_dev, const float* stash_dev,
+                 const float* grad_logit_dev, float* grad_weights_dev, float* workspace_dev, int accumulate, int64_t B,
+                 cudaStream_t st);
 
 }  // namespace gd

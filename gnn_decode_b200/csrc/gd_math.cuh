@@ -436,16 +436,33 @@ __device__ __forceinline__ float bp_log_abs_tanh_half(float a, float log_eps1) {
 }
 // m = log((1+o)/(1-o)), o = sign * exp(ext) clamped to [-1+eps2, 1-eps2]; ext <= 0 (up to rounding).
 //   1 - p = -expm1(ext): series for |ext| < 0.1 (saturated checks), 1 - 2^(ext log2e) otherwise.
-__device__ __forceinline__ float bp_check_out(float ext, bool odd, float eps2) {
-    const float u = fmaxf(-ext, 0.0f);
-    const float p = ex2_approx(-u * kLog2e);
+__device__ __forceinline__ float bp_one_minus_exp(float u, float p) {     // 1 - e^{-u}, p = e^{-u}
     float ser = fmaf(u, -1.0f / 120.0f, 1.0f / 24.0f);
     ser = fmaf(ser, -u, 1.0f / 6.0f);      // builds u (1 - u/2 + u^2/6 - u^3/24 + u^4/120)
     ser = fmaf(-ser, u, 0.5f);
     ser = fmaf(-ser, u, 1.0f);
-    const float one_minus = fmaxf(u < 0.1f ? u * ser : 1.0f - p, eps2);
+    return u < 0.1f ? u * ser : 1.0f - p;
+}
+__device__ __forceinline__ float bp_check_out(float ext, bool odd, float eps2) {
+    const float u = fmaxf(-ext, 0.0f);
+    const float p = ex2_approx(-u * kLog2e);
+    const float one_minus = fmaxf(bp_one_minus_exp(u, p), eps2);
     const float mag = kLn2 * (lg2_approx(1.0f + fminf(p, 1.0f - eps2)) - lg2_approx(one_minus));
     return odd ? -mag : mag;
+}
+// Derivatives of the two sum-product pieces above, for neural BP's training backward (gd_backward_nbp.cu).
+// dm/dext of bp_check_out: m = log((1+o)/(1-o)), o = ±e^ext -> dm/dext = ±1 / sinh(-ext), with no 1 - o^2 to cancel.  0 where
+// the clamp of |o| at 1 - eps2 binds, decided from ext as bp_check_out decides it: in fp32, o rounds to ±1 long before.
+__device__ __forceinline__ float bp_dcheck_out(float ext, bool odd, float eps2) {
+    const float u = fmaxf(-ext, 0.0f);
+    if (bp_one_minus_exp(u, ex2_approx(-u * kLog2e)) < eps2) return 0.0f;
+    const float r = 1.0f / sinhf(u);
+    return odd ? -r : r;
+}
+// d/da log|tanh(a/2)| = 1 / sinh(a) (0 past |a| ~ 89, where sinh overflows); 0 where bp_log_abs_tanh_half<false>(a) returned
+// its lower clamp log(eps1) (lv: that value)
+__device__ __forceinline__ float bp_dlog_abs_tanh_half(float a, float lv, float log_eps1) {
+    return lv > log_eps1 ? 1.0f / sinhf(a) : 0.0f;
 }
 
 // torch.nn.GRUCell(1, 1) (quantum/QGNNNI_ca.py:188,198; gate order r, z, n):

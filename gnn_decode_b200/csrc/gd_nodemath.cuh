@@ -45,6 +45,17 @@ struct NodeMath {
     float rtab_R;
     float alpha;     // neural BP's residual weight
 
+    // neural BP variable phase, one edge and syndrome (neural_BP.py:244-258): u = (sum of the variable's W m) - own W m +
+    // W_p prior, and the value the check phase sums, log|tanh(u/2)| with no input clamp and the sign of u in its sign bit.
+    // Past |u| ~ 87 exp(-|u|) underflows and log|tanh| would be 0, whose negation is not > 0, so the sign of u would be lost:
+    // -FLT_MIN keeps it strictly negative (far below any rounding of the sums it enters).  The training backward
+    // (gd_backward_nbp.cu) recomputes u and t with these two, so its clamp decisions and parities are the forward's.
+    static __device__ __forceinline__ float nbp_u(float acc, float m, float wk, float pr, float wpk) { return acc - m * wk + pr * wpk; }
+    static __device__ __forceinline__ float nbp_t(float a) {
+        const float tv = fminf(bp_log_abs_tanh_half<false>(a, kLogEps1), -1.17549435e-38f);
+        return a < 0.f ? -tv : tv;
+    }
+
     // variable phase: ext = (sum of siblings) - own, prior -> the value the check phase sums
     __device__ __forceinline__ void var_update(const float (&ext)[4], const float (&pr)[4], float (&out)[4]) const {
         if constexpr (PROG == GD_PROG_V2_4) {
@@ -216,15 +227,10 @@ struct NodeMath {
         const float4 s4 = lds4(st + (res ? 2 * d : d) * tile);
         cnt[0] = s4.x < 0.f ? 1 : 0; cnt[1] = s4.y < 0.f ? 1 : 0; cnt[2] = s4.z < 0.f ? 1 : 0; cnt[3] = s4.w < 0.f ? 1 : 0;
     }
-    // degree D, unrolled: exclusive sums as prefix + suffix, in registers
+    // degree D: each edge's exclusive sum of -|t| as prefix + suffix, in registers; cnt += the edges whose t flags a negative u
     template <int D>
-    __device__ __forceinline__ void nbp_chk_node(const float* st, int tile, const int32_t* edges, float* m_out, bool res) const {
-        float4 tv[D];
-#pragma unroll
-        for (int k = 0; k < D; ++k) tv[k] = lds4(st + k * tile);
-        int cnt[4];
-        nbp_sign_count(st, tile, D, res, cnt);
-        float ext[D][4], run[4] = {0.f, 0.f, 0.f, 0.f};
+    static __device__ __forceinline__ void nbp_exclusive(const float4 (&tv)[D], float (&ext)[D][4], int (&cnt)[4]) {
+        float run[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
         for (int k = 0; k < D; ++k) {
             const float t4[4] = {tv[k].x, tv[k].y, tv[k].z, tv[k].w};
@@ -245,6 +251,27 @@ struct NodeMath {
                 run[j] -= fabsf(t4[j]);
             }
         }
+    }
+    // any degree: edge k's exclusive sum directly, ascending over the others; row(i) = t of the check's i-th edge
+    template <class Row>
+    static __device__ __forceinline__ void nbp_exclusive_any(const Row& row, int d, int k, float (&ext)[4]) {
+        ext[0] = ext[1] = ext[2] = ext[3] = 0.f;
+        for (int i = 0; i < d; ++i) {
+            if (i == k) continue;
+            const float4 tv = row(i);
+            ext[0] -= fabsf(tv.x); ext[1] -= fabsf(tv.y); ext[2] -= fabsf(tv.z); ext[3] -= fabsf(tv.w);
+        }
+    }
+    // degree D, unrolled: exclusive sums as prefix + suffix, in registers
+    template <int D>
+    __device__ __forceinline__ void nbp_chk_node(const float* st, int tile, const int32_t* edges, float* m_out, bool res) const {
+        float4 tv[D];
+#pragma unroll
+        for (int k = 0; k < D; ++k) tv[k] = lds4(st + k * tile);
+        int cnt[4];
+        nbp_sign_count(st, tile, D, res, cnt);
+        float ext[D][4];
+        nbp_exclusive<D>(tv, ext, cnt);
 #pragma unroll
         for (int k = 0; k < D; ++k) {
             const float t4[4] = {tv[k].x, tv[k].y, tv[k].z, tv[k].w};
@@ -259,13 +286,10 @@ struct NodeMath {
             const float4 tv = lds4(st + k * tile);
             cnt[0] += tv.x > 0.f ? 1 : 0; cnt[1] += tv.y > 0.f ? 1 : 0; cnt[2] += tv.z > 0.f ? 1 : 0; cnt[3] += tv.w > 0.f ? 1 : 0;
         }
+        const auto row = [&](int i) { return lds4(st + i * tile); };
         for (int k = 0; k < d; ++k) {
-            float ext[4] = {0.f, 0.f, 0.f, 0.f};
-            for (int i = 0; i < d; ++i) {
-                if (i == k) continue;
-                const float4 tv = lds4(st + i * tile);
-                ext[0] -= fabsf(tv.x); ext[1] -= fabsf(tv.y); ext[2] -= fabsf(tv.z); ext[3] -= fabsf(tv.w);
-            }
+            float ext[4];
+            nbp_exclusive_any(row, d, k, ext);
             const float4 tv = lds4(st + k * tile);
             const float t4[4] = {tv.x, tv.y, tv.z, tv.w};
             nbp_chk_out(ext, t4, cnt, st, tile, d, k, res, m_out + (size_t)__ldg(edges + k) * tile);

@@ -63,11 +63,14 @@ __device__ __forceinline__ void wait(uint64_t* bar, uint32_t parity) {
 }
 }  // namespace tma
 
-// STASH: decoder_v2_4's training forward -- also writes (m_it, a_it) of every edge and iteration and the final m into
+// STASH: the training forward.  decoder_v2_4 also writes (m_it, a_it) of every edge and iteration and the final m into
 // p.stash, in the edge-owner kernel's layout [(T+1)][2][E][B], so either backward kernel (gd_backward.cu) can take it.
+// Neural BP writes m after every iteration, [T][E][B] (m^0 = 0 is not stored), as its variable phases and read-out stage it:
+// its backward (gd_backward_nbp.cu) recomputes the rest.
 template <int PROG, int NPAD, bool STASH = false>
 __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const StreamTmaParams p) {
-    static_assert(!STASH || PROG == GD_PROG_V2_4, "the training stash exists for decoder_v2_4 only");
+    static_assert(!STASH || PROG == GD_PROG_V2_4 || PROG == GD_PROG_NEURAL_BP,
+                  "the training stash exists for decoder_v2_4 and neural BP only");
     extern __shared__ __align__(128) unsigned char smem[];
     using NM = NodeMath<PROG, NPAD>;
     constexpr bool kIsBP = NM::kIsBP;
@@ -274,6 +277,10 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
                                         const float wk = __ldg(wl + k);
                                         acc[0] = fmaf(mv.x, wk, acc[0]); acc[1] = fmaf(mv.y, wk, acc[1]);
                                         acc[2] = fmaf(mv.z, wk, acc[2]); acc[3] = fmaf(mv.w, wk, acc[3]);
+                                        if constexpr (STASH) {             // m^it (m^T at the read-out) -> stash slot it - 1
+                                            const float m4[4] = {mv.x, mv.y, mv.z, mv.w};
+                                            stash4((size_t)(it - 1) * E + b + k, s0, nvalid, m4);
+                                        }
                                     }
                                 if (readout) {
                                     float accp[4] = {0.f, 0.f, 0.f, 0.f};
@@ -293,14 +300,7 @@ __global__ void __launch_bounds__(512, 1) decode_streamed_tma_kernel(const Strea
                                         const float m4[4] = {mv.x, mv.y, mv.z, mv.w};
                                         float out[4];
 #pragma unroll
-                                        for (int j = 0; j < 4; ++j) {
-                                            const float a = acc[j] - m4[j] * wk + prv[j] * wpk;
-                                            // No input clamp here: past |a| ~ 87 exp(-|a|) underflows and log|tanh| would be 0, whose
-                                            // negation is not > 0, so the sign of a would be lost.  -FLT_MIN keeps it strictly negative
-                                            // (far below any rounding of the sums it enters).
-                                            const float tv = fminf(bp_log_abs_tanh_half<false>(a, NM::kLogEps1), -1.17549435e-38f);
-                                            out[j] = a < 0.f ? -tv : tv;
-                                        }
+                                        for (int j = 0; j < 4; ++j) out[j] = NM::nbp_t(NM::nbp_u(acc[j], m4[j], wk, prv[j], wpk));
                                         stg4(tout + k * tile, out);
                                     }
                                 }
@@ -612,8 +612,8 @@ int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& plan, const gd_model* 
     pl.p.slab = streamed_slab(g, (size_t)pl.grid * (size_t)pl.p.slab_floats * sizeof(float));
     if (!pl.p.slab) return GD_ERR_CUDA;
     void (*k)(const StreamTmaParams);
-    if (io.stash && model->program != GD_PROG_V2_4) {
-        set_error("gd_decode_fwd_train: the streamed kernel writes a training stash for GD_PROG_V2_4 only");
+    if (io.stash && model->program != GD_PROG_V2_4 && model->program != GD_PROG_NEURAL_BP) {
+        set_error("gd_decode_fwd_train: the streamed kernel writes a training stash for GD_PROG_V2_4 and GD_PROG_NEURAL_BP only");
         return GD_ERR_UNSUPPORTED;
     }
     switch (model->program) {
@@ -629,7 +629,9 @@ int streamed_tma_decode(gd_graph* g, const StreamTmaPlan& plan, const gd_model* 
             k = io.stash ? decode_streamed_tma_kernel<GD_PROG_V2_4, 0, true> : decode_streamed_tma_kernel<GD_PROG_V2_4, 0>;
             break;
         case GD_PROG_BP_QUANTUM: k = decode_streamed_tma_kernel<GD_PROG_BP_QUANTUM, 0>; break;
-        case GD_PROG_NEURAL_BP: k = decode_streamed_tma_kernel<GD_PROG_NEURAL_BP, 0>; break;
+        case GD_PROG_NEURAL_BP:
+            k = io.stash ? decode_streamed_tma_kernel<GD_PROG_NEURAL_BP, 0, true> : decode_streamed_tma_kernel<GD_PROG_NEURAL_BP, 0>;
+            break;
         default: k = decode_streamed_tma_kernel<GD_PROG_BP_CLASSICAL, 0>; break;
     }
     GD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem));

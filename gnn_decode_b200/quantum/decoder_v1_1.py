@@ -94,10 +94,12 @@ class GNNI(DecoderBase):
         return self.n_edges
 
     def _gd_params(self):
-        """The per-edge weight vectors the NEURAL_BP kernel consumes: type tables gathered by edge type."""
+        """The per-edge weight vectors the NEURAL_BP kernel consumes: type tables gathered by edge type.  In training (train()
+        mode, grad enabled) the gather is part of the autograd graph, so the per-edge gradients of the training backward are
+        summed per type by the index's backward; in inference it runs without autograd."""
         t = self.edge_types
-        with torch.no_grad():
+        with torch.set_grad_enabled(torch.is_grad_enabled() and self.training):
             out = []
             for l in range(self.Nc):
                 out += [self.layers[2 * l].W[t], self.layers[2 * l].W_p[t]]
-            return out + [self.W[t], self.W_p[t], self.alpha.detach()]
+            return out + [self.W[t], self.W_p[t], self.alpha if torch.is_grad_enabled() else self.alpha.detach()]
