@@ -417,37 +417,49 @@ __device__ __forceinline__ float tanh_half_fast(float a) {
 // ---- sum-product (BP) pieces (reference quantum/BP.py:103-117, classical/BP.py:101-116), written so
 // that fp32 keeps the accuracy the fp64 reference has in the saturated regime, with MUFU-based
 // evaluation (3 MUFU + ~15 FMA-type instructions each instead of four libm calls) ----
+// 1 - e^{-u} for u >= 0, p = e^{-u} from ex2.approx: the series u (1 - u/2 + u^2/6 - u^3/24 + u^4/120 - u^5/720) below
+// u = 0.25 (truncation <= 5e-8 relative), 1 - p above.  Subtraction turns p's error (up to 2^-22 relative) into a relative
+// error of p / (1 - p) 2^-22 in 1 - p: 9.5 2^-22 at u = 0.1, 3.5 2^-22 at 0.25 (tests/test_sum_product_formula.py).
+__device__ __forceinline__ float bp_one_minus_exp(float u, float p) {
+    float ser = fmaf(u, -1.0f / 720.0f, 1.0f / 120.0f);
+    ser = fmaf(-ser, u, 1.0f / 24.0f);
+    ser = fmaf(-ser, u, 1.0f / 6.0f);
+    ser = fmaf(-ser, u, 0.5f);
+    ser = fmaf(-ser, u, 1.0f);
+    return u < 0.25f ? u * ser : 1.0f - p;
+}
 // log|tanh(a/2)| after clamp(a, -10, 10), clamped below at log(eps1).  With q = e^{-|a|}:
-//   |a| <  1.4 : ln2 * lg2((1 - q) / (1 + q))                    (value <= -0.5: lg2.approx is accurate)
+//   |a| <  1.4 : ln2 * lg2((1 - q) / (1 + q)), 1 - q from bp_one_minus_exp   (value <= -0.5: lg2.approx is accurate; by
+//                subtraction, 1 - q would carry q's absolute error ~2.4e-7, i.e. ~2.4e-7 / |a| in the value)
 //   |a| >= 1.4 : -2 atanh(q) = -2 q (1 + q^2/3 + q^4/5 + q^6/7 + q^8/9)   (q <= 0.25; no cancellation
 //                near saturation, where log|tanh| ~ -2q is tiny and feeds log(1 - prod) downstream)
-template <bool CLAMP_IN = true>   // false: quantum/neural_BP.py:108 takes tanh(m/2) without the +-10 clamp
-__device__ __forceinline__ float bp_log_abs_tanh_half(float a, float log_eps1) {
-    const float aa = CLAMP_IN ? fminf(fabsf(a), 10.0f) : fabsf(a);
-    const float q = ex2_approx(-aa * kLog2e);
+// 2 atanh(q) = log((1 + q) / (1 - q)) = 2 q (1 + q^2/3 + q^4/5 + q^6/7 + q^8/9) for 0 <= q <= 0.25 (truncation <= 1e-7 relative)
+__device__ __forceinline__ float bp_two_atanh_small(float q) {
     const float q2 = q * q;
     float ser = fmaf(q2, 1.0f / 9.0f, 1.0f / 7.0f);
     ser = fmaf(ser, q2, 0.2f);
     ser = fmaf(ser, q2, 1.0f / 3.0f);
     ser = fmaf(ser, q2, 1.0f);
-    const float far = -2.0f * q * ser;
-    const float near = kLn2 * lg2_approx((1.0f - q) * rcp_fast(1.0f + q));     // aa == 0 -> -inf
+    return 2.0f * q * ser;
+}
+template <bool CLAMP_IN = true>   // false: quantum/neural_BP.py:108 takes tanh(m/2) without the +-10 clamp
+__device__ __forceinline__ float bp_log_abs_tanh_half(float a, float log_eps1) {
+    const float aa = CLAMP_IN ? fminf(fabsf(a), 10.0f) : fabsf(a);
+    const float q = ex2_approx(-aa * kLog2e);
+    const float far = -bp_two_atanh_small(q);
+    const float near = kLn2 * lg2_approx(bp_one_minus_exp(aa, q) * rcp_fast(1.0f + q));     // aa == 0 -> -inf
     return fmaxf(aa < 1.4f ? near : far, log_eps1);
 }
-// m = log((1+o)/(1-o)), o = sign * exp(ext) clamped to [-1+eps2, 1-eps2]; ext <= 0 (up to rounding).
-//   1 - p = -expm1(ext): series for |ext| < 0.1 (saturated checks), 1 - 2^(ext log2e) otherwise.
-__device__ __forceinline__ float bp_one_minus_exp(float u, float p) {     // 1 - e^{-u}, p = e^{-u}
-    float ser = fmaf(u, -1.0f / 120.0f, 1.0f / 24.0f);
-    ser = fmaf(ser, -u, 1.0f / 6.0f);      // builds u (1 - u/2 + u^2/6 - u^3/24 + u^4/120)
-    ser = fmaf(-ser, u, 0.5f);
-    ser = fmaf(-ser, u, 1.0f);
-    return u < 0.1f ? u * ser : 1.0f - p;
-}
+// m = log((1+o)/(1-o)), o = sign * exp(ext) clamped to [-1+eps2, 1-eps2]; ext <= 0 (up to rounding).  With p = |o| = e^{-u}:
+//   u <= 1.4 : ln2 (lg2(1 + p) - lg2(1 - p)), 1 - p from bp_one_minus_exp   (where the clamp can bind)
+//   u >  1.4 : 2 atanh(p) as a series (p < 0.25: the clamp cannot bind; 1 + p and 1 - p would round p away below 2^-24,
+//              and m, the next layer's message, would lose its digits)
 __device__ __forceinline__ float bp_check_out(float ext, bool odd, float eps2) {
     const float u = fmaxf(-ext, 0.0f);
     const float p = ex2_approx(-u * kLog2e);
     const float one_minus = fmaxf(bp_one_minus_exp(u, p), eps2);
-    const float mag = kLn2 * (lg2_approx(1.0f + fminf(p, 1.0f - eps2)) - lg2_approx(one_minus));
+    const float near = kLn2 * (lg2_approx(1.0f + fminf(p, 1.0f - eps2)) - lg2_approx(one_minus));
+    const float mag = u > 1.4f ? bp_two_atanh_small(p) : near;
     return odd ? -mag : mag;
 }
 // Derivatives of the two sum-product pieces above, for neural BP's training backward (gd_backward_nbp.cu).

@@ -51,7 +51,8 @@ def _excl(val, idx, n):
 def grads(edge_index, V, C, x, w, T, dlogit, info=None):
     """edge_index [2, E] (variable, check), x [B, V+C] (prior | check sign), w: neural BP state dict (layers.{2l}.W / W_p
     [E, 1], W, W_p [E, 1], alpha [1, 1]), dlogit [B, V].  Returns (logit [B, V], {name: dL/dname}) in float64.
-    info (a dict, optional) receives max |u| and how many (syndrome, edge, layer) items the o-clamp bound."""
+    info (a dict, optional) receives max |u|, how many (syndrome, edge, layer) items the o-clamp bound, and how many have
+    1e-20 < |u| < 1e-3 (small messages off the log clamp, where log|tanh(u/2)| is hardest to form in fp32)."""
     ev, ec = edge_index[0].long(), edge_index[1].long()
     x = x.double()
     B = x.size(0)
@@ -79,6 +80,7 @@ def grads(edge_index, V, C, x, w, T, dlogit, info=None):
         if info is not None:
             info["max_abs_u"] = max(info.get("max_abs_u", 0.0), u.abs().max().item())
             info["o_clamped"] = info.get("o_clamped", 0) + int((~pass_o).sum())
+            info["small_u"] = info.get("small_u", 0) + int(((u.abs() < 1e-3) & (u.abs() > 1e-20)).sum())
         saved.append((m, u, pass_l, S, sigma, pass_o))
         m = sigma * mag + alpha * m
     logit = torch.zeros((B, V), dtype=torch.float64).index_add_(1, ev, W["W"] * m + W["W_p"] * pi)
